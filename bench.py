@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this implementation
     python bench.py --impl reference --steps K --warmup W     # the CPU path of the reference's algorithm
+    python bench.py --steps K --warmup W --dump-outputs DIR   # also writes W and H after the last timed step, .npy
 
 A "step" is one MU iteration = the body of the reference's fit loop (pyDNMF.py:151-172):
 ``update()`` + the every-10th-iteration clamp.  For each norm W warm-up steps run untimed, then
@@ -51,7 +52,11 @@ def parse_args():
     ap.add_argument('--cpu-sample', type=int, default=32768, help='side of the bounded sample of the in-line cpu_baseline leg')
     ap.add_argument('--force-generic', action='store_true', help='disable the tcgen05 path (A/B runs)')
     ap.add_argument('--no-graph', action='store_true', help='launch every step eagerly instead of replaying a CUDA graph')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='after the timed steps, write the factors W and H of every leg as DIR/<leg>_<W|H>.npy')
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error('--steps must be at least 1')
     if a.shard_side is not None:
         a.m = a.shard_side
     a.m_given, a.n_given, a.k_given = a.m is not None, a.n is not None, a.k is not None
@@ -384,6 +389,21 @@ CONFIGS = {
                  metric='HALS & BCD iters/s (FRO, k=16, 131072x65536 fp32)'),
 }
 CFG3_GRIDS = {1: (1, 1), 2: (2, 1), 4: (2, 2), 8: (4, 2)}
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays, limit):
+    """Writes every array of `arrays` (name -> numpy array) as out_dir/<name>.npy.  When together they exceed `limit`
+    bytes, each keeps the same seeded sample of its longest axis on every run, so two builds stay comparable."""
+    os.makedirs(out_dir, exist_ok=True)
+    total = sum(a.nbytes for a in arrays.values())
+    for name, a in arrays.items():
+        if total > limit:
+            ax = int(np.argmax(a.shape))
+            keep = max(1, a.shape[ax] * limit // total)
+            idx = np.sort(np.random.default_rng(0).choice(a.shape[ax], keep, replace=False))
+            a = np.take(a, idx, axis=ax)
+        np.save(os.path.join(out_dir, name + '.npy'), a)
 
 
 def resolve_config(args, world):
@@ -549,7 +569,7 @@ def run_ours(args):
 
     sampler = ClockSampler(local) if rank == 0 else None
     windows = []
-    by_leg, pass_stats = {}, {}
+    by_leg, pass_stats, outputs = {}, {}, {}
     launches = 0
     tot_ms, tot_it = 0.0, 0
     paths = {}
@@ -604,6 +624,11 @@ def run_ours(args):
         t_b = time.perf_counter()
         windows.append((t_a, t_b))
         ms = allmax(e0.elapsed_time(e1))
+        if args.dump_outputs:
+            # the factors after the last timed step (the eager roofline replica below steps them further)
+            sfx = '_rank%d' % rank if world > 1 else ''
+            outputs[leg + '_W' + sfx] = alg._W().cpu().numpy()
+            outputs[leg + '_H' + sfx] = alg._H().cpu().numpy()
         launches += launches_per_step * args.steps     # same launches per replayed step as in the eager one
         if sg is not None:
             # per-kernel CUDA events cannot be placed inside a replayed graph: time the same steps once more, eagerly,
@@ -634,6 +659,8 @@ def run_ours(args):
         gc.collect()
         torch.cuda.synchronize()
 
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs, DUMP_LIMIT_BYTES // world)
     value = tot_it / (tot_ms / 1000.0)
 
     # ---- roofline of the dominant kernel (A-streaming pass), measured live with CUDA events ----

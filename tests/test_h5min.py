@@ -140,13 +140,10 @@ def test_reader_parses_a_library_style_layout(tmp_path):
 
 
 def _libhdf5_sample():
-    """A file written by libhdf5 itself that ships with scipy's test data (MATLAB v7.3 = HDF5 behind a 512-byte user
-    block, earliest format: v0 superblock, symbol-table root group, v1 object headers) -- the only one in this image."""
-    import scipy.io
-    p = os.path.join(os.path.dirname(scipy.io.__file__), 'matlab', 'tests', 'data', 'testhdf5_7.4_GLNX86.mat')
-    if not os.path.exists(p):
-        pytest.skip('scipy test data not installed')
-    return p
+    """A file written by libhdf5 itself, copied from scipy's test data (scipy/io/matlab/tests/data, BSD-3-Clause):
+    MATLAB v7.3 = HDF5 behind a 512-byte user block, earliest format: v0 superblock, symbol-table root group, v1
+    object headers."""
+    return os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden', 'testhdf5_7.4_GLNX86.mat')
 
 
 def test_reader_against_a_file_written_by_libhdf5():

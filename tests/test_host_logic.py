@@ -293,3 +293,25 @@ def test_bench_cpu_arm_allreduce_matches_oracle():
                 st.W = [np.maximum(w, st.eps) for w in st.W]
         for r, W, H in got:
             assert np.allclose(W, st.W[r], rtol=2e-5, atol=1e-7) and np.allclose(H, st.H[r], rtol=2e-5, atol=1e-7)
+
+
+def test_bench_dump_outputs_sample_is_fixed_and_within_the_limit(tmp_path):
+    """bench.py --dump-outputs: arrays under the limit are written whole; above it every array keeps the same seeded
+    sample of its longest axis on every run, and the files together stay within the limit."""
+    import bench
+    rs = np.random.RandomState(0)
+    arrays = {'fro_W': rs.rand(1000, 8).astype(np.float32), 'fro_H': rs.rand(8, 1000).astype(np.float32)}
+    bench.dump_outputs(str(tmp_path / 'whole'), arrays, 1 << 20)
+    for name, a in arrays.items():
+        assert np.array_equal(np.load(tmp_path / 'whole' / (name + '.npy')), a)
+    limit = 16000
+    for run in ('a', 'b'):
+        bench.dump_outputs(str(tmp_path / run), arrays, limit)
+    sizes = 0
+    for name, a in arrays.items():
+        x, y = np.load(tmp_path / 'a' / (name + '.npy')), np.load(tmp_path / 'b' / (name + '.npy'))
+        assert np.array_equal(x, y) and x.dtype == np.float32 and 0 < x.size < a.size
+        sizes += x.nbytes
+    assert sizes <= limit
+    W = np.load(tmp_path / 'a' / 'fro_W.npy')
+    assert all(any(np.array_equal(row, r) for r in arrays['fro_W']) for row in W[:5])
