@@ -36,6 +36,16 @@ extern "C" {
 #define DNMF_F32 0
 #define DNMF_F64 1
 #define DNMF_I64 2   /* collectives only (prune counts, utils.py:122-126) */
+/* 16-bit storage of the data shard A: A is fp16 / bf16, every other operand (factors, eps, partials) and every output
+ * is fp32 (dnmf_compact: 16-bit in, 16-bit out).  Only the entry points that read A accept these codes:
+ *   dnmf_workspace_bytes, dnmf_ah[_p], dnmf_wta[_p], dnmf_kl_uht[_p], dnmf_kl_wtu[_p], dnmf_residual_sqnorm,
+ *   dnmf_ah_residual, dnmf_column_err, dnmf_sqnorm (for ||A||^2), dnmf_nnz_counts, dnmf_compact.
+ * Every other entry point rejects them with DNMF_E_ARG.  dnmf_ah / dnmf_wta (and their _p forms) run on the tcgen05
+ * kind::f16 kernel (dnmf_tc16.cu) for 16-byte aligned shards with lda % 8 == 0, >= 2^20 elements and k <= 64; the
+ * KL contractions and everything else stream the 16-bit shard through the generic CUDA-core kernels.
+ * (2 is DNMF_I64, which the collectives accept, so the 16-bit codes start at 3.) */
+#define DNMF_A_F16 3
+#define DNMF_A_BF16 4
 
 #define DNMF_MATH_ACCURATE 0
 #define DNMF_MATH_TF32 1
@@ -310,7 +320,8 @@ int dnmf_ah_residual(const void* A, int64_t lda, const void* W, int64_t ldw, con
  * the same order: bit-identical results, one launch and one factor-sized HBM round trip less per half-step
  * (dist_nmf.py:730-732, :749-751, :806-830, :808-849 as pass + update = 2 launches).
  * The pass variants return DNMF_E_UNSUPPORTED, without side effects, when the call is not served by the tcgen05 path
- * (fp64, small or unaligned shards): the caller then uses the plain entry points.  fp32 only.
+ * (fp64, small or unaligned shards): the caller then uses the plain entry points.  fp32 A or a 16-bit A (DNMF_A_*) for
+ * the passes; the partials and the _p updates are fp32 (dtype DNMF_F32).
  * The view is valid until the next call that uses the same workspace. */
 int dnmf_ah_p(const void* A, int64_t lda, const void* H, int64_t ldh, int64_t m, int64_t n, int64_t k, int dtype,
               int math_mode, void* ws, int64_t ws_bytes, int64_t* view4, void* stream);

@@ -11,6 +11,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get('DNMF_LIB_PATH') or os.path.join(_HERE, 'libdnmf.so')   # override: A/B builds only
 
 F32, F64, I64 = 0, 1, 2
+A_F16, A_BF16 = 3, 4          # data shard stored in fp16 / bf16; factors and results fp32 (include/dnmf.h)
 MATH_ACCURATE, MATH_TF32 = 0, 1
 E_UNSUPPORTED = -2
 OP_AH, OP_WTA, OP_KL_UHT, OP_KL_WTU, OP_GRAM, OP_RESIDUAL, OP_SUMS, OP_NNZ, OP_AH_RESIDUAL = range(9)

@@ -5,7 +5,7 @@ HERE="$(cd "$(dirname "${BASH_SOURCE[0]}")" && pwd)"
 OUT="${HERE}/../libdnmf.so"
 NVCC="${NVCC:-/usr/local/cuda/bin/nvcc}"
 FLAGS=(-gencode arch=compute_100a,code=sm_100a -O3 -lineinfo -std=c++17 -Xcompiler -fPIC)
-SRCS=(dnmf_core dnmf_api dnmf_bcd dnmf_comm dnmf_nmfk dnmf_resident dnmf_tc dnmf_tc_kl dnmf_tc_kl64 inst_row_f32 inst_row_f64 inst_col_f32 inst_col_f64 inst_small_f32 inst_small_f64)
+SRCS=(dnmf_core dnmf_api dnmf_bcd dnmf_comm dnmf_nmfk dnmf_resident dnmf_tc dnmf_tc_kl dnmf_tc_kl64 inst_row_f32 inst_row_f64 inst_col_f32 inst_col_f64 inst_small_f32 inst_small_f64 inst_row_a16 inst_col_a16 dnmf_tc16)
 mkdir -p "${HERE}/build"
 pids=()
 objs=()

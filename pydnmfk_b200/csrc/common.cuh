@@ -1,5 +1,7 @@
 // Shared helpers for libdnmf (sm_100a).  See include/dnmf.h for the C-ABI.
 #pragma once
+#include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
@@ -79,6 +81,12 @@ __device__ __forceinline__ void vstore(T* p, const T (&in)[VecOf<T>::N]) {
   for (int i = 0; i < VecOf<T>::N; ++i) q[i] = in[i];
   *reinterpret_cast<V*>(p) = v;
 }
+
+// widening of an element of A (fp32 / fp64, or the 16-bit storage formats DNMF_A_F16 / DNMF_A_BF16)
+template <typename T>
+__device__ __forceinline__ double to_f64(T x) { return (double)x; }
+__device__ __forceinline__ double to_f64(__half x) { return (double)__half2float(x); }
+__device__ __forceinline__ double to_f64(__nv_bfloat16 x) { return (double)__bfloat162float(x); }
 
 __device__ __forceinline__ double warp_sum(double v) {
 #pragma unroll

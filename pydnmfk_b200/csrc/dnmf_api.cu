@@ -8,6 +8,12 @@
 using namespace dnmf;
 
 #define DISPATCH_T DNMF_DISPATCH_T
+// T: factor / output type, TA: element type of A
+#define DISPATCH_A(dtype, ...)                                                           \
+  if ((dtype) == DNMF_A_F16) { using T = float; using TA = __half; __VA_ARGS__; }        \
+  else if ((dtype) == DNMF_A_BF16) { using T = float; using TA = __nv_bfloat16; __VA_ARGS__; } \
+  else if ((dtype) == DNMF_F32) { using T = float; using TA = float; __VA_ARGS__; }      \
+  else { using T = double; using TA = double; __VA_ARGS__; }
 
 namespace {
 
@@ -18,14 +24,21 @@ inline int check_common(int64_t m, int64_t n, int64_t k, int dtype) {
   return 0;
 }
 
-inline size_t esize(int dtype) { return dtype == DNMF_F32 ? 4 : 8; }
+// entry points that read the data shard A also accept the 16-bit storage codes (fp32 factors and outputs)
+inline bool is_a16(int dtype) { return dtype == DNMF_A_F16 || dtype == DNMF_A_BF16; }
+inline int check_a(int64_t m, int64_t n, int64_t k, int dtype) {
+  return check_common(m, n, k, is_a16(dtype) ? DNMF_F32 : dtype);
+}
+
+// element size of the factors and outputs
+inline size_t esize(int dtype) { return dtype == DNMF_F64 ? 8 : 4; }
 
 }  // namespace
 
 extern "C" {
 
 int64_t dnmf_workspace_bytes(int op, int64_t m, int64_t n, int64_t k, int dtype) {
-  if (check_common(m, n, k, dtype) != 0) return -1;
+  if (check_a(m, n, k, dtype) != 0) return -1;
   const int kp = padded_k(k);
   int64_t bytes = 0;
   switch (op) {
@@ -33,7 +46,7 @@ int64_t dnmf_workspace_bytes(int op, int64_t m, int64_t n, int64_t k, int dtype)
     case DNMF_OP_KL_UHT: {
       const bool kl = (op == DNMF_OP_KL_UHT);
       Split sp;
-      DISPATCH_T(dtype, sp = row_pass_plan_rt<T>(kp, kl, m, n));
+      DISPATCH_A(dtype, sp = row_pass_plan_rt<T>(kp, kl, m, n));
       bytes = sp.splits > 1 ? sp.splits * m * k * (int64_t)esize(dtype) : 0;
       break;
     }
@@ -41,7 +54,7 @@ int64_t dnmf_workspace_bytes(int op, int64_t m, int64_t n, int64_t k, int dtype)
     case DNMF_OP_KL_WTU: {
       const bool kl = (op == DNMF_OP_KL_WTU);
       Split sp;
-      DISPATCH_T(dtype, sp = col_pass_plan_rt<T>(kp, kl, m, n));
+      DISPATCH_A(dtype, sp = col_pass_plan_rt<T>(kp, kl, m, n));
       bytes = sp.splits * k * n * (int64_t)esize(dtype);   // also covers transposed_out with one split
       break;
     }
@@ -95,7 +108,7 @@ int64_t dnmf_workspace_bytes(int op, int64_t m, int64_t n, int64_t k, int dtype)
 
 int dnmf_ah(const void* A, int64_t lda, const void* H, int64_t ldh, void* V, int64_t ldv, int64_t m, int64_t n,
             int64_t k, int dtype, int math_mode, void* ws, int64_t ws_bytes, void* stream) {
-  if (int rc = check_common(m, n, k, dtype)) return rc;
+  if (int rc = check_a(m, n, k, dtype)) return rc;
   DNMF_CHECK_ARG(A && H && V, "null pointer");
   DNMF_CHECK_ARG(lda >= n && ldh >= n && ldv >= k, "leading dimension too small");
   if (m == 0 || k == 0) return 0;
@@ -103,17 +116,18 @@ int dnmf_ah(const void* A, int64_t lda, const void* H, int64_t ldh, void* V, int
   if (tc_eligible(DNMF_OP_AH, A, lda, m, n, k, dtype)) {
     tls().last_path = 1;
     tls().tc_passes++;
+    if (is_a16(dtype)) return tc16_ah(A, lda, (const float*)H, ldh, (float*)V, ldv, m, n, (int)k, dtype, ws, ws_bytes, st);
     return tc_ah((const float*)A, lda, (const float*)H, ldh, (float*)V, ldv, m, n, (int)k, math_mode, ws, ws_bytes, st);
   }
   tls().last_path = 0;
   tls().generic_passes++;
-  DISPATCH_T(dtype, return row_pass_dispatch<T>(false, (const T*)A, lda, (const T*)H, ldh, (const T*)nullptr, 0, (T*)V, ldv, m, n, (int)k, T(0), ws, ws_bytes, st));
+  DISPATCH_A(dtype, return row_pass_dispatch<T, TA>(false, (const TA*)A, lda, (const T*)H, ldh, (const T*)nullptr, 0, (T*)V, ldv, m, n, (int)k, T(0), ws, ws_bytes, st));
   return 0;
 }
 
 int dnmf_wta(const void* A, int64_t lda, const void* W, int64_t ldw, void* Y, int64_t ldy, int64_t m, int64_t n,
              int64_t k, int transposed_out, int dtype, int math_mode, void* ws, int64_t ws_bytes, void* stream) {
-  if (int rc = check_common(m, n, k, dtype)) return rc;
+  if (int rc = check_a(m, n, k, dtype)) return rc;
   DNMF_CHECK_ARG(A && W && Y, "null pointer");
   DNMF_CHECK_ARG(lda >= n && ldw >= k && ldy >= (transposed_out ? k : n), "leading dimension too small");
   if (n == 0 || k == 0) return 0;
@@ -121,18 +135,20 @@ int dnmf_wta(const void* A, int64_t lda, const void* W, int64_t ldw, void* Y, in
   if (tc_eligible(DNMF_OP_WTA, A, lda, m, n, k, dtype)) {
     tls().last_path = 1;
     tls().tc_passes++;
+    if (is_a16(dtype))
+      return tc16_wta(A, lda, (const float*)W, ldw, (float*)Y, ldy, m, n, (int)k, transposed_out, dtype, ws, ws_bytes, st);
     return tc_wta((const float*)A, lda, (const float*)W, ldw, (float*)Y, ldy, m, n, (int)k, transposed_out, math_mode, ws, ws_bytes, st);
   }
   tls().last_path = 0;
   tls().generic_passes++;
-  DISPATCH_T(dtype, return col_pass_dispatch<T>(false, (const T*)A, lda, (const T*)W, ldw, (const T*)nullptr, 0, (T*)Y, ldy, m, n, (int)k, T(0), transposed_out, ws, ws_bytes, st));
+  DISPATCH_A(dtype, return col_pass_dispatch<T, TA>(false, (const TA*)A, lda, (const T*)W, ldw, (const T*)nullptr, 0, (T*)Y, ldy, m, n, (int)k, T(0), transposed_out, ws, ws_bytes, st));
   return 0;
 }
 
 int dnmf_kl_uht(const void* A, int64_t lda, const void* W, int64_t ldw, const void* H, int64_t ldh, void* V,
                 int64_t ldv, int64_t m, int64_t n, int64_t k, double eps, int dtype, int math_mode, void* ws,
                 int64_t ws_bytes, void* stream) {
-  if (int rc = check_common(m, n, k, dtype)) return rc;
+  if (int rc = check_a(m, n, k, dtype)) return rc;
   DNMF_CHECK_ARG(A && W && H && V, "null pointer");
   DNMF_CHECK_ARG(lda >= n && ldh >= n && ldw >= k && ldv >= k, "leading dimension too small");
   if (m == 0 || k == 0) return 0;
@@ -144,14 +160,14 @@ int dnmf_kl_uht(const void* A, int64_t lda, const void* W, int64_t ldw, const vo
   }
   tls().last_path = 0;
   tls().generic_passes++;
-  DISPATCH_T(dtype, return row_pass_dispatch<T>(true, (const T*)A, lda, (const T*)H, ldh, (const T*)W, ldw, (T*)V, ldv, m, n, (int)k, (T)eps, ws, ws_bytes, st));
+  DISPATCH_A(dtype, return row_pass_dispatch<T, TA>(true, (const TA*)A, lda, (const T*)H, ldh, (const T*)W, ldw, (T*)V, ldv, m, n, (int)k, (T)eps, ws, ws_bytes, st));
   return 0;
 }
 
 int dnmf_kl_wtu(const void* A, int64_t lda, const void* W, int64_t ldw, const void* H, int64_t ldh, void* Y,
                 int64_t ldy, int64_t m, int64_t n, int64_t k, double eps, int transposed_out, int dtype,
                 int math_mode, void* ws, int64_t ws_bytes, void* stream) {
-  if (int rc = check_common(m, n, k, dtype)) return rc;
+  if (int rc = check_a(m, n, k, dtype)) return rc;
   DNMF_CHECK_ARG(A && W && H && Y, "null pointer");
   DNMF_CHECK_ARG(lda >= n && ldh >= n && ldw >= k && ldy >= (transposed_out ? k : n), "leading dimension too small");
   if (n == 0 || k == 0) return 0;
@@ -163,7 +179,7 @@ int dnmf_kl_wtu(const void* A, int64_t lda, const void* W, int64_t ldw, const vo
   }
   tls().last_path = 0;
   tls().generic_passes++;
-  DISPATCH_T(dtype, return col_pass_dispatch<T>(true, (const T*)A, lda, (const T*)W, ldw, (const T*)H, ldh, (T*)Y, ldy, m, n, (int)k, (T)eps, transposed_out, ws, ws_bytes, st));
+  DISPATCH_A(dtype, return col_pass_dispatch<T, TA>(true, (const TA*)A, lda, (const T*)W, ldw, (const T*)H, ldh, (T*)Y, ldy, m, n, (int)k, (T)eps, transposed_out, ws, ws_bytes, st));
   return 0;
 }
 
@@ -277,31 +293,39 @@ int fill_view(const TcPartials& d, int64_t* view4) {
 
 int dnmf_ah_p(const void* A, int64_t lda, const void* H, int64_t ldh, int64_t m, int64_t n, int64_t k, int dtype,
               int math_mode, void* ws, int64_t ws_bytes, int64_t* view4, void* stream) {
-  if (int rc = check_common(m, n, k, dtype)) return rc;
+  if (int rc = check_a(m, n, k, dtype)) return rc;
   DNMF_CHECK_ARG(A && H && view4, "null pointer");
   if (m == 0 || k == 0 || !tc_eligible(DNMF_OP_AH, A, lda, m, n, k, dtype)) return DNMF_E_UNSUPPORTED;
   tls().last_path = 1;
   tls().tc_passes++;
   TcPartials d;
+  if (is_a16(dtype)) {
+    if (int rc = tc16_ah(A, lda, (const float*)H, ldh, nullptr, 0, m, n, (int)k, dtype, ws, ws_bytes, (cudaStream_t)stream, &d)) return rc;
+    return fill_view(d, view4);
+  }
   if (int rc = tc_ah((const float*)A, lda, (const float*)H, ldh, nullptr, 0, m, n, (int)k, math_mode, ws, ws_bytes, (cudaStream_t)stream, &d)) return rc;
   return fill_view(d, view4);
 }
 
 int dnmf_wta_p(const void* A, int64_t lda, const void* W, int64_t ldw, int64_t m, int64_t n, int64_t k, int dtype,
                int math_mode, void* ws, int64_t ws_bytes, int64_t* view4, void* stream) {
-  if (int rc = check_common(m, n, k, dtype)) return rc;
+  if (int rc = check_a(m, n, k, dtype)) return rc;
   DNMF_CHECK_ARG(A && W && view4, "null pointer");
   if (n == 0 || k == 0 || !tc_eligible(DNMF_OP_WTA, A, lda, m, n, k, dtype)) return DNMF_E_UNSUPPORTED;
   tls().last_path = 1;
   tls().tc_passes++;
   TcPartials d;
+  if (is_a16(dtype)) {
+    if (int rc = tc16_wta(A, lda, (const float*)W, ldw, nullptr, 0, m, n, (int)k, 1, dtype, ws, ws_bytes, (cudaStream_t)stream, &d)) return rc;
+    return fill_view(d, view4);
+  }
   if (int rc = tc_wta((const float*)A, lda, (const float*)W, ldw, nullptr, 0, m, n, (int)k, 1, math_mode, ws, ws_bytes, (cudaStream_t)stream, &d)) return rc;
   return fill_view(d, view4);
 }
 
 int dnmf_kl_uht_p(const void* A, int64_t lda, const void* W, int64_t ldw, const void* H, int64_t ldh, int64_t m, int64_t n,
                   int64_t k, double eps, int dtype, int math_mode, void* ws, int64_t ws_bytes, int64_t* view4, void* stream) {
-  if (int rc = check_common(m, n, k, dtype)) return rc;
+  if (int rc = check_a(m, n, k, dtype)) return rc;
   DNMF_CHECK_ARG(A && W && H && view4, "null pointer");
   if (m == 0 || k == 0 || !tc_eligible(DNMF_OP_KL_UHT, A, lda, m, n, k, dtype)) return DNMF_E_UNSUPPORTED;
   tls().last_path = 1;
@@ -313,7 +337,7 @@ int dnmf_kl_uht_p(const void* A, int64_t lda, const void* W, int64_t ldw, const 
 
 int dnmf_kl_wtu_p(const void* A, int64_t lda, const void* W, int64_t ldw, const void* H, int64_t ldh, int64_t m, int64_t n,
                   int64_t k, double eps, int dtype, int math_mode, void* ws, int64_t ws_bytes, int64_t* view4, void* stream) {
-  if (int rc = check_common(m, n, k, dtype)) return rc;
+  if (int rc = check_a(m, n, k, dtype)) return rc;
   DNMF_CHECK_ARG(A && W && H && view4, "null pointer");
   if (n == 0 || k == 0 || !tc_eligible(DNMF_OP_KL_WTU, A, lda, m, n, k, dtype)) return DNMF_E_UNSUPPORTED;
   tls().last_path = 1;
@@ -442,7 +466,7 @@ int dnmf_rowsum(const void* X, int64_t ldx, int64_t rows, int64_t cols, void* ou
 
 int dnmf_sqnorm(const void* X, int64_t ldx, int64_t rows, int64_t cols, double* out, int dtype, void* ws,
                 int64_t ws_bytes, void* stream) {
-  if (int rc = check_common(rows, cols, 0, dtype)) return rc;
+  if (int rc = check_a(rows, cols, 0, dtype)) return rc;
   DNMF_CHECK_ARG(X && out, "null pointer");
   cudaStream_t st = (cudaStream_t)stream;
   if (rows == 0 || cols == 0) {
@@ -455,7 +479,7 @@ int dnmf_sqnorm(const void* X, int64_t ldx, int64_t rows, int64_t cols, double* 
   const int64_t need = nparts * (int64_t)sizeof(double);
   if (ws == nullptr || ws_bytes < need) return fail(DNMF_E_WORKSPACE, "sqnorm needs %lld workspace bytes, got %lld", (long long)need, (long long)ws_bytes);
   dim3 grid((unsigned)rows, (unsigned)sp.chunks);
-  DISPATCH_T(dtype, (rowsum_partial_kernel<T><<<grid, 256, 0, st>>>((const T*)X, ldx, rows, cols, sp.per_chunk, (double*)ws, 1)));
+  DISPATCH_A(dtype, (rowsum_partial_kernel<TA><<<grid, 256, 0, st>>>((const TA*)X, ldx, rows, cols, sp.per_chunk, (double*)ws, 1)));
   DNMF_LAUNCH_CHECK("rowsum_partial_kernel<sq>");
   sum_all_kernel<<<1, 256, 0, st>>>((const double*)ws, nparts, out);
   DNMF_LAUNCH_CHECK("sum_all_kernel");
@@ -512,7 +536,7 @@ int dnmf_normalize(void* W, int64_t ldw, int64_t m, void* H, int64_t ldh, int64_
 int dnmf_residual_sqnorm(const void* A, int64_t lda, const void* W, int64_t ldw, const void* H, int64_t ldh,
                          int64_t m, int64_t n, int64_t k, double* out, int dtype, void* ws, int64_t ws_bytes,
                          void* stream) {
-  if (int rc = check_common(m, n, k, dtype)) return rc;
+  if (int rc = check_a(m, n, k, dtype)) return rc;
   DNMF_CHECK_ARG(A && W && H && out, "null pointer");
   cudaStream_t st = (cudaStream_t)stream;
   if (m == 0 || n == 0) {
@@ -536,7 +560,7 @@ int dnmf_residual_sqnorm(const void* A, int64_t lda, const void* W, int64_t ldw,
   if (ws == nullptr || ws_bytes < need) return fail(DNMF_E_WORKSPACE, "residual needs %lld workspace bytes, got %lld", (long long)need, (long long)ws_bytes);
   {
     int rc = 0;
-    DISPATCH_T(dtype, rc = residual_dispatch<T>((const T*)A, lda, (const T*)W, ldw, (const T*)H, ldh, m, n, (int)k, rp.chunk, (unsigned)rp.col_blocks, (unsigned)rp.chunks, (double*)ws, nullptr, nullptr, st));
+    DISPATCH_A(dtype, rc = residual_dispatch<T, TA>((const TA*)A, lda, (const T*)W, ldw, (const T*)H, ldh, m, n, (int)k, rp.chunk, (unsigned)rp.col_blocks, (unsigned)rp.chunks, (double*)ws, nullptr, nullptr, st));
     if (rc) return rc;
   }
   sum_pairs_kernel<<<1, 256, 0, st>>>((const double*)ws, nb, out);
@@ -547,7 +571,7 @@ int dnmf_residual_sqnorm(const void* A, int64_t lda, const void* W, int64_t ldw,
 int dnmf_ah_residual(const void* A, int64_t lda, const void* W, int64_t ldw, const void* H, int64_t ldh, void* V,
                      int64_t ldv, int64_t m, int64_t n, int64_t k, double* out, int dtype, void* ws, int64_t ws_bytes,
                      void* stream) {
-  if (int rc = check_common(m, n, k, dtype)) return rc;
+  if (int rc = check_a(m, n, k, dtype)) return rc;
   DNMF_CHECK_ARG(A && W && H && V && out, "null pointer");
   DNMF_CHECK_ARG(lda >= n && ldh >= n && ldw >= k && ldv >= k, "leading dimension too small");
   cudaStream_t st = (cudaStream_t)stream;
@@ -569,12 +593,12 @@ int dnmf_ah_residual(const void* A, int64_t lda, const void* W, int64_t ldw, con
 
 int dnmf_column_err(const void* A, int64_t lda, const void* W, int64_t ldw, const void* H, int64_t ldh, int64_t m,
                     int64_t n, int64_t k, double* num, double* den, int dtype, void* stream) {
-  if (int rc = check_common(m, n, k, dtype)) return rc;
+  if (int rc = check_a(m, n, k, dtype)) return rc;
   DNMF_CHECK_ARG(A && W && H && num && den, "null pointer");
   if (n == 0) return 0;
   cudaStream_t st = (cudaStream_t)stream;
   const int64_t chunk = round_up(m > 0 ? m : 1, kColPassBR);
-  DISPATCH_T(dtype, return residual_dispatch<T>((const T*)A, lda, (const T*)W, ldw, (const T*)H, ldh, m, n, (int)k, chunk, (unsigned)ceil_div(n, kColPassThreads), 1u, nullptr, num, den, st));
+  DISPATCH_A(dtype, return residual_dispatch<T, TA>((const TA*)A, lda, (const T*)W, ldw, (const T*)H, ldh, m, n, (int)k, chunk, (unsigned)ceil_div(n, kColPassThreads), 1u, nullptr, num, den, st));
   return 0;
 }
 
@@ -629,7 +653,7 @@ int dnmf_axpby(void* out, const void* x, const void* y, double a, double b, int6
 
 int dnmf_nnz_counts(const void* A, int64_t lda, int64_t m, int64_t n, int64_t* row_nnz, int64_t* col_nnz, int dtype,
                     void* stream) {
-  if (int rc = check_common(m, n, 0, dtype)) return rc;
+  if (int rc = check_a(m, n, 0, dtype)) return rc;
   DNMF_CHECK_ARG(A && row_nnz && col_nnz, "null pointer");
   cudaStream_t st = (cudaStream_t)stream;
   if (n > 0) {
@@ -640,22 +664,22 @@ int dnmf_nnz_counts(const void* A, int64_t lda, int64_t m, int64_t n, int64_t* r
     if (m > 0) cudaMemsetAsync(row_nnz, 0, m * sizeof(int64_t), st);
     return 0;
   }
-  DISPATCH_T(dtype, (row_nnz_kernel<T><<<(unsigned)ceil_div(m, 8), 256, 0, st>>>((const T*)A, lda, m, n, (long long*)row_nnz)));
+  DISPATCH_A(dtype, (row_nnz_kernel<TA><<<(unsigned)ceil_div(m, 8), 256, 0, st>>>((const TA*)A, lda, m, n, (long long*)row_nnz)));
   DNMF_LAUNCH_CHECK("row_nnz_kernel");
   const SumPlan sp = sum_plan(m, 256, 256);
   dim3 grid((unsigned)ceil_div(n, 256), (unsigned)sp.chunks);
-  DISPATCH_T(dtype, (col_nnz_kernel<T><<<grid, 256, 0, st>>>((const T*)A, lda, m, n, sp.per_chunk, (unsigned long long*)col_nnz)));
+  DISPATCH_A(dtype, (col_nnz_kernel<TA><<<grid, 256, 0, st>>>((const TA*)A, lda, m, n, sp.per_chunk, (unsigned long long*)col_nnz)));
   DNMF_LAUNCH_CHECK("col_nnz_kernel");
   return 0;
 }
 
 int dnmf_compact(const void* A, int64_t lda, const int64_t* row_idx, int64_t mr, const int64_t* col_idx, int64_t nc,
                  void* out, int64_t ldo, int dtype, void* stream) {
-  if (int rc = check_common(mr, nc, 0, dtype)) return rc;
+  if (int rc = check_a(mr, nc, 0, dtype)) return rc;
   if (mr * nc == 0) return 0;
   DNMF_CHECK_ARG(A && row_idx && col_idx && out, "null pointer");
   cudaStream_t st = (cudaStream_t)stream;
-  DISPATCH_T(dtype, (compact_kernel<T><<<(unsigned)ceil_div(mr * nc, 256), 256, 0, st>>>((const T*)A, lda, (const long long*)row_idx, mr, (const long long*)col_idx, nc, (T*)out, ldo)));
+  DISPATCH_A(dtype, (compact_kernel<TA><<<(unsigned)ceil_div(mr * nc, 256), 256, 0, st>>>((const TA*)A, lda, (const long long*)row_idx, mr, (const long long*)col_idx, nc, (TA*)out, ldo)));
   DNMF_LAUNCH_CHECK("compact_kernel");
   return 0;
 }

@@ -443,10 +443,10 @@ int make_map(CUtensorMap* map, const float* ptr, int64_t rows, int64_t cols, int
 
 int tc_padded_k(int k) { return k <= 16 ? 16 : (k <= 32 ? 32 : 64); }
 
-TcPlan tc_plan(int64_t x_len, int64_t r_len, int k) {
+TcPlan tc_plan(int64_t x_len, int64_t r_len, int k, int bk) {
   TcPlan p;
   p.x_blocks = (int)ceil_div(x_len, TC_BM);
-  p.kt_total = (int)ceil_div(r_len, TC_BK);
+  p.kt_total = (int)ceil_div(r_len, bk);
   const int sms = sm_count();
   // Number of K splits: units = x_blocks * splits are dealt to the CTAs round-robin (unit % grid), so the pass lasts
   // ceil(units / sms) * (tiles per unit + fill / drain of the unit's pipeline), plus the traffic of the partials every
@@ -454,7 +454,8 @@ TcPlan tc_plan(int64_t x_len, int64_t r_len, int k) {
   // of a fixed 12 units per SM: for a short x (8192 rows on 8 GPUs: 64 x-blocks) the old rule gave 28 splits -- 8.6 % over
   // the ideal time and 28 MiB of partials -- where 9 splits are 3 % over with a third of the partial traffic.
   const int64_t kUnitOverhead = 4;                                   // tile-times to fill + drain one unit
-  const double tile_bytes = (double)sms * TC_BM * TC_BK * 4.0;       // A bytes the machine streams per tile-time
+  const double tile_bytes = (double)sms * TC_BM * TC_BK * 4.0;       // A bytes the machine streams per tile-time (128-byte
+                                                                     // tile rows: 32 fp32 or 64 16-bit elements)
   const double split_cost = 2.0 * (double)x_len * k * 4.0 / tile_bytes;   // tile-times per extra split (write + read)
   int best_s = 1;
   double best = 1e300;
@@ -624,6 +625,21 @@ int tc_make_map(CUtensorMap* map, const float* ptr, int64_t rows, int64_t cols, 
                 CUtensorMapSwizzle swz) {
   return make_map(map, ptr, rows, cols, ld, box_cols, box_rows, swz);
 }
+// the same for a 16-bit (fp16 / bf16) row-major tensor, 128-byte swizzle (dnmf_tc16.cu)
+int tc_make_map_16(CUtensorMap* map, const void* ptr, int64_t rows, int64_t cols, int64_t ld, int box_cols, int box_rows,
+                   int bf16) {
+  EncodeTiledFn fn = encode_fn();
+  if (!fn) return fail(DNMF_E_UNSUPPORTED, "cuTensorMapEncodeTiled is not available from this driver");
+  cuuint64_t dims[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
+  cuuint64_t strides[1] = {(cuuint64_t)ld * 2};
+  cuuint32_t box[2] = {(cuuint32_t)box_cols, (cuuint32_t)box_rows};
+  cuuint32_t estr[2] = {1, 1};
+  CUresult r = fn(map, bf16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, const_cast<void*>(ptr),
+                  dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
+                  CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  if (r != CUDA_SUCCESS) return fail(DNMF_E_ARG, "cuTensorMapEncodeTiled failed with CUresult %d", (int)r);
+  return 0;
+}
 int tc_hi_mode() { return g_hi_mode; }
 unsigned long long* tc_prof_ptr() { return g_prof; }
 namespace {
@@ -647,14 +663,20 @@ bool tc_eligible(int op, const void* A, int64_t lda, int64_t m, int64_t n, int64
   if (tls().force_generic) return false;
   const bool kl = (op == DNMF_OP_KL_UHT || op == DNMF_OP_KL_WTU);
   if (op != DNMF_OP_AH && op != DNMF_OP_WTA && !kl) return false;
-  if (kl && !tc_kl_supported(k) && !tc_kl_supported_k64(k)) return false;
-  if (dtype != DNMF_F32) return false;
-  if (k < 1 || k > 64) return false;
-  if (((uintptr_t)A % 16) != 0 || (lda % 4) != 0) return false;
   if (g_min_elems < 0) {
     const char* env = getenv("DNMF_TC_MIN_ELEMS");
     g_min_elems = env ? atoll(env) : (int64_t)1 << 20;
   }
+  if (dtype == DNMF_A_F16 || dtype == DNMF_A_BF16) {
+    // 16-bit A: the kind::f16 kernel of dnmf_tc16.cu (AH / WTA only; an exact operand, no tf32 calibration involved)
+    if (kl || k < 1 || k > 64) return false;
+    if (((uintptr_t)A % 16) != 0 || (lda % 8) != 0) return false;
+    return m * n >= g_min_elems && device_is_sm100();
+  }
+  if (kl && !tc_kl_supported(k) && !tc_kl_supported_k64(k)) return false;
+  if (dtype != DNMF_F32) return false;
+  if (k < 1 || k > 64) return false;
+  if (((uintptr_t)A % 16) != 0 || (lda % 4) != 0) return false;
   if (m * n < g_min_elems) return false;
   if (!device_is_sm100()) return false;
   calibrate();
@@ -666,6 +688,7 @@ void tc_set_profile(void* buf) { g_prof = reinterpret_cast<unsigned long long*>(
 void tc_set_min_elems(int64_t elems) { g_min_elems = elems < 0 ? 0 : elems; }
 
 int64_t tc_workspace_bytes(int op, int64_t m, int64_t n, int64_t k, int dtype) {
+  if ((dtype == DNMF_A_F16 || dtype == DNMF_A_BF16) && k >= 1 && k <= 64) return tc16_workspace_bytes(op, m, n, k, dtype);
   if (dtype != DNMF_F32 || k < 1 || k > 64) return 0;
   if (op == DNMF_OP_AH) { const TcPlan p = tc_plan(m, n, tc_padded_k((int)k)); return p.bcat_bytes + p.partial_bytes; }
   if (op == DNMF_OP_WTA) { const TcPlan p = tc_plan(n, m, tc_padded_k((int)k)); return p.bcat_bytes + p.partial_bytes; }

@@ -14,6 +14,8 @@
 // Both split the reduced dimension over blockIdx.y into partial buffers that are summed in a fixed
 // order by reduce_partials_kernel (deterministic).
 #pragma once
+#include <type_traits>
+
 #include "common.cuh"
 
 namespace dnmf {
@@ -41,9 +43,9 @@ struct RowPassCfg {
   static constexpr size_t smem_bytes = sizeof(T) * ((size_t)BM * AS + (size_t)kRowPassBK * HS);
 };
 
-template <typename T, int KP, bool KL>
+template <typename T, int KP, bool KL, typename TA = T>
 __global__ void __launch_bounds__(kRowPassThreads)
-row_pass_kernel(const T* __restrict__ A, int64_t lda, const T* __restrict__ H, int64_t ldh,
+row_pass_kernel(const TA* __restrict__ A, int64_t lda, const T* __restrict__ H, int64_t ldh,
                 const T* __restrict__ W, int64_t ldw, T* __restrict__ out, int64_t ldo,
                 int64_t split_stride, int64_t m, int64_t n, int k, int64_t chunk, T eps, int vec_ok) {
   using Cfg = RowPassCfg<T, KP, KL>;
@@ -83,10 +85,16 @@ row_pass_kernel(const T* __restrict__ A, int64_t lda, const T* __restrict__ H, i
       const int64_t row = row0 + r, col = c0 + cv;
       Pack<T, VN> p;
       if (row < m && vec_ok && col + VN <= c_end) {
-        p = ldpack<T, VN>(A + row * lda + col);
+        if constexpr (std::is_same<TA, T>::value) {
+          p = ldpack<T, VN>(A + row * lda + col);
+        } else {
+          const Pack<TA, VN> pa = ldpack<TA, VN>(A + row * lda + col);
+#pragma unroll
+          for (int j = 0; j < VN; ++j) p.v[j] = static_cast<T>(pa.v[j]);
+        }
       } else {
 #pragma unroll
-        for (int j = 0; j < VN; ++j) p.v[j] = (row < m && col + j < c_end) ? A[row * lda + col + j] : T(0);
+        for (int j = 0; j < VN; ++j) p.v[j] = (row < m && col + j < c_end) ? static_cast<T>(A[row * lda + col + j]) : T(0);
       }
       *reinterpret_cast<Pack<T, VN>*>(As + r * AS + cv) = p;
     }
@@ -168,9 +176,9 @@ struct ColPassCfg {
   static constexpr int CPT = raw >= vmax ? vmax : (raw >= 2 ? 2 : 1);
 };
 
-template <typename T, int KP, bool KL>
+template <typename T, int KP, bool KL, typename TA = T>
 __global__ void __launch_bounds__(kColPassThreads)
-col_pass_kernel(const T* __restrict__ A, int64_t lda, const T* __restrict__ W, int64_t ldw,
+col_pass_kernel(const TA* __restrict__ A, int64_t lda, const T* __restrict__ W, int64_t ldw,
                 const T* __restrict__ H, int64_t ldh, T* __restrict__ out, int64_t ldo,
                 int64_t split_stride, int64_t m, int64_t n, int k, int64_t chunk, T eps, int vec_ok) {
   constexpr int NT = kColPassThreads, BR = kColPassBR, RB = 4;
@@ -215,11 +223,17 @@ col_pass_kernel(const T* __restrict__ A, int64_t lda, const T* __restrict__ W, i
       for (int q = 0; q < RB; ++q) {
         const int64_t row = r0 + r + q;
         if (row < r_end && full) {
-          a[q] = ldpack<T, CPT>(A + row * lda + col0);
+          if constexpr (std::is_same<TA, T>::value) {
+            a[q] = ldpack<T, CPT>(A + row * lda + col0);
+          } else {
+            const Pack<TA, CPT> pa = ldpack<TA, CPT>(A + row * lda + col0);
+#pragma unroll
+            for (int cc = 0; cc < CPT; ++cc) a[q].v[cc] = static_cast<T>(pa.v[cc]);
+          }
         } else {
 #pragma unroll
           for (int cc = 0; cc < CPT; ++cc)
-            a[q].v[cc] = (row < r_end && col0 + cc < n) ? A[row * lda + col0 + cc] : T(0);
+            a[q].v[cc] = (row < r_end && col0 + cc < n) ? static_cast<T>(A[row * lda + col0 + cc]) : T(0);
         }
       }
 #pragma unroll

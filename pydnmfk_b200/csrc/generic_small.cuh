@@ -338,7 +338,7 @@ rowsum_partial_kernel(const T* __restrict__ X, int64_t ldx, int64_t rows, int64_
   const int64_t c_end = (c_begin + cols_per_chunk < cols) ? (c_begin + cols_per_chunk) : cols;
   double acc = 0.0;
   for (int64_t c = c_begin + threadIdx.x; c < c_end; c += 256) {
-    const double v = (double)X[r * ldx + c];
+    const double v = to_f64(X[r * ldx + c]);
     acc += sq ? v * v : v;
   }
   const double s = block_sum<256>(acc, red);
@@ -449,9 +449,9 @@ __global__ void axpby_kernel(T* __restrict__ out, const T* __restrict__ x, const
 // residual: per block partial (||A - W H||^2, ||A||^2) over a [row chunk] x [column block]
 // column-owner layout as col_pass (coalesced A, W rows broadcast from shared memory)
 // ---------------------------------------------------------------------------------------------
-template <typename T, int KP>
+template <typename T, int KP, typename TA = T>
 __global__ void __launch_bounds__(kColPassThreads)
-residual_kernel(const T* __restrict__ A, int64_t lda, const T* __restrict__ W, int64_t ldw,
+residual_kernel(const TA* __restrict__ A, int64_t lda, const T* __restrict__ W, int64_t ldw,
                 const T* __restrict__ H, int64_t ldh, int64_t m, int64_t n, int k, int64_t chunk,
                 double* __restrict__ P, double* __restrict__ col_num, double* __restrict__ col_den) {
   constexpr int NT = kColPassThreads, BR = kColPassBR;
@@ -476,7 +476,7 @@ residual_kernel(const T* __restrict__ A, int64_t lda, const T* __restrict__ W, i
     const int rows_here = (r_end - r0 < BR) ? (int)(r_end - r0) : BR;
     if (c < n) {
       for (int r = 0; r < rows_here; ++r) {
-        const T a = A[(r0 + r) * lda + c];
+        const T a = static_cast<T>(A[(r0 + r) * lda + c]);
         T s = T(0);
 #pragma unroll
         for (int kk = 0; kk < KP; ++kk) s = fma(Ws[r][kk], h[kk], s);

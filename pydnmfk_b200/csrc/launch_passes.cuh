@@ -39,14 +39,14 @@ inline int launch_reduce(const T* P, int64_t split_stride, int splits, int64_t R
   return 0;
 }
 
-// V[m x k] = A H^T  or  (A/(WH+eps)) H^T
-template <typename T, int KP, bool KL>
-int run_row_pass(const T* A, int64_t lda, const T* H, int64_t ldh, const T* W, int64_t ldw, T* V, int64_t ldv,
+// V[m x k] = A H^T  or  (A/(WH+eps)) H^T   (A's elements of type TA are widened to T as they are staged)
+template <typename T, int KP, bool KL, typename TA = T>
+int run_row_pass(const TA* A, int64_t lda, const T* H, int64_t ldh, const T* W, int64_t ldw, T* V, int64_t ldv,
                  int64_t m, int64_t n, int k, T eps, void* ws, int64_t ws_bytes, cudaStream_t st) {
   using Cfg = RowPassCfg<T, KP, KL>;
   const Split sp = row_pass_plan<T, KP, KL>(m, n);
-  const int vec_ok = (((uintptr_t)A % 16) == 0) && (lda % Cfg::VN == 0);
-  auto kern = row_pass_kernel<T, KP, KL>;
+  const int vec_ok = (((uintptr_t)A % (Cfg::VN * sizeof(TA))) == 0) && (lda % Cfg::VN == 0);
+  auto kern = row_pass_kernel<T, KP, KL, TA>;
   static bool attr_set = false;
   if (Cfg::smem_bytes > 48 * 1024 && !attr_set) {
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::smem_bytes);
@@ -68,23 +68,23 @@ int run_row_pass(const T* A, int64_t lda, const T* H, int64_t ldh, const T* W, i
 }
 
 // Y[k x n] = W^T A  or  W^T (A/(WH+eps));  transposed_out: Y^T [n x k]
-template <typename T, int KP, bool KL>
-int run_col_pass(const T* A, int64_t lda, const T* W, int64_t ldw, const T* H, int64_t ldh, T* Y, int64_t ldy,
+template <typename T, int KP, bool KL, typename TA = T>
+int run_col_pass(const TA* A, int64_t lda, const T* W, int64_t ldw, const T* H, int64_t ldh, T* Y, int64_t ldy,
                  int64_t m, int64_t n, int k, T eps, int transposed_out, void* ws, int64_t ws_bytes,
                  cudaStream_t st) {
   constexpr int CPT = ColPassCfg<T, KP, KL>::CPT;
   const Split sp = col_pass_plan<T, KP, KL>(m, n);
-  const int vec_ok = (((uintptr_t)A % (CPT * sizeof(T))) == 0) && (lda % CPT == 0);
+  const int vec_ok = (((uintptr_t)A % (CPT * sizeof(TA))) == 0) && (lda % CPT == 0);
   dim3 grid((unsigned)sp.blocks, (unsigned)sp.splits);
   if (sp.splits == 1 && !transposed_out) {
-    col_pass_kernel<T, KP, KL><<<grid, kColPassThreads, 0, st>>>(A, lda, W, ldw, H, ldh, Y, ldy, 0, m, n, k, sp.chunk, eps, vec_ok);
+    col_pass_kernel<T, KP, KL, TA><<<grid, kColPassThreads, 0, st>>>(A, lda, W, ldw, H, ldh, Y, ldy, 0, m, n, k, sp.chunk, eps, vec_ok);
     DNMF_LAUNCH_CHECK("col_pass_kernel");
     return 0;
   }
   const int64_t need = sp.splits * (int64_t)k * n * (int64_t)sizeof(T);
   if (ws == nullptr || ws_bytes < need) return fail(DNMF_E_WORKSPACE, "col pass needs %lld workspace bytes, got %lld", (long long)need, (long long)ws_bytes);
   T* P = reinterpret_cast<T*>(ws);
-  col_pass_kernel<T, KP, KL><<<grid, kColPassThreads, 0, st>>>(A, lda, W, ldw, H, ldh, P, n, (int64_t)k * n, m, n, k, sp.chunk, eps, vec_ok);
+  col_pass_kernel<T, KP, KL, TA><<<grid, kColPassThreads, 0, st>>>(A, lda, W, ldw, H, ldh, P, n, (int64_t)k * n, m, n, k, sp.chunk, eps, vec_ok);
   DNMF_LAUNCH_CHECK("col_pass_kernel");
   if (transposed_out) return launch_reduce<T>(P, (int64_t)k * n, (int)sp.splits, k, n, Y, 1, ldy, st);
   return launch_reduce<T>(P, (int64_t)k * n, (int)sp.splits, k, n, Y, ldy, 1, st);
@@ -104,36 +104,37 @@ Split col_pass_plan_rt(int kp, bool kl, int64_t m, int64_t n) {
   return sp;
 }
 
-// defined (explicitly instantiated) in inst_row_f32.cu / inst_row_f64.cu / inst_col_f32.cu / inst_col_f64.cu
-template <typename T>
-int row_pass_dispatch(bool kl, const T* A, int64_t lda, const T* H, int64_t ldh, const T* W, int64_t ldw, T* V,
+// defined (explicitly instantiated) in inst_row_f32.cu / inst_row_f64.cu / inst_col_f32.cu / inst_col_f64.cu, and for
+// 16-bit A with fp32 factors in inst_row_a16.cu / inst_col_a16.cu
+template <typename T, typename TA = T>
+int row_pass_dispatch(bool kl, const TA* A, int64_t lda, const T* H, int64_t ldh, const T* W, int64_t ldw, T* V,
                       int64_t ldv, int64_t m, int64_t n, int k, T eps, void* ws, int64_t ws_bytes, cudaStream_t st);
-template <typename T>
-int col_pass_dispatch(bool kl, const T* A, int64_t lda, const T* W, int64_t ldw, const T* H, int64_t ldh, T* Y,
+template <typename T, typename TA = T>
+int col_pass_dispatch(bool kl, const TA* A, int64_t lda, const T* W, int64_t ldw, const T* H, int64_t ldh, T* Y,
                       int64_t ldy, int64_t m, int64_t n, int k, T eps, int transposed_out, void* ws,
                       int64_t ws_bytes, cudaStream_t st);
 
 #ifdef DNMF_INSTANTIATE_ROW
-template <typename T>
-int row_pass_dispatch(bool kl, const T* A, int64_t lda, const T* H, int64_t ldh, const T* W, int64_t ldw, T* V,
+template <typename T, typename TA>
+int row_pass_dispatch(bool kl, const TA* A, int64_t lda, const T* H, int64_t ldh, const T* W, int64_t ldw, T* V,
                       int64_t ldv, int64_t m, int64_t n, int k, T eps, void* ws, int64_t ws_bytes, cudaStream_t st) {
   const int kp = padded_k(k);
   DNMF_DISPATCH_KP(kp, {
-    if (kl) return run_row_pass<T, KP, true>(A, lda, H, ldh, W, ldw, V, ldv, m, n, k, eps, ws, ws_bytes, st);
-    return run_row_pass<T, KP, false>(A, lda, H, ldh, W, ldw, V, ldv, m, n, k, eps, ws, ws_bytes, st);
+    if (kl) return run_row_pass<T, KP, true, TA>(A, lda, H, ldh, W, ldw, V, ldv, m, n, k, eps, ws, ws_bytes, st);
+    return run_row_pass<T, KP, false, TA>(A, lda, H, ldh, W, ldw, V, ldv, m, n, k, eps, ws, ws_bytes, st);
   });
   return 0;
 }
 #endif
 #ifdef DNMF_INSTANTIATE_COL
-template <typename T>
-int col_pass_dispatch(bool kl, const T* A, int64_t lda, const T* W, int64_t ldw, const T* H, int64_t ldh, T* Y,
+template <typename T, typename TA>
+int col_pass_dispatch(bool kl, const TA* A, int64_t lda, const T* W, int64_t ldw, const T* H, int64_t ldh, T* Y,
                       int64_t ldy, int64_t m, int64_t n, int k, T eps, int transposed_out, void* ws,
                       int64_t ws_bytes, cudaStream_t st) {
   const int kp = padded_k(k);
   DNMF_DISPATCH_KP(kp, {
-    if (kl) return run_col_pass<T, KP, true>(A, lda, W, ldw, H, ldh, Y, ldy, m, n, k, eps, transposed_out, ws, ws_bytes, st);
-    return run_col_pass<T, KP, false>(A, lda, W, ldw, H, ldh, Y, ldy, m, n, k, eps, transposed_out, ws, ws_bytes, st);
+    if (kl) return run_col_pass<T, KP, true, TA>(A, lda, W, ldw, H, ldh, Y, ldy, m, n, k, eps, transposed_out, ws, ws_bytes, st);
+    return run_col_pass<T, KP, false, TA>(A, lda, W, ldw, H, ldh, Y, ldy, m, n, k, eps, transposed_out, ws, ws_bytes, st);
   });
   return 0;
 }

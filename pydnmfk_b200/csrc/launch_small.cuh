@@ -51,8 +51,9 @@ template <typename T>
 int col_update_dispatch(int mode, T* H, int64_t ldh, const T* X, int64_t ldx, const T* Y, int64_t ysk, int64_t ysc,
                         const T* G, int k, int64_t n, T p0, int clamp, const double* p0_dev, cudaStream_t st, int splits = 1,
                         int64_t sstride = 0);
-template <typename T>
-int residual_dispatch(const T* A, int64_t lda, const T* W, int64_t ldw, const T* H, int64_t ldh, int64_t m,
+// (TA: element type of A; 16-bit A with fp32 factors is instantiated in inst_col_a16.cu)
+template <typename T, typename TA = T>
+int residual_dispatch(const TA* A, int64_t lda, const T* W, int64_t ldw, const T* H, int64_t ldh, int64_t m,
                       int64_t n, int k, int64_t chunk, unsigned gx, unsigned gy, double* P, double* col_num,
                       double* col_den, cudaStream_t st);
 template <typename T>
@@ -103,13 +104,13 @@ int col_update_dispatch(int mode, T* H, int64_t ldh, const T* X, int64_t ldx, co
   return 0;
 }
 
-template <typename T>
-int residual_dispatch(const T* A, int64_t lda, const T* W, int64_t ldw, const T* H, int64_t ldh, int64_t m,
+template <typename T, typename TA>
+int residual_dispatch(const TA* A, int64_t lda, const T* W, int64_t ldw, const T* H, int64_t ldh, int64_t m,
                       int64_t n, int k, int64_t chunk, unsigned gx, unsigned gy, double* P, double* col_num,
                       double* col_den, cudaStream_t st) {
   const int kp = padded_k(k);
   dim3 grid(gx, gy);
-  DNMF_DISPATCH_KP(kp, (residual_kernel<T, KP><<<grid, kColPassThreads, 0, st>>>(A, lda, W, ldw, H, ldh, m, n, k, chunk, P, col_num, col_den)));
+  DNMF_DISPATCH_KP(kp, (residual_kernel<T, KP, TA><<<grid, kColPassThreads, 0, st>>>(A, lda, W, ldw, H, ldh, m, n, k, chunk, P, col_num, col_den)));
   DNMF_LAUNCH_CHECK("residual_kernel");
   return 0;
 }

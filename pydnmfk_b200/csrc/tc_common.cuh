@@ -507,7 +507,8 @@ struct TcPlan {
   int64_t bcat_bytes, partial_bytes;
 };
 int tc_padded_k(int k);
-TcPlan tc_plan(int64_t x_len, int64_t r_len, int k);
+// bk: reduced-dimension elements per tile (TC_BK fp32, TC16_BK for a 16-bit A)
+TcPlan tc_plan(int64_t x_len, int64_t r_len, int k, int bk = TC_BK);
 int tc_hi_mode();                       // 0: the tensor core truncates fp32 -> tf32, 1: rounds to nearest (calibrated)
 unsigned long long* tc_prof_ptr();      // debug buffer or nullptr
 int tc_dbg_flags();

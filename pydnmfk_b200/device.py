@@ -14,6 +14,14 @@ import torch
 from . import _lib as L
 
 _DT = {torch.float32: L.F32, torch.float64: L.F64}
+# dtype codes of the entry points that read the data shard A, which may also be stored in 16 bits
+_DT_A = {**_DT, torch.float16: L.A_F16, torch.bfloat16: L.A_BF16}
+_A16 = (torch.float16, torch.bfloat16)
+
+
+def out_dtype(a_dtype):
+    """dtype of the factors and of every result computed from a shard stored as ``a_dtype`` (float32 for 16-bit A)."""
+    return torch.float32 if a_dtype in _A16 else a_dtype
 
 
 def require_cuda():
@@ -57,6 +65,26 @@ def to_device_view(x, dtype=None):
         t = torch.from_numpy(a.copy() if not a.flags.writeable else a).cuda()
     if dtype is not None and t.dtype != dtype:
         t = t.to(dtype)
+    return t
+
+
+def to_device_a16(x, dtype):
+    """The data shard rounded to nearest even into ``dtype`` (torch.float16 / torch.bfloat16) as a contiguous CUDA tensor.
+    Host data is rounded on the host by torch's CPU cast (multi-threaded; the same nearest-even result as numpy's
+    ``astype(np.float16)``), so only 2 bytes per element cross the bus; a CUDA float32 tensor is rounded on the device; a CUDA tensor already in ``dtype`` is used as it
+    is.  Raises ValueError when an entry overflows to inf (|a| > 65504 in float16)."""
+    require_cuda()
+    if isinstance(x, torch.Tensor) and x.is_cuda:
+        t = x.to(dtype).contiguous()
+    else:
+        h = x if isinstance(x, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(x))
+        h = h.contiguous().to(dtype)
+        t = h.to(torch.device('cuda', torch.cuda.current_device()))
+    if t.numel() > 0:
+        lo, hi = torch.aminmax(t)
+        if bool(torch.isinf(lo) | torch.isinf(hi)):
+            raise ValueError('params.a_storage=%r: the data has entries beyond the %s range (largest finite magnitude %g)'
+                             % (str(dtype).replace('torch.', ''), dtype, torch.finfo(dtype).max))
     return t
 
 
@@ -128,8 +156,8 @@ class DeviceOps:
         """V = A @ H.T   (dist_nmf.py:198, :730)"""
         m, n = A.shape
         k = H.shape[0]
-        dt = _DT[A.dtype]
-        V = out if out is not None else self.empty((m, k), A.dtype)
+        dt = _DT_A[A.dtype]
+        V = out if out is not None else self.empty((m, k), out_dtype(A.dtype))
         ws, wsb = self._ws_for(L.OP_AH, m, n, k, dt)
         ev = self._t0('ah')
         L.call('dnmf_ah', A.data_ptr(), _ld(A), H.data_ptr(), _ld(H), V.data_ptr(), _ld(V), m, n, k, dt,
@@ -141,8 +169,8 @@ class DeviceOps:
         """Y = W.T @ A (k x n), or Y.T (n x k) when transposed_out   (dist_nmf.py:166, :749)"""
         m, n = A.shape
         k = W.shape[1]
-        dt = _DT[A.dtype]
-        Y = out if out is not None else self.empty((n, k) if transposed_out else (k, n), A.dtype)
+        dt = _DT_A[A.dtype]
+        Y = out if out is not None else self.empty((n, k) if transposed_out else (k, n), out_dtype(A.dtype))
         ws, wsb = self._ws_for(L.OP_WTA, m, n, k, dt)
         ev = self._t0('wta')
         L.call('dnmf_wta', A.data_ptr(), _ld(A), W.data_ptr(), _ld(W), Y.data_ptr(), _ld(Y), m, n, k,
@@ -154,8 +182,8 @@ class DeviceOps:
         """V = (A / (W @ H + eps)) @ H.T without materialising W @ H   (dist_nmf.py:338-339, :806,:810)"""
         m, n = A.shape
         k = H.shape[0]
-        dt = _DT[A.dtype]
-        V = out if out is not None else self.empty((m, k), A.dtype)
+        dt = _DT_A[A.dtype]
+        V = out if out is not None else self.empty((m, k), out_dtype(A.dtype))
         ws, wsb = self._ws_for(L.OP_KL_UHT, m, n, k, dt)
         ev = self._t0('kl_uht')
         L.call('dnmf_kl_uht', A.data_ptr(), _ld(A), W.data_ptr(), _ld(W), H.data_ptr(), _ld(H), V.data_ptr(),
@@ -167,8 +195,8 @@ class DeviceOps:
         """Y = W.T @ (A / (W @ H + eps))   (dist_nmf.py:312-313, :806,:808)"""
         m, n = A.shape
         k = H.shape[0]
-        dt = _DT[A.dtype]
-        Y = out if out is not None else self.empty((n, k) if transposed_out else (k, n), A.dtype)
+        dt = _DT_A[A.dtype]
+        Y = out if out is not None else self.empty((n, k) if transposed_out else (k, n), out_dtype(A.dtype))
         ws, wsb = self._ws_for(L.OP_KL_WTU, m, n, k, dt)
         ev = self._t0('kl_wtu')
         L.call('dnmf_kl_wtu', A.data_ptr(), _ld(A), W.data_ptr(), _ld(W), H.data_ptr(), _ld(H), Y.data_ptr(),
@@ -181,10 +209,10 @@ class DeviceOps:
     def _pass_partials(self, name, timer, op, A, k, *args):
         """Run a `_p` pass; returns the int64[4] view (host array kept alive by the caller) or None when the call is
         not served by the tcgen05 path (the caller then uses the plain op)."""
-        if not fused_epilogue_enabled() or A.dtype != torch.float32:
+        if not fused_epilogue_enabled() or out_dtype(A.dtype) != torch.float32:
             return None
         m, n = A.shape
-        dt = _DT[A.dtype]
+        dt = _DT_A[A.dtype]
         ws, wsb = self._ws_for(op, m, n, k, dt)
         view = (C.c_int64 * 4)()
         ev = self._t0(timer)
@@ -302,8 +330,8 @@ class DeviceOps:
         """sum(X**2) as a float64 device scalar (shape [1])."""
         r, c = X.shape
         out = self.empty((1,), torch.float64)
-        ws, wsb = self._ws_for(L.OP_SUMS, r, c, min(c, L.MAX_K), _DT[X.dtype])
-        L.call('dnmf_sqnorm', X.data_ptr(), _ld(X), r, c, out.data_ptr(), _DT[X.dtype], ws, wsb, self._stream())
+        ws, wsb = self._ws_for(L.OP_SUMS, r, c, min(c, L.MAX_K), _DT[out_dtype(X.dtype)])
+        L.call('dnmf_sqnorm', X.data_ptr(), _ld(X), r, c, out.data_ptr(), _DT_A[X.dtype], ws, wsb, self._stream())
         return out
 
     def normalize(self, W, H, s, eps):
@@ -330,7 +358,7 @@ class DeviceOps:
         """[||A - W H||_F^2, ||A||_F^2] as a float64 device tensor of shape [2]."""
         m, n = A.shape
         k = W.shape[1]
-        dt = _DT[A.dtype]
+        dt = _DT_A[A.dtype]
         out = self.empty((2,), torch.float64)
         ws, wsb = self._ws_for(L.OP_RESIDUAL, m, n, k, dt)
         L.call('dnmf_residual_sqnorm', A.data_ptr(), _ld(A), W.data_ptr(), _ld(W), H.data_ptr(), _ld(H), m, n, k,
@@ -341,8 +369,8 @@ class DeviceOps:
         """(A @ H.T, [||A - W H||_F^2, ||A||_F^2]) in one pass over A (dist_nmf.py:1023-1024)."""
         m, n = A.shape
         k = W.shape[1]
-        dt = _DT[A.dtype]
-        V = self.empty((m, k), A.dtype)
+        dt = _DT_A[A.dtype]
+        V = self.empty((m, k), out_dtype(A.dtype))
         out = self.empty((2,), torch.float64)
         ws, wsb = self._ws_for(L.OP_AH_RESIDUAL, m, n, k, dt)
         ev = self._t0('ah_res')
@@ -357,7 +385,7 @@ class DeviceOps:
         num = self.empty((n,), torch.float64)
         den = self.empty((n,), torch.float64)
         L.call('dnmf_column_err', A.data_ptr(), _ld(A), W.data_ptr(), _ld(W), H.data_ptr(), _ld(H), m, n, k,
-               num.data_ptr(), den.data_ptr(), _DT[A.dtype], self._stream())
+               num.data_ptr(), den.data_ptr(), _DT_A[A.dtype], self._stream())
         return num, den
 
     # ---- HALS / BCD ---------------------------------------------------------------------------
@@ -444,7 +472,7 @@ class DeviceOps:
         m, n = A.shape
         rows = self.empty((m,), torch.int64)
         cols = self.empty((n,), torch.int64)
-        L.call('dnmf_nnz_counts', A.data_ptr(), _ld(A), m, n, rows.data_ptr(), cols.data_ptr(), _DT[A.dtype],
+        L.call('dnmf_nnz_counts', A.data_ptr(), _ld(A), m, n, rows.data_ptr(), cols.data_ptr(), _DT_A[A.dtype],
                self._stream())
         return rows, cols
 
@@ -452,7 +480,7 @@ class DeviceOps:
         mr, nc = row_idx.numel(), col_idx.numel()
         out = self.empty((mr, nc), A.dtype)
         L.call('dnmf_compact', A.data_ptr(), _ld(A), row_idx.data_ptr(), mr, col_idx.data_ptr(), nc, out.data_ptr(),
-               max(nc, 1), _DT[A.dtype], self._stream())
+               max(nc, 1), _DT_A[A.dtype], self._stream())
         return out
 
     def scatter_rows(self, X, row_idx, total_rows):

@@ -52,7 +52,9 @@ class _AlgBase:
         self._numpy_io = not isinstance(A_ij, torch.Tensor)
         self._np_dtype = A_ij.dtype if self._numpy_io else None
         A = D.to_device(A_ij)
-        return A, D.to_device(W, A.dtype), D.to_device(H, A.dtype)
+        # factor dtype: the data dtype, or float32 when the shard is stored in 16 bits (PyNMF's params.a_storage)
+        self.fdtype = D.out_dtype(A.dtype)
+        return A, D.to_device(W, self.fdtype), D.to_device(H, self.fdtype)
 
     def _out(self, W, H):
         if self._numpy_io:
@@ -92,7 +94,7 @@ class _AlgBase:
         m = type('Monitor', (), {})()
         m.hist = torch.zeros((slots, 2), dtype=torch.float64, device=dev)
         m.counter = torch.zeros(1, dtype=torch.int64, device=dev)
-        m.wtw = torch.zeros((self.k, self.k), dtype=self.A_ij.dtype, device=dev)   # persistent: captured graphs keep its address
+        m.wtw = torch.zeros((self.k, self.k), dtype=self.fdtype, device=dev)   # persistent: captured graphs keep its address
         m.have_wtw = False
         m.anorm2 = self._sqnorm_dev(self.A_ij)            # global ||A||^2, float64 device scalar
         m.w_sharded = (self.p > 1) and not (self.p_r == 1)   # <W, A H^T> is a sum over the ranks that own W rows
@@ -225,7 +227,7 @@ class nmf_algorithms_2D(_AlgBase):
     @comm_timing()
     def global_gram(self, A):
         """A^T A summed over all ranks (dist_nmf.py:94-116); ``A`` is W_ij or H_ij.T."""
-        A = D.to_device_view(A, self.A_ij.dtype)
+        A = D.to_device_view(A, self.fdtype)
         G = self.ops.gram(A, trans=False) if A.is_contiguous() else self.ops.gram(A.t().contiguous(), trans=True)
         return self.comm1.allreduce_(G)
 
@@ -265,7 +267,7 @@ class nmf_algorithms_2D(_AlgBase):
     @comm_timing()
     def AH_glob(self, H_ij=None):
         """A H^T: allgather(row comm) -> skinny GEMM -> reduce-scatter(column comm) (dist_nmf.py:174-205)."""
-        return self._AH(self.H_ij if H_ij is None else D.to_device(H_ij, self.A_ij.dtype))
+        return self._AH(self.H_ij if H_ij is None else D.to_device(H_ij, self.fdtype))
 
     @comm_timing()
     def ATW_glob(self):
@@ -365,7 +367,7 @@ class nmf_algorithms_2D(_AlgBase):
     @comm_timing()
     def globalSqNorm(self, comm, X):
         """Global squared Frobenius norm (dist_nmf.py:474-480)."""
-        return self._sqnorm_global(D.to_device(X, self.A_ij.dtype))
+        return self._sqnorm_global(D.to_device(X, self.fdtype))
 
     def _colsum_W(self, W, force):
         return self.comm1.allreduce_(self.ops.colsum(W))
@@ -424,7 +426,7 @@ class nmf_algorithms_1D(_AlgBase):
     @comm_timing()
     def global_gram(self, A, p=1):
         """A^T A, all-reduced iff p != 1 (dist_nmf.py:662-685)."""
-        A = D.to_device_view(A, self.A_ij.dtype)
+        A = D.to_device_view(A, self.fdtype)
         G = self.ops.gram(A, trans=False) if A.is_contiguous() else self.ops.gram(A.t().contiguous(), trans=True)
         return self.comm1.allreduce_(G) if p != 1 else G
 
@@ -434,7 +436,7 @@ class nmf_algorithms_1D(_AlgBase):
         ``global_mm(A_ij, H_j.T, p_c)`` and ``global_mm(W_i.T, A_ij, p_r)``, run as one pass over the resident shard; any
         other pair of matrices goes through the same skinny contraction in column chunks of the factor width the kernels
         support (the left operand is streamed once per chunk)."""
-        dt = self.A_ij.dtype
+        dt = self.fdtype
         if A is self.A_ij or A is self._A_orig:
             Bt = D.to_device_view(B, dt).t().contiguous()
             if Bt.shape[0] <= D.L.MAX_K:
@@ -450,7 +452,7 @@ class nmf_algorithms_1D(_AlgBase):
     def _mm_chunked(self, A, B):
         """A [r x c] @ B [c x s] for any s: out[:, j0:j1] = A (B[:, j0:j1]^T)^T in chunks of <= MAX_K columns."""
         r, s_cols = A.shape[0], B.shape[1]
-        out = self.ops.empty((r, s_cols), A.dtype)
+        out = self.ops.empty((r, s_cols), D.out_dtype(A.dtype))
         step = D.L.MAX_K
         for j0 in range(0, s_cols, step):
             j1 = min(s_cols, j0 + step)
@@ -521,7 +523,7 @@ class nmf_algorithms_1D(_AlgBase):
     @comm_timing()
     def sum_along_axis(self, X, p=1, axis=0):
         """dist_nmf.py:775-801."""
-        X = D.to_device(X, self.A_ij.dtype)
+        X = D.to_device(X, self.fdtype)
         s = self.ops.colsum(X) if axis == 0 else self.ops.rowsum(X)
         return self.comm1.allreduce_(s) if p != 1 else s
 
@@ -620,7 +622,7 @@ class nmf_algorithms_1D(_AlgBase):
     @comm_timing()
     def globalSqNorm(self, X, p=-1):
         """dist_nmf.py:939-949."""
-        sq = self.ops.sqnorm(D.to_device(X, self.A_ij.dtype))
+        sq = self.ops.sqnorm(D.to_device(X, self.fdtype))
         if p != 1:
             sq = self.comm1.allreduce_(sq)
         return float(sq.item())

@@ -22,6 +22,31 @@ from .dist_comm import MPI
 from .graphs import StepGraphs, graphs_enabled
 
 
+_A_STORAGE = {'float16': torch.float16, 'bfloat16': torch.bfloat16}
+
+
+def a_storage_dtype(a_storage, A):
+    """The torch dtype the data shard ``A`` is stored in on the device for ``params.a_storage``, or None (``a_storage`` None:
+    the data dtype, nothing changes).  With 'float16' / 'bfloat16' only the shard is held in 16 bits -- the fit is the
+    float32 fit of the rounded matrix -- so the data must be float32, or a CUDA tensor already in that 16-bit format.
+    Raises ValueError otherwise.  Needs no device."""
+    if a_storage is None:
+        return None
+    if a_storage not in _A_STORAGE:
+        raise ValueError("params.a_storage must be None, 'float16' or 'bfloat16', not %r" % (a_storage,))
+    want = _A_STORAGE[a_storage]
+    if isinstance(A, torch.Tensor):
+        if A.dtype == torch.float32 or (A.dtype == want and A.is_cuda):
+            return want
+        got = str(A.dtype).replace('torch.', '') + ('' if A.is_cuda else ' (host tensor)')
+    else:
+        got = str(np.asarray(A).dtype)
+        if got == 'float32':
+            return want
+    raise ValueError('params.a_storage=%r needs float32 data (or a CUDA tensor already in %s), got %s'
+                     % (a_storage, a_storage, got))
+
+
 def draw_rand_factors(topo, p_c, rank, a_shape, factor_shape, k, dt):
     """Host draws of the 'rand' initialisation in the reference's exact order (pyDNMF.py:110-129):
     2-D: W_ij = rand(m_loc, k) then H_ij = rand(k, n_loc) on every rank; 1-D row grid: W_i on every
@@ -45,16 +70,29 @@ class PyNMF():
     Parameters (identical to the reference, pyDNMF.py:9-52): ``A_ij`` local shard (numpy array or
     CUDA tensor), ``factors`` optional ``[W, H]`` shards, ``params`` attribute bag with ``init,
     comm1, comm, k, p_r, p_c (or grid), row_comm, col_comm, verbose`` and optional ``itr, norm,
-    method, prune, W_update``.
+    method, prune, W_update``, ``a_storage``.
+
+    ``params.a_storage`` = 'float16' / 'bfloat16' holds only the data shard in 16 bits on the device (half the memory and
+    half the bytes each pass streams); W, H, every update and every reduction stay float32.  The fit is then the float32
+    fit of the rounded matrix (round to nearest even): ``recon_err`` is relative to the rounded matrix, prune masks come
+    from it (an entry that underflows to 0 is a zero), W and H come back as float32 (float64 after un-pruning).  Float32
+    data only; 'float16' raises ValueError when an entry overflows (|a| > 65504); ``init='nnsvd'`` is not supported.
     """
 
     @comm_timing()
     def __init__(self, A_ij, factors=None, save_factors=False, params=None):
         self.params = params
         self._numpy_in = not isinstance(A_ij, torch.Tensor)
-        self._np_dtype = np.dtype(A_ij.dtype) if self._numpy_in else np.dtype(str(A_ij.dtype).replace('torch.', ''))
+        self._a_dtype = a_storage_dtype(getattr(params, 'a_storage', None), A_ij)
+        if self._a_dtype is not None:
+            self._np_dtype = np.dtype(np.float32)                   # factors, eps and recon_err stay float32
+        else:
+            self._np_dtype = np.dtype(A_ij.dtype) if self._numpy_in else np.dtype(str(A_ij.dtype).replace('torch.', ''))
         self.m_loc, self.n_loc = A_ij.shape
         self.init = self.params.init if self.params.init else 'rand'
+        if self._a_dtype is not None and self.init == 'nnsvd':
+            raise ValueError("params.a_storage does not support init='nnsvd' (DistSVD deflates a copy of A in the data "
+                             "dtype); use init='rand' or given factors")
         if "grid" in vars(self.params) and self.params.grid:
             self.p_r, self.p_c, self.k = self.params.grid[0], self.params.grid[1], self.params.k
         else:
@@ -85,7 +123,10 @@ class PyNMF():
         # the shard goes to HBM once and stays there.  From page-locked host memory the copy runs asynchronously while
         # the host draws the initial factors (the RNG replay below is ~0.1 s at 65536 x 32); the constructor waits for it
         # before returning, so the caller's buffer is never read after this call
-        self.A_ij = D.to_device(A_ij, self._tdtype, non_blocking=True)
+        if self._a_dtype is not None:
+            self.A_ij = D.to_device_a16(A_ij, self._a_dtype)
+        else:
+            self.A_ij = D.to_device(A_ij, self._tdtype, non_blocking=True)
         self.data_op = data_operations(self.A_ij, self.params)
         self.params = self.data_op.params
         if factors is not None:
@@ -147,7 +188,9 @@ class PyNMF():
     def _resident_ok(self):
         """Whole-fit on-chip path (dnmf_mu_fit_resident): single-process grid, MU, shard + factors fit in one SM."""
         W, H = self._get_factors()
-        return (self.comm1.size == 1 and self.method.lower() == 'mu' and self.norm.lower() in ('fro', 'kl')
+        # (the on-chip kernel reads A in the factor dtype: a 16-bit shard takes the per-kernel path)
+        return (self._a_dtype is None and self.comm1.size == 1 and self.method.lower() == 'mu'
+                and self.norm.lower() in ('fro', 'kl')
                 and var_init(self.params, 'resident_fit', True) and self.itr >= 1 and W.shape[0] > 0 and H.shape[1] > 0
                 and self.ops.resident_fit_fits(W.shape[0], H.shape[1], self.k, self.norm, self._tdtype))
 

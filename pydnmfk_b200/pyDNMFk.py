@@ -30,6 +30,9 @@ class sample():
 
     @comm_timing()
     def __init__(self, data, noise_var, method, seed=None):
+        if isinstance(data, torch.Tensor) and data.dtype in (torch.float16, torch.bfloat16):
+            raise ValueError('sample: a 16-bit data shard (params.a_storage) is not supported: the perturbed matrix would '
+                             'need its own rounding rule; perturb the float32 data instead')
         self.X = data
         self.noise_var = noise_var
         self.seed = seed
@@ -78,6 +81,9 @@ class PyNMFk():
 
     @comm_timing()
     def __init__(self, A_ij, factors=None, params=None):
+        if getattr(params, 'a_storage', None) is not None:
+            raise ValueError('params.a_storage is not supported by PyNMFk: the perturbed ensemble would need its own '
+                             'rounding rule; fit the rounded matrix in float32 instead')
         self.A_ij = A_ij
         self.local_m, self.local_n = self.A_ij.shape
         self.params = params
