@@ -85,13 +85,6 @@ int dnmf_device_info(int* sm_count, int* cc_major, int* cc_minor);
 int dnmf_set_force_generic(int on);
 /* smallest shard (m*n elements) routed to the tcgen05 path; default 2^20, tests lower it */
 int dnmf_set_tc_min_elems(int64_t elems);
-/* 1: dnmf_residual_sqnorm uses the tcgen05 pipeline (fp32, k <= 32) instead of the CUDA-core kernel; default 0
- * (or the DNMF_TC_RESIDUAL environment variable) */
-int dnmf_set_tc_residual(int on);
-/* debug: timing-ablation bits of the tcgen05 kernels (tools/prof_tc.py); non-zero values give WRONG results */
-int dnmf_set_tc_debug(int flags);
-/* debug/profiling: device buffer of [n_sm][16] uint64 cycle counters filled by the tcgen05 kernels (NULL = off) */
-int dnmf_set_tc_profile(void* device_buf);
 
 int64_t dnmf_workspace_bytes(int op, int64_t m, int64_t n, int64_t k, int dtype);
 

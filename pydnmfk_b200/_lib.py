@@ -29,9 +29,6 @@ SIGNATURES = {
     'dnmf_device_info': (i32, [C.POINTER(i32)] * 3),
     'dnmf_set_force_generic': (i32, [i32]),
     'dnmf_set_tc_min_elems': (i32, [i64]),
-    'dnmf_set_tc_profile': (i32, [vp]),
-    'dnmf_set_tc_debug': (i32, [i32]),
-    'dnmf_set_tc_residual': (i32, [i32]),
     'dnmf_workspace_bytes': (i64, [i32, i64, i64, i64, i32]),
     'dnmf_ah': (i32, [vp, i64, vp, i64, vp, i64, i64, i64, i64, i32, i32, vp, i64, vp]),
     'dnmf_wta': (i32, [vp, i64, vp, i64, vp, i64, i64, i64, i64, i32, i32, i32, vp, i64, vp]),
@@ -122,7 +119,7 @@ SIGNATURES = {
 }
 
 _NO_STATUS = {'dnmf_trace_terms_workspace_bytes', 'dnmf_xchg_bytes', 'dnmf_pass_count', 'dnmf_version', 'dnmf_last_error', 'dnmf_last_path', 'dnmf_launch_count', 'dnmf_workspace_bytes',
-              'dnmf_set_force_generic', 'dnmf_set_tc_min_elems', 'dnmf_set_tc_profile', 'dnmf_set_tc_debug', 'dnmf_set_tc_residual', 'dnmf_colsum_workspace_bytes',
+              'dnmf_set_force_generic', 'dnmf_set_tc_min_elems', 'dnmf_colsum_workspace_bytes',
               'dnmf_matvec_workspace_bytes', 'dnmf_mu_fit_resident_smem_bytes', 'dnmf_mu_fit_resident_cluster_size'}
 
 

@@ -66,10 +66,6 @@ int64_t dnmf_workspace_bytes(int op, int64_t m, int64_t n, int64_t k, int dtype)
     case DNMF_OP_RESIDUAL: {
       const ResPlan r = residual_plan(m, n);
       bytes = r.col_blocks * r.chunks * 2 * (int64_t)sizeof(double);
-      if (tc_residual_enabled() && dtype == DNMF_F32 && k <= 32) {
-        const int64_t t = tc_residual_workspace_bytes(m, n);
-        if (t > bytes) bytes = t;
-      }
       break;
     }
     case DNMF_OP_AH_RESIDUAL: {
@@ -542,17 +538,6 @@ int dnmf_residual_sqnorm(const void* A, int64_t lda, const void* W, int64_t ldw,
   if (m == 0 || n == 0) {
     cudaError_t e = cudaMemsetAsync(out, 0, 2 * sizeof(double), st);
     return e == cudaSuccess ? 0 : cuda_fail(e, "dnmf_residual_sqnorm memset");
-  }
-  if (tc_residual_enabled() && k <= 32 && tc_eligible(DNMF_OP_KL_UHT, A, lda, m, n, k, dtype)) {
-    double* pairs = nullptr;
-    int64_t n_pairs = 0;
-    if (int rc = tc_residual_run((const float*)A, lda, (const float*)W, ldw, (const float*)H, ldh, m, n, (int)k, ws, ws_bytes,
-                                 &pairs, &n_pairs, st))
-      return rc;
-    tls().last_path = 1;
-    sum_pairs_kernel<<<1, 256, 0, st>>>(pairs, n_pairs, out);
-    DNMF_LAUNCH_CHECK("sum_pairs_kernel");
-    return 0;
   }
   const ResPlan rp = residual_plan(m, n);
   const int64_t nb = rp.col_blocks * rp.chunks;

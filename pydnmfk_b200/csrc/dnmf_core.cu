@@ -83,21 +83,6 @@ int dnmf_set_force_generic(int on) {
   return 0;
 }
 
-int dnmf_set_tc_profile(void* buf) {
-  tc_set_profile(buf);
-  return 0;
-}
-
-int dnmf_set_tc_residual(int on) {
-  tc_set_residual(on);
-  return 0;
-}
-
-int dnmf_set_tc_debug(int flags) {
-  tc_set_debug(flags);
-  return 0;
-}
-
 int dnmf_set_tc_min_elems(int64_t elems) {
   tc_set_min_elems(elems);
   return 0;

@@ -30,7 +30,8 @@ constexpr int TC_CHUNK = 4;      // K-tiles accumulated in TMEM before the drain
 
 // Three decoupled rings:
 //   A ring   (shared memory, SA slots x 16 KB): TMA -> splitter warps; freed as soon as the tile is in registers
-//   B ring   (shared memory, SB slots x 2K*128 B): TMA -> tensor core (B operand); freed by tcgen05.commit
+//   B ring   (shared memory, SB slots x 2K*128 B): TMA -> tensor core (B operand); freed by a splitter warp once the
+//            tile's MMAs have completed (see umma_tile_ts)
 //   operand ring (TENSOR memory, NT slots x 64 columns): raw A (= A_hi for the tensor core) and A_lo, written by the
 //            splitters with tcgen05.st, read by tcgen05.mma as the A operand; freed by tcgen05.commit
 // plus NBUF accumulator buffers of 2K TMEM columns.  The tensor core therefore reads only B from shared memory.
@@ -71,12 +72,9 @@ template <int K, int MODE>
 __global__ void __launch_bounds__(TcCfg<K>::THREADS, 1)
 tc_pass_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
                float* __restrict__ P, int64_t split_stride, int64_t x_len, int x_blocks, int kt_total,
-               int kt_per_split, int num_units, int hi_mode, int dbg_arg, unsigned long long* __restrict__ prof_arg) {
-  TC_LAB_ARGS(dbg_arg, prof_arg)
+               int kt_per_split, int num_units) {
   using Cfg = TcCfg<K>;
   constexpr int SA = Cfg::SA, SB = Cfg::SB, NT = Cfg::NT, NBUF = Cfg::NBUF, N2 = Cfg::N2;
-  // dbg (DNMF_TC_DBG, timing experiments only, results become wrong): 1 = splitter skips its work, 4 = skip the
-  // A_lo MMAs
   constexpr int chunk = TC_CHUNK;
   extern __shared__ uint8_t smem_raw[];
   const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
@@ -119,32 +117,18 @@ tc_pass_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     if (lane == 0) {
       int s = 0;
       uint32_t ph = 0;
-      long long tprev = clock64(), t_wait = 0, t_issue = 0, t0 = tprev;
-      // L2 prefetch cursor, pf tiles ahead of the ring's loads
-      const int pf = tc_pf_dist(dbg);
-      TileCursor pc;
-      pc.init(blockIdx.x, gridDim.x, x_blocks, kt_total, kt_per_split, num_units);
-      for (int i = 0; i < pf && pc.valid(); ++i) pc.next();
       for (int unit = blockIdx.x; unit < num_units; unit += gridDim.x) {
         const int xb = unit % x_blocks, sp = unit / x_blocks;
         const int kt0 = sp * kt_per_split;
         const int kt1 = min(kt_total, kt0 + kt_per_split);
         for (int kt = kt0; kt < kt1; ++kt) {
           mbar_wait(a_free(s), ph ^ 1u);
-          TC_T(t_wait);
           mbar_expect_tx(a_full(s), Cfg::A_BYTES);
           if (MODE == 0) tma_load_2d(sA0 + s * Cfg::A_BYTES, &tmA, a_full(s), kt * TC_BK, xb * TC_BM);
           else tma_load_2d(sA0 + s * Cfg::A_BYTES, &tmA, a_full(s), xb * TC_BM, kt * TC_BK);
-          if (pf > 0 && pc.valid()) {
-            if (MODE == 0) tma_prefetch_2d(&tmA, pc.kt * TC_BK, pc.xb() * TC_BM);
-            else tma_prefetch_2d(&tmA, pc.xb() * TC_BM, pc.kt * TC_BK);
-            pc.next();
-          }
           if (++s == SA) { s = 0; ph ^= 1u; }
-          TC_T(t_issue);
         }
       }
-      if (prof) { prof[blockIdx.x * 16 + 0] = t_wait; prof[blockIdx.x * 16 + 1] = t_issue; prof[blockIdx.x * 16 + 15] = clock64() - t0; }
     }
   } else if (warp == 10) {
     // ===================== B producer (TMA) =====================
@@ -157,7 +141,6 @@ tc_pass_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         const int kt1 = min(kt_total, kt0 + kt_per_split);
         for (int kt = kt0; kt < kt1; ++kt) {
           mbar_wait(b_free(s), ph ^ 1u);
-          if (dbg & 0x10000) { mbar_arrive(b_full(s)); if (++s == SB) { s = 0; ph ^= 1u; } continue; }    // ablation: no B traffic
           mbar_expect_tx(b_full(s), Cfg::B_BYTES);
           tma_load_2d(sB0 + s * Cfg::B_BYTES, &tmB, b_full(s), kt * TC_BK, 0);
           if (++s == SB) { s = 0; ph ^= 1u; }
@@ -172,7 +155,6 @@ tc_pass_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
       constexpr uint32_t idesc_half = make_idesc(K, 0);
       int sb = 0, ts = 0, buf = 0;
       uint32_t pb = 0, pt = 0, accphase = 0;
-      long long tprev = clock64(), t_acce = 0, t_tfull = 0, t_bfull = 0, t_mma = 0, t_commit = 0;
       for (int unit = blockIdx.x; unit < num_units; unit += gridDim.x) {
         const int sp = unit / x_blocks;
         const int kt0 = sp * kt_per_split;
@@ -182,11 +164,8 @@ tc_pass_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
           if (in_chunk == 0) {                      // new accumulation chunk: wait for the drain warps
             mbar_wait(acce_bar(buf), accphase ^ 1u);
           }
-          TC_T(t_acce);
           mbar_wait(t_full(ts), pt);
-          TC_T(t_tfull);
           mbar_wait(b_full(sb), pb);
-          TC_T(t_bfull);
           tc_fence_after();
           const uint32_t d_tmem = tmem_base + (uint32_t)(buf * N2);
           const uint32_t a_raw = tmem_base + (uint32_t)(Cfg::OP_COL0 + ts * 64);
@@ -194,20 +173,14 @@ tc_pass_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
           const bool chunk_end = (in_chunk == chunk - 1) || (kt == kt1 - 1);
           // cols [0,K): Ah*Bh (large term, alone in its accumulator);  cols [K,2K): Ah*Bl + Al*Bh (small terms)
           umma_tile_ts<K>(d_tmem, a_raw, make_smem_desc(sB, 16, 1024), in_chunk > 0 ? 1u : 0u, idesc_full, idesc_half,
-                          t_free(ts), TC_SOFT_FREE ? 0u : b_free(sb), accf_bar(buf), chunk_end ? 1u : 0u, (dbg & 4) ? 1u : 0u);
-          TC_T(t_mma);
+                          t_free(ts), accf_bar(buf), chunk_end ? 1u : 0u);
           if (++ts == NT) { ts = 0; pt ^= 1u; }
           if (++sb == SB) { sb = 0; pb ^= 1u; }
           if (chunk_end) {
             if (++buf == NBUF) { buf = 0; accphase ^= 1u; }
           }
-          TC_T(t_commit);
           __syncwarp();
         }
-      }
-      if (prof && lane == 0) {
-        prof[blockIdx.x * 16 + 2] = t_acce; prof[blockIdx.x * 16 + 3] = t_tfull; prof[blockIdx.x * 16 + 4] = t_bfull;
-        prof[blockIdx.x * 16 + 5] = t_mma; prof[blockIdx.x * 16 + 6] = t_commit;
       }
     }
   } else if (warp < 6 || (warp >= 11 && warp < 15)) {
@@ -218,29 +191,19 @@ tc_pass_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     const int r = q * 32 + lane;
     const int group = (warp >= 11) ? 1 : 0;
     int tile = 0;
-    long long tprev = clock64(), t_afull = 0, t_load = 0, t_tfree = 0, t_store = 0;
     for (int unit = blockIdx.x; unit < num_units; unit += gridDim.x) {
       const int sp = unit / x_blocks;
       const int kt0 = sp * kt_per_split;
       const int kt1 = min(kt_total, kt0 + kt_per_split);
-#if TC_STEP_GROUPS
       const int tile0 = tile;                      // this group's tiles of the unit, stepping by the group count
       for (int kt = kt0 + ((group - tile0) & (Cfg::SG - 1)); kt < kt1; kt += Cfg::SG) {
         tile = tile0 + (kt - kt0);
-#else
-      for (int kt = kt0; kt < kt1; ++kt, ++tile) {
-        if (Cfg::SG > 1 && (tile & 1) != group) continue;
-#endif
         const int sa = tile % SA, ts = tile % NT;
         const uint32_t pa = (uint32_t)(tile / SA) & 1u, pt = (uint32_t)(tile / NT) & 1u;
         mbar_wait(a_full(sa), pa);
-        TC_T(t_afull);
         const uint8_t* tile_smem = base_ptr + sa * Cfg::A_BYTES;
         uint32_t raw[32], lo[32];
-        if (dbg & 1) {
-#pragma unroll
-          for (int j = 0; j < 32; ++j) raw[j] = 0;
-        } else if (MODE == 0) {
+        if (MODE == 0) {
           // row r = 128 contiguous bytes, 16-byte chunk c stored at position c ^ (r & 7)  (SWIZZLE_128B)
           const uint8_t* row = tile_smem + r * 128;
 #pragma unroll
@@ -254,51 +217,28 @@ tc_pass_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
 #pragma unroll
           for (int j = 0; j < 32; ++j) raw[j] = *reinterpret_cast<const uint32_t*>(col + j * 512);
         }
-#if TC_EARLY_RELEASE
-        {
-          // every register of the tile has arrived (xor_all reads them all): the smem slot goes back to TMA now
-          const uint32_t x = xor_all(raw);
-          __syncwarp();
-          if (lane == 0) mbar_arrive(a_free(sa) + (x & ((uint32_t)dbg_arg & 0x40000000u)));
-        }
-#endif
         // a - hi(a) is exact; rounding it to tf32 here (nearest) instead of letting the tensor core truncate it
         // removes the one-sided error of the third term
 #pragma unroll
         for (int j = 0; j < 32; j += 2) tf32_lo_bits2(raw[j], raw[j + 1], lo[j], lo[j + 1]);
-        TC_T(t_load);
         mbar_wait(t_free(ts), pt ^ 1u);
-        TC_T(t_tfree);
-#if TC_SOFT_FREE
         // the MMAs of tile (tile - NT) have completed (this operand slot is free again): so is that tile's B slot
         if (q == 0 && lane == 0 && tile >= NT) mbar_arrive(b_free((tile - NT) % SB));
-#endif
         tc_fence_after();
-        if (!(dbg & 1)) {
-          const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(Cfg::OP_COL0 + ts * 64);
-          tmem_st_x32(taddr, raw);
-          tmem_st_x32(taddr + 32, lo);
-        }
-#if !TC_EARLY_RELEASE
+        const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(Cfg::OP_COL0 + ts * 64);
+        tmem_st_x32(taddr, raw);
+        tmem_st_x32(taddr + 32, lo);
         // Release the smem slot only now: the tcgen05.st instructions above consume every loaded register, so all
         // shared-memory loads of this tile have completed (an arrive placed right after the loads could overtake
         // loads still in flight and let TMA overwrite the tile under them).
         __syncwarp();
         if (lane == 0) mbar_arrive(a_free(sa));
-#endif
-        if (!(dbg & 1)) tmem_st_wait();
+        tmem_st_wait();
         tc_fence_before();
         __syncwarp();
         if (lane == 0) mbar_arrive(t_full(ts));
-        TC_T(t_store);
       }
-#if TC_STEP_GROUPS
       tile = tile0 + max(0, kt1 - kt0);
-#endif
-    }
-    if (prof && warp == 2 && lane == 0) {
-      prof[blockIdx.x * 16 + 7] = t_afull; prof[blockIdx.x * 16 + 8] = t_load; prof[blockIdx.x * 16 + 9] = t_tfree;
-      prof[blockIdx.x * 16 + 10] = t_store;
     }
   } else {
     // ===================== drain warps 6-9: TMEM chunk -> fp32 register accumulators -> global partial ==========
@@ -310,7 +250,6 @@ tc_pass_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     int buf = 0;
     uint32_t accphase = 0;
     constexpr int CH = 16;
-    long long tprev = clock64(), t_accf = 0, t_drain = 0;
     for (int unit = blockIdx.x; unit < num_units; unit += gridDim.x) {
       const int xb = unit % x_blocks, sp = unit / x_blocks;
       const int kt0 = sp * kt_per_split;
@@ -321,7 +260,6 @@ tc_pass_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
       for (int j = 0; j < KD; ++j) acc[j] = 0.f;
       for (int c = 0; c < nchunks; ++c) {
         mbar_wait(accf_bar(buf), accphase);
-        TC_T(t_accf);
         tc_fence_after();
         const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(buf * N2 + c0);
         constexpr int HALF = (Cfg::DW == 2) ? 16 : ((KD >= 32) ? 32 : KD);       // columns folded per batch of loads
@@ -341,7 +279,6 @@ tc_pass_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         __syncwarp();
         if (lane == 0) mbar_arrive(acce_bar(buf));   // TMEM buffer may be overwritten
         if (++buf == NBUF) { buf = 0; accphase ^= 1u; }
-        TC_T(t_drain);
       }
       const int64_t x = (int64_t)xb * TC_BM + q * 32 + lane;
       if (x < x_len) {
@@ -351,7 +288,6 @@ tc_pass_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
           *reinterpret_cast<float4*>(orow + j) = make_float4(acc[j], acc[j + 1], acc[j + 2], acc[j + 3]);
       }
     }
-    if (prof && warp == 6 && lane == 0) { prof[blockIdx.x * 16 + 11] = t_accf; prof[blockIdx.x * 16 + 12] = t_drain; }
   }
 
   tc_fence_before();
@@ -374,7 +310,7 @@ __global__ void __launch_bounds__(256) tc_split_h_kernel(const float* __restrict
   const int j = (int)(idx / n);
   const int64_t c = idx % n;
   const float h = H[(int64_t)j * ldh + c];
-  const float hi = tf32_hi(h, 1);     // nearest: the low part is then signed and half as large
+  const float hi = tf32_rn(h);     // nearest: the low part is then signed and half as large
   Bcat[(int64_t)j * ldb + c] = hi;
   Bcat[(int64_t)(kp + j) * ldb + c] = h - hi;
 }
@@ -392,7 +328,7 @@ __global__ void __launch_bounds__(256) tc_split_wt_kernel(const float* __restric
     const int j = idx / 64, r = idx % 64;
     if (r0 + r < m) {
       const float w = tile[r][j];
-      const float hi = tf32_hi(w, 1);
+      const float hi = tf32_rn(w);
       Bcat[(int64_t)j * ldb + r0 + r] = hi;
       Bcat[(int64_t)(kp + j) * ldb + r0 + r] = w - hi;
     }
@@ -480,13 +416,12 @@ TcPlan tc_plan(int64_t x_len, int64_t r_len, int k, int bk) {
 
 namespace {
 
-unsigned long long* g_prof = nullptr;   // debug: per-CTA role timings (dnmf_set_tc_profile)
-int g_hi_mode = -1;     // -1 unknown, 0 truncate, 1 round-to-nearest-even, 2 = tensor path unusable
+int g_tc_usable = -1;   // -1 not probed yet, 1 the tensor core truncates tf32 operands as the splitters assume, 0 it does not
 int64_t g_min_elems = -1;
 
 template <int K, int MODE>
 int launch_pass(const CUtensorMap& tmA, const CUtensorMap& tmB, float* P, int64_t split_stride, int64_t x_len,
-                const TcPlan& pl, int hi_mode, cudaStream_t st) {
+                const TcPlan& pl, cudaStream_t st) {
   auto kern = tc_pass_kernel<K, MODE>;
   static bool attr_set = false;      // once per instantiation (and never during a stream capture)
   if (!attr_set) {
@@ -495,25 +430,25 @@ int launch_pass(const CUtensorMap& tmA, const CUtensorMap& tmB, float* P, int64_
     attr_set = true;
   }
   kern<<<pl.grid, TcCfg<K>::THREADS, TcCfg<K>::SMEM_BYTES, st>>>(tmA, tmB, P, split_stride, x_len, pl.x_blocks, pl.kt_total,
-                                                            pl.kt_per_split, pl.num_units, hi_mode, tc_dbg_flags(), g_prof);
+                                                            pl.kt_per_split, pl.num_units);
   DNMF_LAUNCH_CHECK("tc_pass_kernel");
   return 0;
 }
 
 template <int MODE>
 int launch_pass_k(int k, const CUtensorMap& tmA, const CUtensorMap& tmB, float* P, int64_t split_stride, int64_t x_len,
-                  const TcPlan& pl, int hi_mode, cudaStream_t st) {
+                  const TcPlan& pl, cudaStream_t st) {
   switch (k) {
-    case 16: return launch_pass<16, MODE>(tmA, tmB, P, split_stride, x_len, pl, hi_mode, st);
-    case 32: return launch_pass<32, MODE>(tmA, tmB, P, split_stride, x_len, pl, hi_mode, st);
-    case 64: return launch_pass<64, MODE>(tmA, tmB, P, split_stride, x_len, pl, hi_mode, st);
+    case 16: return launch_pass<16, MODE>(tmA, tmB, P, split_stride, x_len, pl, st);
+    case 32: return launch_pass<32, MODE>(tmA, tmB, P, split_stride, x_len, pl, st);
+    case 64: return launch_pass<64, MODE>(tmA, tmB, P, split_stride, x_len, pl, st);
   }
   return fail(DNMF_E_UNSUPPORTED, "tcgen05 path: k must be 16, 32 or 64");
 }
 
 // V (AH) or Y / Y^T (WTA) through the tensor path.  ws = [Bcat | partials]
 int tc_run(int mode, const float* A, int64_t lda, const float* B, int64_t ldbsrc, float* out, int64_t ldo,
-           int64_t m, int64_t n, int k, int transposed_out, int hi_mode, void* ws, int64_t ws_bytes, cudaStream_t st,
+           int64_t m, int64_t n, int k, int transposed_out, void* ws, int64_t ws_bytes, cudaStream_t st,
            TcPartials* defer) {
   const int64_t x_len = mode == 0 ? m : n;
   const int64_t r_len = mode == 0 ? n : m;
@@ -544,8 +479,8 @@ int tc_run(int mode, const float* A, int64_t lda, const float* B, int64_t ldbsrc
   rc = make_map(&tmB, Bcat, 2 * kp, r_len, pl.ldb, TC_BK, 2 * kp);
   if (rc) return rc;
   const int64_t split_stride = x_len * kp;
-  rc = mode == 0 ? launch_pass_k<0>(kp, tmA, tmB, P, split_stride, x_len, pl, hi_mode, st)
-                 : launch_pass_k<1>(kp, tmA, tmB, P, split_stride, x_len, pl, hi_mode, st);
+  rc = mode == 0 ? launch_pass_k<0>(kp, tmA, tmB, P, split_stride, x_len, pl, st)
+                 : launch_pass_k<1>(kp, tmA, tmB, P, split_stride, x_len, pl, st);
   if (rc) return rc;
   if (defer != nullptr) {      // the consumer (an update kernel) sums the splits itself, in the same order
     defer->P = P; defer->ldp = kp; defer->split_stride = split_stride; defer->splits = pl.splits;
@@ -562,13 +497,11 @@ int tc_run(int mode, const float* A, int64_t lda, const float* B, int64_t ldbsrc
   return 0;
 }
 
-// One-time probe: does kind::tf32 truncate or round the fp32 bits it reads?  A = 1 + 1.5 * 2^-11 everywhere, H = 1:
-// V = 32 * (1 + 1.5 * 2^-11) exactly iff the splitter's notion of A_hi matches the hardware's.
+// One-time probe: does kind::tf32 truncate the fp32 bits it reads, as the splitters assume?  A = 1 + 1.5 * 2^-11
+// everywhere, H = 1: V = 32 * (1 + 1.5 * 2^-11) exactly iff the splitter's notion of A_hi matches the hardware's.
 void calibrate() {
-  if (g_hi_mode >= 0) return;
-  const char* env = getenv("DNMF_TF32_HI_MODE");
-  if (env) { g_hi_mode = atoi(env); return; }
-  g_hi_mode = 2;
+  if (g_tc_usable >= 0) return;
+  g_tc_usable = 0;
   const int m = 128, n = 32, k = 16;
   const TcPlan pl = tc_plan(m, n, k);
   const int64_t wsb = pl.bcat_bytes + pl.partial_bytes;
@@ -588,18 +521,19 @@ void calibrate() {
   cudaMemcpy(dA, hA, m * n * 4, cudaMemcpyHostToDevice);
   cudaMemcpy(dH, hH, k * n * 4, cudaMemcpyHostToDevice);
   const float expect = 32.0f * aval;
-  for (int mode = 0; mode < 1; ++mode) {      // only the truncating split is compiled into the kernels
-    cudaMemset(dV, 0, m * k * 4);
-    const int64_t saved = tls().launches;
-    int rc = tc_run(0, dA, n, dH, n, dV, k, m, n, k, 0, mode, dws, wsb, 0, nullptr);
-    tls().launches = saved;
-    if (rc != 0 || cudaDeviceSynchronize() != cudaSuccess) { cudaGetLastError(); break; }
+  cudaMemset(dV, 0, m * k * 4);
+  const int64_t saved = tls().launches;
+  const int rc = tc_run(0, dA, n, dH, n, dV, k, m, n, k, 0, dws, wsb, 0, nullptr);
+  tls().launches = saved;
+  if (rc != 0 || cudaDeviceSynchronize() != cudaSuccess) {
+    cudaGetLastError();
+  } else {
     cudaMemcpy(hV, dV, m * k * 4, cudaMemcpyDeviceToHost);
     bool ok = true;
     for (int i = 0; i < m * k; ++i) ok = ok && (hV[i] == expect);
-    if (ok) { g_hi_mode = mode; break; }
+    g_tc_usable = ok ? 1 : 0;
   }
-  if (getenv("DNMF_VERBOSE")) fprintf(stderr, "[libdnmf] tf32 operand mode: %d (0 trunc, 1 rn, 2 tensor path off)\n", g_hi_mode);
+  if (getenv("DNMF_VERBOSE")) fprintf(stderr, "[libdnmf] tcgen05 tf32 path: %s\n", g_tc_usable ? "usable" : "off");
   delete[] hA; delete[] hH; delete[] hV;
   cudaFree(dA); cudaFree(dH); cudaFree(dV); cudaFree(dws);
 }
@@ -640,16 +574,6 @@ int tc_make_map_16(CUtensorMap* map, const void* ptr, int64_t rows, int64_t cols
   if (r != CUDA_SUCCESS) return fail(DNMF_E_ARG, "cuTensorMapEncodeTiled failed with CUresult %d", (int)r);
   return 0;
 }
-int tc_hi_mode() { return g_hi_mode; }
-unsigned long long* tc_prof_ptr() { return g_prof; }
-namespace {
-int g_dbg = -1;       // timing-ablation bits of the tcgen05 kernels (0 in production)
-}
-int tc_dbg_flags() {
-  if (g_dbg < 0) { const char* e = getenv("DNMF_TC_DBG"); g_dbg = e ? (atoi(e) & 0x3FFFFFFF) : 0; }    // read once
-  return g_dbg;
-}
-void tc_set_debug(int flags) { g_dbg = flags < 0 ? 0 : (flags & 0x3FFFFFFF); }
 void tc_launch_split_h(const float* H, int64_t ldh, float* Bcat, int64_t ldb, int k, int kp, int64_t n, cudaStream_t st) {
   tc_split_h_kernel<<<(unsigned)ceil_div((int64_t)k * n, 256), 256, 0, st>>>(H, ldh, Bcat, ldb, k, kp, n);
   tls().launches++;
@@ -680,10 +604,8 @@ bool tc_eligible(int op, const void* A, int64_t lda, int64_t m, int64_t n, int64
   if (m * n < g_min_elems) return false;
   if (!device_is_sm100()) return false;
   calibrate();
-  return g_hi_mode == 0;      // the splitters assume a truncating kind::tf32 (what B200 does); anything else: generic path
+  return g_tc_usable == 1;    // the splitters assume a truncating kind::tf32 (what B200 does); anything else: generic path
 }
-
-void tc_set_profile(void* buf) { g_prof = reinterpret_cast<unsigned long long*>(buf); }
 
 void tc_set_min_elems(int64_t elems) { g_min_elems = elems < 0 ? 0 : elems; }
 
@@ -699,12 +621,12 @@ int64_t tc_workspace_bytes(int op, int64_t m, int64_t n, int64_t k, int dtype) {
 
 int tc_ah(const float* A, int64_t lda, const float* H, int64_t ldh, float* V, int64_t ldv, int64_t m, int64_t n, int k,
           int math_mode, void* ws, int64_t ws_bytes, cudaStream_t st, TcPartials* defer) {
-  return tc_run(0, A, lda, H, ldh, V, ldv, m, n, k, 0, g_hi_mode, ws, ws_bytes, st, defer);
+  return tc_run(0, A, lda, H, ldh, V, ldv, m, n, k, 0, ws, ws_bytes, st, defer);
 }
 
 int tc_wta(const float* A, int64_t lda, const float* W, int64_t ldw, float* Y, int64_t ldy, int64_t m, int64_t n, int k,
            int transposed_out, int math_mode, void* ws, int64_t ws_bytes, cudaStream_t st, TcPartials* defer) {
-  return tc_run(1, A, lda, W, ldw, Y, ldy, m, n, k, transposed_out, g_hi_mode, ws, ws_bytes, st, defer);
+  return tc_run(1, A, lda, W, ldw, Y, ldy, m, n, k, transposed_out, ws, ws_bytes, st, defer);
 }
 
 int tc_kl_uht(const float* A, int64_t lda, const float* W, int64_t ldw, const float* H, int64_t ldh, float* V, int64_t ldv,

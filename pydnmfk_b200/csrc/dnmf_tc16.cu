@@ -68,7 +68,7 @@ __host__ __device__ constexpr uint32_t make_idesc16(int n, int a_mn_major, int b
 }
 
 // One K tile (4 MMAs of K = 16) plus the commits that release the ring slot and, at a chunk end, the accumulator; one
-// asm block under a single elect.sync, issued by a converged warp (see umma_tf32_ts in tc_common.cuh).  ASTEP: the A
+// asm block under a single elect.sync, issued by a converged warp (see umma_tile_ts in tc_common.cuh).  ASTEP: the A
 // descriptor advance per K step (K-major: 32 bytes; MN-major: two 8-row groups of 1024 bytes).
 template <int ASTEP>
 __device__ __forceinline__ void umma16_tile(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc,

@@ -6,27 +6,28 @@
 // W H is never materialised.  Flash-attention-like structure per 128 x 32 tile of A (x = accumulator row: a row of A
 // for UHT, a column of A for WTU; r = the 32 reduced indices of the tile):
 //   GEMM1  S[x, r] = Fx[x, :] . Fr[r, :]        Fx = the x-side factor block (128 x k), resident in TENSOR MEMORY
-//                                                for the whole unit; Fr tile (32 x k, hi|lo) streamed by TMA
+//                                                for the whole unit; Fr tile (64 x k, hi|lo) streamed by TMA
 //   U[x, r] = A[x, r] / (S[x, r] + eps)          splitter warps: A tile from smem, S from TMEM (tcgen05.ld)
 //   GEMM2  D[x, :] += U[x, r] . B[:, r]^T        exactly the FRO contraction with A replaced by U
 // Both GEMMs use the 3-term tf32 split (see dnmf_tc.cu) so the result is fp32-accurate; U and U_lo go to the TMEM
-// operand ring like A and A_lo do on the FRO path.  The MMA warp issues GEMM1 two tiles ahead of GEMM2.
+// operand ring like A and A_lo do on the FRO path.  GEMM1 works on PAIRS of tiles (64 reduced indices): its three split
+// terms are K-concatenated into ONE accumulator of N = 64 MMAs (umma_tile_cat), whose columns [0,32) hold the S tile of
+// the even tile and [32,64) the odd one's.  N = 64 runs at the tensor pipe's full rate (an N = 32 MMA costs 22 cycles
+// instead of 16), the splitters load 32 S columns per tile, and one S slot / one factor-tile slot serves two tiles
+// (round 2: -6 % UHT / -0 % WTU isolated, -3 % sustained against two separate accumulators per tile).  The MMA warp
+// issues GEMM1 ahead of GEMM2.
 //
-// MODE 2 (residual only, tc_residual_run): the same GEMM1 and tile traffic, but the splitters accumulate sum (A - S)^2 and
-// sum A^2 instead of forming U; GEMM2, its B producer and the drain warps idle.
 // MODE 3 (A H^T AND residual in one pass, tc_ah_residual_run; the BCD iteration's second pass, dist_nmf.py:1023-1024):
 // rows of A like MODE 0, U = A itself (so GEMM2 yields V = A H^T exactly as the FRO kernel does), and the splitters
 // accumulate the residual terms on the side.
 //
-// Warp roles (one persistent CTA per SM, warpgroup-aligned so that setmaxnreg can move registers between them):
-// w0 A-TMA | w1 GEMM2 issuer + TMEM owner | w2 Bcat-TMA (lane 0) + Fr-TMA (lane 1) | w3 GEMM1 issuer | w4-7 drain |
-// w8-11, w12-15 [, w16-19] splitter groups.
+// Warp roles (one persistent CTA per SM), see KlCfg::GROUPS:
+//   KK = 32: w0-11 three splitter groups | w12-15 drain | w16 A-TMA | w17 Bcat-TMA (lane 0) + Fr-TMA (lane 1) |
+//            w18 GEMM2 issuer | w19 GEMM1 issuer
+//   KK = 64: w0 A-TMA | w1 GEMM2 issuer | w2-5, w11-14 two splitter groups | w6-9 drain | w10 Bcat-TMA + Fr-TMA |
+//            w15 GEMM1 issuer
+// Barrier waits spin on try_wait without the suspend-time hint (mbar_wait_spin, see tc_common.cuh).
 #include "generic_passes.cuh"
-// Barrier waits of this file spin on try_wait without the suspend-time hint: measured 2-4 % faster for the KL kernels
-// (the FRO kernels in dnmf_tc.cu keep the hint, which is worth 5 % there) -- tools/kl_lab.py, profiles/r02_kl_lab.md.
-#ifndef DNMF_WAIT_HINT
-#define DNMF_WAIT_HINT 0
-#endif
 #include "tc_common.cuh"
 #include "tc_api.cuh"
 
@@ -46,112 +47,37 @@ static_assert(KK == 32 || KK == 64, "KL_KK must be 32 or 64");
 #else
 #define KL_FN(name) name
 #endif
-// KL_GROUPS splitter groups of 4 warps work on tiles round-robin; the per-tile chain (A tile -> S load -> divide -> split ->
-// tensor-memory store -> GEMM2 -> slot free) is latency-bound, so the number of tiles in flight sets the pass time.
-#ifndef KL_GROUPS
-#if KL_KK == 64
-#define KL_GROUPS 2       // tensor memory: 128 (accumulator) + 2 x 64 (U ring) + 2 x 64 (S pair ring) + 128 (Fx) = 512 columns
-#else
-#define KL_GROUPS 3       // round 2: 3 groups are 10-17 % faster than 2 (profiles/r02_kl_lab.md)
-#endif
-#endif
-constexpr int KL_THREADS = 512 + 128 * (KL_GROUPS - 2);
-// Warp-role placement.  The SM's issue arbiter prefers the higher warp id, and setmaxnreg moves registers per warpgroup:
-//   KL_PLACE 0  round-1 placement: w0 A-TMA, w1 GEMM2, w2-5 / w11-14 splitters, w6-9 drain, w10 B/F-TMA, w15 GEMM1
-//   KL_PLACE 1  warpgroups, control at the bottom: w0-3 control (A-TMA, GEMM2, B/F-TMA, GEMM1), w4-7 drain, w8+ splitters
-//   KL_PLACE 2  warpgroups, control at the top:    w0.. splitters, then the drain warpgroup, then the control warpgroup
-#ifndef KL_PLACE
-#ifdef KL_WG_ALIGNED
-#define KL_PLACE KL_WG_ALIGNED
-#else
-#define KL_PLACE (KL_GROUPS == 3 ? 2 : 0)
-#endif
-#endif
-#if KL_GROUPS == 3 && KL_PLACE == 0
-#error "three splitter groups need a warpgroup-aligned role placement"
-#endif
-constexpr int KL_PAIRS = KL_GROUPS * 128;      // residual pairs per CTA (one per splitter thread)
-#ifndef KL_CHUNK_TILES
-#define KL_CHUNK_TILES 4
-#endif
-constexpr int KL_CHUNK = KL_CHUNK_TILES;       // K-tiles accumulated in TMEM before the drain warps fold them into registers
-
-// KL_PACKED = 1: the splitters' fp32 arithmetic uses the packed two-element instructions (FADD2 / FMUL2).
-// KL_S1 = 1: GEMM1 adds its three split terms into ONE 32-column accumulator (umma_tile_cat); the splitters then load
-// 32 S columns per row instead of 64 and skip an addition, and the freed tensor-memory columns deepen the rings.
-// KL_S1 = 2: the same single accumulator, but GEMM1 works on PAIRS of tiles (64 reduced indices): twelve N = 64 MMAs per
-// pair (K-concatenated hi.hi + hi.lo + lo.hi) fill columns [0,32) with the S tile of the even tile and [32,64) with the
-// odd one's.  N = 64 runs at the tensor pipe's full rate (an N = 32 MMA costs 22 cycles instead of 16, which is what made
-// KL_S1 = 1 slower), the splitters load half the S columns, and one S slot / one factor-tile slot serves two tiles.
-#ifndef KL_PACKED
-#define KL_PACKED 1
-#endif
-#ifndef KL_S1
-#define KL_S1 2       // round 2: 0 -> 2 is -6 % (UHT) / -0 % (WTU) isolated, -3 % sustained; 1 is slower than 0 (N = 32 MMA floor)
-#endif
 
 struct KlCfg {
+  // GROUPS splitter groups of 4 warps work on tiles round-robin; the per-tile chain (A tile -> S load -> divide -> split ->
+  // tensor-memory store -> GEMM2 -> slot free) is latency-bound, so the number of tiles in flight sets the pass time.
+  // KK = 32: 3 groups are 10-17 % faster than 2 (profiles/r02_kl_lab.md).  KK = 64: tensor memory holds 128
+  // (accumulator) + 2 x 64 (U ring) + 2 x 64 (S pair ring) + 128 (Fx) = 512 columns, which leaves room for two.
+  static constexpr int GROUPS = (KK == 32) ? 3 : 2;
+  static constexpr int THREADS = 512 + 128 * (GROUPS - 2);
+  static constexpr int PAIRS = GROUPS * 128;         // residual pairs per CTA (one per splitter thread)
+  static constexpr int CHUNK = 4;                    // K-tiles accumulated in TMEM before the drain warps fold them
   static constexpr int N2 = 2 * KK;                    // 64
   static constexpr int A_BYTES = TC_BM * TC_BK * 4;    // 16 KB
   static constexpr int B_BYTES = N2 * TC_BK * 4;       // 8 KB  Bcat tile  [2k][32 r]
-#if KL_S1 == 2
   static constexpr int F_ROWS = 2 * TC_BK;             // reduced indices per factor tile: a pair of tiles
-#else
-  static constexpr int F_ROWS = TC_BK;
-#endif
   static constexpr int F_ATOM_BYTES = F_ROWS * 128;    // F_ROWS rows of one 128-byte swizzle atom (32 factor columns)
-  static constexpr int F_BYTES = 2 * KATOMS * F_ATOM_BYTES;   // FrCat tile [hi: KATOMS atoms | lo: KATOMS atoms]: 8 / 16 / 32 KB
-#ifndef KL_SA
-#if KL_KK == 64
-#define KL_SA 5           // 80 KB A ring + 3 x 16 KB Bcat + 2 x 32 KB FrCat pairs = 192 KB
-#define KL_SB 3
-#else
-#define KL_SA 8
-#define KL_SB 4
-#endif
-#if KL_S1 == 2
-#define KL_SF 2
-#else
-#define KL_SF 4
-#endif
-#endif
-  static constexpr int SA = KL_SA, SB = KL_SB, SF = KL_SF;
-#if KL_S1 == 2 && KL_KK == 64
-  static constexpr int NBUF = 1, NT = 2, NS = 2, S_COLS = 64;
-#elif KL_S1 == 2
-  static constexpr int NBUF = 2, NT = 3, NS = 2, S_COLS = 64;           // one S slot = the S tiles of a pair
-#elif KL_S1
-  static constexpr int NBUF = 2, NT = 3, NS = 4, S_COLS = 32;
-#else
-#ifndef KL_NT
-#if KL_GROUPS == 3
-#define KL_NBUF 1
-#define KL_NT 3
-#define KL_NS 3
-#else
-#define KL_NBUF 2
-#define KL_NT 2
-#define KL_NS 3
-#endif
-#endif
-  static constexpr int NBUF = KL_NBUF, NT = KL_NT, NS = KL_NS, S_COLS = 64;
-#endif
+  static constexpr int F_BYTES = 2 * KATOMS * F_ATOM_BYTES;   // FrCat tile [hi: KATOMS atoms | lo: KATOMS atoms]: 16 / 32 KB
+  // ring depths; KK = 64: 80 KB A ring + 3 x 16 KB Bcat + 2 x 32 KB FrCat pairs = 192 KB
+  static constexpr int SA = (KK == 32) ? 8 : 5, SB = (KK == 32) ? 4 : 3, SF = 2;
+  static constexpr int NBUF = (KK == 32) ? 2 : 1, NT = (KK == 32) ? 3 : 2;
+  static constexpr int NS = 2, S_COLS = 64;            // one S slot = the S tiles of a pair
   static constexpr int ACC_COL0 = 0;
   static constexpr int OP_COL0 = NBUF * N2;            // 128
   static constexpr int S_COL0 = OP_COL0 + NT * 64;
   static constexpr int FX_COL0 = S_COL0 + NS * S_COLS; // 448 (384 for KK = 64)
   static_assert(FX_COL0 + 2 * KK <= 512, "TMEM has 512 columns");
-  static_assert(KK == 32 || KL_S1 == 2, "the 64-wide build needs the paired S tiles");
   // A splitter group waits on a ring slot by phase PARITY, which is only unambiguous while the slot's previous use has
-  // completed.  The group knows that for every tile up to its own previous one (tile - KL_GROUPS; GEMM1 and GEMM2 complete
-  // in tile order), and the slot's previous use is tile - NS (resp. tile - NT): both rings need at least KL_GROUPS slots,
-  // otherwise a group that runs ahead passes the wait one phase early (observed as a hang with NS = 2 and 3 groups).
-#if KL_S1 == 2
-  // (pairs: the slot's previous use is pair p - NS and the group knows every pair up to p - ceil(KL_GROUPS / 2) complete)
-  static_assert(2 * NS >= KL_GROUPS + 1 && NT >= KL_GROUPS, "S and operand rings too shallow for the splitter groups");
-#else
-  static_assert(NS >= KL_GROUPS && NT >= KL_GROUPS, "S and operand rings need one slot per splitter group");
-#endif
+  // completed.  The group knows that for every tile up to its own previous one (tile - GROUPS; GEMM1 and GEMM2 complete
+  // in tile order), and the slot's previous use is tile - NT (resp. pair p - NS, where the group knows every pair up to
+  // p - ceil(GROUPS / 2) complete): both rings need enough slots, otherwise a group that runs ahead passes the wait one
+  // phase early (observed as a hang with one S slot per tile, NS = 2 and 3 groups).
+  static_assert(2 * NS >= GROUPS + 1 && NT >= GROUPS, "S and operand rings too shallow for the splitter groups");
   static constexpr int NBARS = 2 * SA + 2 * SB + 2 * SF + 2 * NT + 2 * NS + 2 * NBUF + 2;
   static constexpr int BAR_BYTES = 1024;
   static_assert((NBARS + 1) * 8 <= BAR_BYTES, "barrier area too small");
@@ -162,18 +88,14 @@ struct KlCfg {
 // MODE 0 (UHT): x = rows of A, A tile = TMA box {32 cols, 128 rows} with 128B swizzle, Fx = W rows
 // MODE 1 (WTU): x = columns of A, A tile = TMA box {128 cols, 32 rows} unswizzled,   Fx = H^T rows
 template <int MODE>
-__global__ void __launch_bounds__(KL_THREADS, 1)
+__global__ void __launch_bounds__(KlCfg::THREADS, 1)
 tc_kl_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
              const __grid_constant__ CUtensorMap tmF, const float* __restrict__ Fx, int64_t ldfx, int64_t fr_rows_pad,
              float* __restrict__ P, int64_t split_stride, int64_t x_len, int x_blocks, int kt_total, int kt_per_split,
-             int num_units, int k_real, float eps, int dbg_arg, double* __restrict__ pairs_out,
-             unsigned long long* __restrict__ prof_arg) {
-  TC_LAB_ARGS(dbg_arg, prof_arg)
-  // dbg (dnmf_set_tc_debug, timing ablations only -- results become wrong): 1 skip the division, 2 skip the S load,
-  // 4 skip the GEMM1 MMAs, 8 skip the GEMM2 low-order MMAs, 16 skip all GEMM2 MMAs, 32 skip the U split, 64 skip the
-  // shared-memory read of the A tile, 0x10000 skip the Bcat TMA loads, 0x20000 skip the FrCat TMA loads
+             int num_units, int k_real, float eps, double* __restrict__ pairs_out) {
   using Cfg = KlCfg;
   constexpr int SA = Cfg::SA, SB = Cfg::SB, SF = Cfg::SF, NT = Cfg::NT, NS = Cfg::NS, NBUF = Cfg::NBUF, N2 = Cfg::N2;
+  constexpr int GROUPS = Cfg::GROUPS, CHUNK = Cfg::CHUNK;
   extern __shared__ uint8_t smem_raw[];
   const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
   uint8_t* base_ptr = smem_raw + (base - smem_u32(smem_raw));
@@ -203,7 +125,7 @@ tc_kl_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
     for (int s = 0; s < SB; ++s) { mbar_init(bar(iBF + s), 1); mbar_init(bar(iBE + s), 1); }
     for (int s = 0; s < SF; ++s) { mbar_init(bar(iFF + s), 1); mbar_init(bar(iFE + s), 1); }
     for (int s = 0; s < NT; ++s) { mbar_init(bar(iTF + s), 4); mbar_init(bar(iTE + s), 1); }
-    for (int s = 0; s < NS; ++s) { mbar_init(bar(iSF + s), 1); mbar_init(bar(iSE + s), KL_S1 == 2 ? 8 : 4); }
+    for (int s = 0; s < NS; ++s) { mbar_init(bar(iSF + s), 1); mbar_init(bar(iSE + s), 8); }
     for (int b = 0; b < NBUF; ++b) { mbar_init(bar(iCF + b), 1); mbar_init(bar(iCE + b), 4); }
     mbar_init(bar(iXF), 4);
     mbar_init(bar(iXE), 1);
@@ -215,83 +137,62 @@ tc_kl_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot_ptr;
 
+  // Warp-role placement.  The SM's issue arbiter prefers the higher warp id, and setmaxnreg moves registers per warpgroup.
   // With three splitter groups the CTA has 640 threads = 96 registers per thread at launch; the producer / issuer
   // warpgroup needs far fewer and hands the rest to the splitter warpgroups (setmaxnreg works per warpgroup, hence the
-  // warpgroup-aligned roles).  setmaxnreg.inc can only draw on what the CTA's own warpgroups released (the CTA's pool is
-  // its launch allocation, 640 x 96): 4 x 32 + 4 x 80 + 12 x 120 registers x 32 lanes = 60416 <= 61440.
-#if KL_PLACE == 1
-  constexpr int W_APROD = 0, W_G2 = 1, W_BPROD = 2, W_G1 = 3;
-  const bool is_ctrl = warp < 4, is_split = warp >= 8;
-  const int split_group = (warp - 8) >> 2, first_split_warp = 8;
-#elif KL_PLACE == 2
-  constexpr int W_CTRL0 = 4 * KL_GROUPS + 4;
-  constexpr int W_APROD = W_CTRL0, W_BPROD = W_CTRL0 + 1, W_G2 = W_CTRL0 + 2, W_G1 = W_CTRL0 + 3;
-  const bool is_ctrl = warp >= W_CTRL0, is_split = warp < 4 * KL_GROUPS;
-  const int split_group = warp >> 2, first_split_warp = 0;
-#else
-  constexpr int W_APROD = 0, W_G2 = 1, W_BPROD = 10, W_G1 = 15;
-  const bool is_ctrl = warp < 2 || warp == W_BPROD || warp == W_G1;
-  const bool is_split = (warp >= 2 && warp < 6) || (warp >= 11 && warp < 15);
-  const int split_group = warp >= 11 ? 1 : 0, first_split_warp = 2;
-#endif
+  // warpgroup-aligned roles, control at the top).  setmaxnreg.inc can only draw on what the CTA's own warpgroups released
+  // (the CTA's pool is its launch allocation, 640 x 96): 4 x 32 + 4 x 80 + 12 x 120 registers x 32 lanes = 60416 <= 61440.
+  // With two groups (KK = 64) the round-1 placement stays, without register moves.
+  constexpr bool WG_ALIGNED = (GROUPS == 3);
+  constexpr int W_CTRL0 = 4 * GROUPS + 4;
+  constexpr int W_APROD = WG_ALIGNED ? W_CTRL0 : 0, W_BPROD = WG_ALIGNED ? W_CTRL0 + 1 : 10;
+  constexpr int W_G1 = WG_ALIGNED ? W_CTRL0 + 3 : 15;    // GEMM2 issuer: the remaining control warp (W_CTRL0 + 2 or 1)
+  const bool is_ctrl = WG_ALIGNED ? warp >= W_CTRL0 : (warp < 2 || warp == W_BPROD || warp == W_G1);
+  const bool is_split = WG_ALIGNED ? warp < 4 * GROUPS : ((warp >= 2 && warp < 6) || (warp >= 11 && warp < 15));
+  const int split_group = WG_ALIGNED ? warp >> 2 : (warp >= 11 ? 1 : 0);
   if (is_ctrl) {
-#if KL_GROUPS == 3
-  asm volatile("setmaxnreg.dec.sync.aligned.u32 32;");
-#endif
-  (void)W_G2;
+  if constexpr (WG_ALIGNED) asm volatile("setmaxnreg.dec.sync.aligned.u32 32;");
   if (warp == W_APROD) {
     // ===================== A producer =====================
     if (lane == 0) {
       int s = 0;
       uint32_t ph = 0;
-      const int pf = tc_pf_dist(dbg);            // L2 prefetch cursor, pf tiles ahead of the ring's loads (tc_common.cuh)
-      TileCursor pc;
-      pc.init(blockIdx.x, gridDim.x, x_blocks, kt_total, kt_per_split, num_units);
-      for (int i = 0; i < pf && pc.valid(); ++i) pc.next();
       for (int unit = blockIdx.x; unit < num_units; unit += gridDim.x) {
         const int xb = unit % x_blocks, sp = unit / x_blocks;
         const int kt0 = sp * kt_per_split, kt1 = min(kt_total, kt0 + kt_per_split);
         for (int kt = kt0; kt < kt1; ++kt) {
-          mbar_wait(bar(iAE + s), ph ^ 1u);
+          mbar_wait_spin(bar(iAE + s), ph ^ 1u);
           mbar_expect_tx(bar(iAF + s), Cfg::A_BYTES);
           if (MODE != 1) tma_load_2d(sA0 + s * Cfg::A_BYTES, &tmA, bar(iAF + s), kt * TC_BK, xb * TC_BM);
           else tma_load_2d(sA0 + s * Cfg::A_BYTES, &tmA, bar(iAF + s), xb * TC_BM, kt * TC_BK);
-          if (pf > 0 && pc.valid()) {
-            if (MODE != 1) tma_prefetch_2d(&tmA, pc.kt * TC_BK, pc.xb() * TC_BM);
-            else tma_prefetch_2d(&tmA, pc.xb() * TC_BM, pc.kt * TC_BK);
-            pc.next();
-          }
           if (++s == SA) { s = 0; ph ^= 1u; }
         }
       }
     }
   } else if (warp == W_BPROD) {
     // ===================== Bcat producer (lane 0, GEMM2 B operand) and FrCat producer (lane 1, GEMM1 B operand) =====
-    if (lane == 0 && MODE != 2) {
+    if (lane == 0) {
       int s = 0;
       uint32_t ph = 0;
       for (int unit = blockIdx.x; unit < num_units; unit += gridDim.x) {
         const int sp = unit / x_blocks;
         const int kt0 = sp * kt_per_split, kt1 = min(kt_total, kt0 + kt_per_split);
         for (int kt = kt0; kt < kt1; ++kt) {
-          mbar_wait(bar(iBE + s), ph ^ 1u);
-          if (dbg & 0x10000) { mbar_arrive(bar(iBF + s)); if (++s == SB) { s = 0; ph ^= 1u; } continue; }   // ablation
+          mbar_wait_spin(bar(iBE + s), ph ^ 1u);
           mbar_expect_tx(bar(iBF + s), Cfg::B_BYTES);
           tma_load_2d(sB0 + s * Cfg::B_BYTES, &tmB, bar(iBF + s), kt * TC_BK, 0);
           if (++s == SB) { s = 0; ph ^= 1u; }
         }
       }
     } else if (lane == 1) {
-      // hi rows then lo rows of the 32 reduced indices
+      // hi rows then lo rows of the 64 reduced indices of a PAIR of K tiles (the TMA box has 64 rows)
       int s = 0;
       uint32_t ph = 0;
       for (int unit = blockIdx.x; unit < num_units; unit += gridDim.x) {
         const int sp = unit / x_blocks;
         const int kt0 = sp * kt_per_split, kt1 = min(kt_total, kt0 + kt_per_split);
-        // one factor tile per K tile, or per PAIR of K tiles (KL_S1 == 2: the TMA box then has 64 rows)
-        for (int kt = kt0; kt < kt1; kt += (KL_S1 == 2 ? 2 : 1)) {
-          mbar_wait(bar(iFE + s), ph ^ 1u);
-          if (dbg & 0x20000) { mbar_arrive(bar(iFF + s)); if (++s == SF) { s = 0; ph ^= 1u; } continue; }   // ablation
+        for (int kt = kt0; kt < kt1; kt += 2) {
+          mbar_wait_spin(bar(iFE + s), ph ^ 1u);
           mbar_expect_tx(bar(iFF + s), Cfg::F_BYTES);
 #pragma unroll
           for (int a = 0; a < KATOMS; ++a) {      // one TMA box per 128-byte swizzle atom along k
@@ -304,117 +205,78 @@ tc_kl_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
       }
     }
   } else if (warp == W_G1) {
-    // ===================== GEMM1 issuer: S = Fx . Fr^T, runs ahead of GEMM2 by up to NS tiles =====================
-    //   KL_S1: cols [0,32) = Fx_hi*Fr_hi + Fx_hi*Fr_lo + Fx_lo*Fr_hi
-    //   else : cols [0,32) Fx_hi*Fr_hi ; cols [32,64) Fx_hi*Fr_lo + Fx_lo*Fr_hi
-    constexpr uint32_t idesc_full = make_idesc(N2, 0);
-    constexpr uint32_t idesc_half = make_idesc(KK, 0);
-    constexpr uint32_t idesc_pair = make_idesc(64, 0);      // GEMM1 on a tile pair: N = 64 reduced indices
-    (void)idesc_full; (void)idesc_half; (void)idesc_pair;
+    // ===================== GEMM1 issuer: S = Fx . Fr^T on tile pairs, runs ahead of GEMM2 by up to NS pairs ==========
+    //   cols [0,64) = Fx_hi*Fr_hi + Fx_hi*Fr_lo + Fx_lo*Fr_hi
+    constexpr uint32_t idesc_pair = make_idesc(64, 0);      // N = 64 reduced indices
     int sf = 0, ss = 0;
     uint32_t pf = 0, ps = 0, pxu = 0;
     const uint32_t fx_tmem = tmem_base + (uint32_t)Cfg::FX_COL0;
-    long long tprev = clock64(), t_g1wait = 0, t_g1 = 0;
     for (int unit = blockIdx.x; unit < num_units; unit += gridDim.x) {
       const int sp = unit / x_blocks;
       const int kt0 = sp * kt_per_split, kt1 = min(kt_total, kt0 + kt_per_split);
       const int ntiles = kt1 - kt0;
-      mbar_wait(bar(iXF), pxu);                     // this unit's Fx block is in tensor memory
-      constexpr int JSTEP = (KL_S1 == 2) ? 2 : 1;
-      for (int j = 0; j < ntiles; j += JSTEP) {
-        mbar_wait(bar(iFF + sf), pf);
-        mbar_wait(bar(iSE + ss), ps ^ 1u);
-        TC_T(t_g1wait);
+      mbar_wait_spin(bar(iXF), pxu);                     // this unit's Fx block is in tensor memory
+      for (int j = 0; j < ntiles; j += 2) {
+        mbar_wait_spin(bar(iFF + sf), pf);
+        mbar_wait_spin(bar(iSE + ss), ps ^ 1u);
         tc_fence_after();
-        if (dbg & 4)
-          umma_commits_only(bar(iSF + ss), bar(iFE + sf), bar(iXE), (j + JSTEP >= ntiles) ? 1u : 0u);
-        else
-#if KL_S1 == 2 && KL_KK == 64
+        if constexpr (KK == 64)
           umma_tile_cat64(tmem_base + (uint32_t)(Cfg::S_COL0 + ss * Cfg::S_COLS), fx_tmem,
                           make_smem_desc(sF0 + sf * Cfg::F_BYTES, 16, 1024), idesc_pair,
-                          bar(iSF + ss), bar(iFE + sf), bar(iXE), (j + JSTEP >= ntiles) ? 1u : 0u);
-#elif KL_S1 == 2
+                          bar(iSF + ss), bar(iFE + sf), bar(iXE), (j + 2 >= ntiles) ? 1u : 0u);
+        else
           umma_tile_cat<64>(tmem_base + (uint32_t)(Cfg::S_COL0 + ss * Cfg::S_COLS), fx_tmem,
                             make_smem_desc(sF0 + sf * Cfg::F_BYTES, 16, 1024), idesc_pair,
-                            bar(iSF + ss), bar(iFE + sf), bar(iXE), (j + JSTEP >= ntiles) ? 1u : 0u);
-#elif KL_S1
-          umma_tile_cat<KK>(tmem_base + (uint32_t)(Cfg::S_COL0 + ss * Cfg::S_COLS), fx_tmem,
-                            make_smem_desc(sF0 + sf * Cfg::F_BYTES, 16, 1024), idesc_half,
-                            bar(iSF + ss), bar(iFE + sf), bar(iXE), (j == ntiles - 1) ? 1u : 0u);
-#else
-          umma_tile_ts<KK>(tmem_base + (uint32_t)(Cfg::S_COL0 + ss * Cfg::S_COLS), fx_tmem,
-                           make_smem_desc(sF0 + sf * Cfg::F_BYTES, 16, 1024), 0u, idesc_full, idesc_half,
-                           bar(iSF + ss), (TC_SOFT_FREE && !KL_S1) ? 0u : bar(iFE + sf), bar(iXE),
-                           (j == ntiles - 1) ? 1u : 0u, 0u);
-#endif
+                            bar(iSF + ss), bar(iFE + sf), bar(iXE), (j + 2 >= ntiles) ? 1u : 0u);
         if (++sf == SF) { sf = 0; pf ^= 1u; }
         if (++ss == NS) { ss = 0; ps ^= 1u; }
         __syncwarp();
-        TC_T(t_g1);
       }
       pxu ^= 1u;
     }
-    if (prof && lane == 0) { prof[blockIdx.x * 16 + 0] = t_g1wait; prof[blockIdx.x * 16 + 1] = t_g1; }
   } else {
-    // ===================== GEMM2 issuer, warp 1 (converged warp, elected lane inside the asm block) ==============
+    // ===================== GEMM2 issuer (converged warp, elected lane inside the asm block) ======================
     constexpr uint32_t idesc_full = make_idesc(N2, 0);
     constexpr uint32_t idesc_half = make_idesc(KK, 0);
     int sb = 0, ts = 0, buf = 0;
     uint32_t pb = 0, pt = 0, accphase = 0;
-    long long tprev = clock64(), t_acce = 0, t_tfull = 0, t_bfull = 0, t_g2 = 0, t0 = tprev;
-    for (int unit = blockIdx.x; MODE != 2 && unit < num_units; unit += gridDim.x) {
+    for (int unit = blockIdx.x; unit < num_units; unit += gridDim.x) {
       const int sp = unit / x_blocks;
       const int kt0 = sp * kt_per_split, kt1 = min(kt_total, kt0 + kt_per_split);
       const int ntiles = kt1 - kt0;
       for (int i = 0; i < ntiles; ++i) {
-        const int in_chunk = i % KL_CHUNK;
-        if (in_chunk == 0) mbar_wait(bar(iCE + buf), accphase ^ 1u);
-        TC_T(t_acce);
-        mbar_wait(bar(iTF + ts), pt);
-        TC_T(t_tfull);
-        mbar_wait(bar(iBF + sb), pb);
-        TC_T(t_bfull);
+        const int in_chunk = i % CHUNK;
+        if (in_chunk == 0) mbar_wait_spin(bar(iCE + buf), accphase ^ 1u);
+        mbar_wait_spin(bar(iTF + ts), pt);
+        mbar_wait_spin(bar(iBF + sb), pb);
         tc_fence_after();
-        const bool chunk_end = (in_chunk == KL_CHUNK - 1) || (i == ntiles - 1);
-        if (dbg & 16)
-          umma_commits_only(bar(iTE + ts), bar(iBE + sb), bar(iCF + buf), chunk_end ? 1u : 0u);
-        else
-          umma_tile_ts<KK>(tmem_base + (uint32_t)(Cfg::ACC_COL0 + buf * N2), tmem_base + (uint32_t)(Cfg::OP_COL0 + ts * 64),
-                           make_smem_desc(sB0 + sb * Cfg::B_BYTES, 16, 1024), in_chunk > 0 ? 1u : 0u, idesc_full, idesc_half,
-                           bar(iTE + ts), (TC_SOFT_FREE && MODE != 2) ? 0u : bar(iBE + sb), bar(iCF + buf),
-                           chunk_end ? 1u : 0u, (dbg & 8) ? 1u : 0u);
+        const bool chunk_end = (in_chunk == CHUNK - 1) || (i == ntiles - 1);
+        umma_tile_ts<KK>(tmem_base + (uint32_t)(Cfg::ACC_COL0 + buf * N2), tmem_base + (uint32_t)(Cfg::OP_COL0 + ts * 64),
+                         make_smem_desc(sB0 + sb * Cfg::B_BYTES, 16, 1024), in_chunk > 0 ? 1u : 0u, idesc_full, idesc_half,
+                         bar(iTE + ts), bar(iCF + buf), chunk_end ? 1u : 0u);
         if (++ts == NT) { ts = 0; pt ^= 1u; }
         if (++sb == SB) { sb = 0; pb ^= 1u; }
         if (chunk_end) { if (++buf == NBUF) { buf = 0; accphase ^= 1u; } }
         __syncwarp();
-        TC_T(t_g2);
       }
-    }
-    if (prof && lane == 0) {
-      prof[blockIdx.x * 16 + 2] = t_acce; prof[blockIdx.x * 16 + 3] = t_tfull; prof[blockIdx.x * 16 + 4] = t_bfull;
-      prof[blockIdx.x * 16 + 5] = t_g2; prof[blockIdx.x * 16 + 15] = clock64() - t0;
     }
   }
   } else if (is_split) {
-#if KL_GROUPS == 3
-    asm volatile("setmaxnreg.inc.sync.aligned.u32 120;");
-#endif
+    if constexpr (WG_ALIGNED) asm volatile("setmaxnreg.inc.sync.aligned.u32 120;");
     // ===================== splitters: A tile + S tile -> U = A / (S + eps) -> {U, U_lo} in TMEM ====================
     const int q = warp & 3;
     const int r = q * 32 + lane;
     const int group = split_group;
     int tile = 0;
-    int pair_base = 0;                      // KL_S1 == 2: tile pairs of the units this CTA has finished
-    (void)pair_base;
+    int pair_base = 0;                      // tile pairs of the units this CTA has finished
     uint32_t pxe = 0;
-    double res_sum = 0.0, a_sum = 0.0;      // MODE 2 only
-    long long tprev = clock64(), t_afull = 0, t_load = 0, t_sfull = 0, t_div = 0, t_tfree = 0, t_store = 0;
+    double res_sum = 0.0, a_sum = 0.0;      // MODE 3 only
     for (int unit = blockIdx.x; unit < num_units; unit += gridDim.x) {
       const int xb = unit % x_blocks, sp = unit / x_blocks;
       const int kt0 = sp * kt_per_split, kt1 = min(kt_total, kt0 + kt_per_split);
       if (group == 0) {
         // x-side factor row of this thread -> tensor memory (hi | lo), once per unit
-        mbar_wait(bar(iXE), pxe ^ 1u);              // the previous unit's GEMM1s have finished reading Fx
+        mbar_wait_spin(bar(iXE), pxe ^ 1u);              // the previous unit's GEMM1s have finished reading Fx
         tc_fence_after();
         const int64_t x = (int64_t)xb * TC_BM + r;
         const float* frow = Fx + x * ldfx;
@@ -425,7 +287,7 @@ tc_kl_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
 #pragma unroll
           for (int j = 0; j < 32; ++j) {
             const float w = (x < x_len && c0 + j < k_real) ? frow[c0 + j] : 0.f;      // factor columns beyond k: zero padding
-            const float h = tf32_hi(w, 1);
+            const float h = tf32_rn(w);
             hi[j] = __float_as_uint(h);
             lo[j] = __float_as_uint(tf32_round_up(w - h));
           }
@@ -438,21 +300,15 @@ tc_kl_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
         if (lane == 0) mbar_arrive(bar(iXF));
         pxe ^= 1u;
       }
-#if TC_STEP_GROUPS
       // this group's tiles of the unit, stepping by the group count (the walk over every tile with a modulo test per
       // tile cost 10 % of the kernel's warp samples, profiles/r02_ncu_source_hotspots.txt)
       const int tile0 = tile;
-      int first = group - tile0 % KL_GROUPS;
-      if (first < 0) first += KL_GROUPS;
-      for (int kt = kt0 + first; kt < kt1; kt += KL_GROUPS) {
+      int first = group - tile0 % GROUPS;
+      if (first < 0) first += GROUPS;
+      for (int kt = kt0 + first; kt < kt1; kt += GROUPS) {
         tile = tile0 + (kt - kt0);
-#else
-      for (int kt = kt0; kt < kt1; ++kt, ++tile) {
-        if (tile % KL_GROUPS != group) continue;
-#endif
         const int sa = tile % SA, ts = tile % NT;
         const uint32_t pa = (uint32_t)(tile / SA) & 1u, pt = (uint32_t)(tile / NT) & 1u;
-#if KL_S1 == 2
         // S slots hold PAIRS of tiles: pair index inside this CTA's sequence, which half of the slot is this tile's, and
         // whether the tile has no partner (odd tile count of the unit: it then releases the slot for both)
         const int jt = kt - kt0;
@@ -460,20 +316,10 @@ tc_kl_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
         const int ss = pairid % NS, s_half = jt & 1;
         const uint32_t ps = (uint32_t)(pairid / NS) & 1u;
         const bool s_lone = (s_half == 0) && (kt == kt1 - 1);
-#else
-        const int ss = tile % NS, s_half = 0;
-        const uint32_t ps = (uint32_t)(tile / NS) & 1u;
-        const bool s_lone = false;
-#endif
-        TC_T(t_store);
-        mbar_wait(bar(iAF + sa), pa);
-        TC_T(t_afull);
+        mbar_wait_spin(bar(iAF + sa), pa);
         const uint8_t* tl = base_ptr + sa * Cfg::A_BYTES;
         uint32_t u[32], lo[32];
-        if (dbg & 64) {
-#pragma unroll
-          for (int j = 0; j < 32; ++j) u[j] = 0x3F800000u + (uint32_t)(j + lane);
-        } else if (MODE != 1) {
+        if (MODE != 1) {
           const uint8_t* row = tl + r * 128;
 #pragma unroll
           for (int c = 0; c < 8; ++c) {
@@ -485,103 +331,38 @@ tc_kl_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
 #pragma unroll
           for (int j = 0; j < 32; ++j) u[j] = *reinterpret_cast<const uint32_t*>(col + j * 512);
         }
-#if TC_EARLY_RELEASE
-        if (MODE != 2) {
-          // every register of the tile has arrived (xor_all reads them all): the smem slot goes back to TMA now
-          const uint32_t x = xor_all(u);
-          __syncwarp();
-          if (lane == 0) mbar_arrive(bar(iAE + sa) + (x & ((uint32_t)dbg_arg & 0x40000000u)));
-        }
-#endif
         // S tile of this accumulator row
-        TC_T(t_load);
-        mbar_wait(bar(iSF + ss), ps);
-        TC_T(t_sfull);
-#if TC_SOFT_FREE && !KL_S1
-        // GEMM1 of this tile has completed (it committed to the S barrier): its factor tile may be overwritten
-        if (q == 0 && lane == 0 && !(dbg & 4)) mbar_arrive(bar(iFE + tile % SF));
-#endif
+        mbar_wait_spin(bar(iSF + ss), ps);
         tc_fence_after();
         const uint32_t saddr = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(Cfg::S_COL0 + ss * Cfg::S_COLS + s_half * 32);
         {
-#if KL_S1
           uint32_t s0[32];
-          if (dbg & 2) {
-#pragma unroll
-            for (int j = 0; j < 32; ++j) s0[j] = 0x3F800000u;
-          } else {
-            tmem_ld_x32(saddr, s0);         // Fx_hi * Fr_hi + Fx_hi * Fr_lo + Fx_lo * Fr_hi
-            tmem_ld_wait();
-          }
-#define KL_S_OF(j) __uint_as_float(s0[j])
-#else
-          uint32_t s0[32], s1[32];
-          if (dbg & 2) {
-#pragma unroll
-            for (int j = 0; j < 32; ++j) { s0[j] = 0x3F800000u; s1[j] = 0u; }
-          } else {
-            tmem_ld_x32(saddr, s0);           // Fx_hi * Fr_hi
-            tmem_ld_x32(saddr + 32, s1);      // Fx_hi * Fr_lo + Fx_lo * Fr_hi
-            tmem_ld_wait();
-          }
-#define KL_S_OF(j) (__uint_as_float(s0[j]) + __uint_as_float(s1[j]))
-#endif
-          if (MODE == 2 || MODE == 3) {
+          tmem_ld_x32(saddr, s0);         // Fx_hi * Fr_hi + Fx_hi * Fr_lo + Fx_lo * Fr_hi
+          tmem_ld_wait();
+          if (MODE == 3) {
             // residual: this row's 32 elements of (A - W H)^2 and A^2, fp32 within the tile, float64 across tiles
             float t_res = 0.f, t_a = 0.f;
 #pragma unroll
             for (int j = 0; j < 32; ++j) {
               const float a = __uint_as_float(u[j]);
-              const float d = a - KL_S_OF(j);
+              const float d = a - __uint_as_float(s0[j]);
               t_res = fmaf(d, d, t_res);
               t_a = fmaf(a, a, t_a);
             }
             res_sum += (double)t_res;
             a_sum += (double)t_a;
           }
-          if (MODE == 2) {
-            tc_fence_before();
-            __syncwarp();
-            if (lane == 0) {
-              mbar_arrive(bar(iSE + ss));       // S slot may be overwritten
-              if (s_lone) mbar_arrive(bar(iSE + ss));
-              mbar_arrive(bar(iAE + sa));       // every register loaded from the A tile has been consumed above
-            }
-            continue;
-          }
-#if KL_PACKED && KL_S1
+          // U = A / (S + eps), two elements per FADD2 / FMUL2 (sm_100 packed fp32).  den >= eps > 0 and far from
+          // overflow: one MUFU.RCP (1 ulp) and one multiply, no range handling.  The rounding errors of the 65536
+          // quotients of a row are independent and average out in the contraction.
 #pragma unroll
           for (int j = 0; MODE != 3 && j < 32; j += 2) {
             const float2 den = __fadd2_rn(make_float2(__uint_as_float(s0[j]), __uint_as_float(s0[j + 1])), make_float2(eps, eps));
-            const float2 q2 = (dbg & 1) ? den : make_float2(rcp_approx(den.x), rcp_approx(den.y));
+            const float2 q2 = make_float2(rcp_approx(den.x), rcp_approx(den.y));
             const float2 uu = __fmul2_rn(make_float2(__uint_as_float(u[j]), __uint_as_float(u[j + 1])), q2);
             u[j] = __float_as_uint(uu.x);
             u[j + 1] = __float_as_uint(uu.y);
           }
-#elif KL_PACKED
-          // two elements per FADD2 / FMUL2 (sm_100 packed fp32): the same roundings as the scalar code below, half the
-          // FMA-pipe instructions of the warps whose instruction stream sets the pass time
-#pragma unroll
-          for (int j = 0; MODE != 3 && j < 32; j += 2) {
-            float2 den = __fadd2_rn(make_float2(__uint_as_float(s0[j]), __uint_as_float(s0[j + 1])),
-                                    make_float2(__uint_as_float(s1[j]), __uint_as_float(s1[j + 1])));
-            den = __fadd2_rn(den, make_float2(eps, eps));
-            const float2 q2 = (dbg & 1) ? den : make_float2(rcp_approx(den.x), rcp_approx(den.y));
-            const float2 uu = __fmul2_rn(make_float2(__uint_as_float(u[j]), __uint_as_float(u[j + 1])), q2);
-            u[j] = __float_as_uint(uu.x);
-            u[j + 1] = __float_as_uint(uu.y);
-          }
-#else
-#pragma unroll
-          for (int j = 0; MODE != 3 && j < 32; ++j) {
-            const float den = KL_S_OF(j) + eps;
-            const float a = __uint_as_float(u[j]);
-            // den >= eps > 0 and far from overflow: one MUFU.RCP (1 ulp) and one multiply, no range handling.  The
-            // rounding errors of the 65536 quotients of a row are independent and average out in the contraction.
-            u[j] = __float_as_uint((dbg & 1) ? a * den : a * rcp_approx(den));
-          }
-#endif
-#undef KL_S_OF
         }
         tc_fence_before();
         __syncwarp();
@@ -589,72 +370,46 @@ tc_kl_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
           mbar_arrive(bar(iSE + ss));                       // S slot may be overwritten
           if (s_lone) mbar_arrive(bar(iSE + ss));           // ... on behalf of the missing odd tile as well
         }
-#if KL_PACKED
 #pragma unroll
-        for (int j = 0; j < 32; j += 2) {
-          if (dbg & 32) { lo[j] = u[j]; lo[j + 1] = u[j + 1]; continue; }
-          tf32_lo_bits2(u[j], u[j + 1], lo[j], lo[j + 1]);
-        }
-#else
-#pragma unroll
-        for (int j = 0; j < 32; ++j) {
-          lo[j] = (dbg & 32) ? u[j] : tf32_lo_bits(u[j]);
-        }
-#endif
-        TC_T(t_div);
-        mbar_wait(bar(iTE + ts), pt ^ 1u);
-        TC_T(t_tfree);
-#if TC_SOFT_FREE
+        for (int j = 0; j < 32; j += 2) tf32_lo_bits2(u[j], u[j + 1], lo[j], lo[j + 1]);
+        mbar_wait_spin(bar(iTE + ts), pt ^ 1u);
         // GEMM2 of tile (tile - NT) has completed (this operand slot is free again): so is that tile's Bcat slot
-        if (q == 0 && lane == 0 && tile >= NT && !(dbg & 16)) mbar_arrive(bar(iBE + (tile - NT) % SB));
-#endif
+        if (q == 0 && lane == 0 && tile >= NT) mbar_arrive(bar(iBE + (tile - NT) % SB));
         tc_fence_after();
         const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(Cfg::OP_COL0 + ts * 64);
-        if (!(dbg & 0x80)) {
-          tmem_st_x32(taddr, u);
-          tmem_st_x32(taddr + 32, lo);
-        }
-#if !TC_EARLY_RELEASE
+        tmem_st_x32(taddr, u);
+        tmem_st_x32(taddr + 32, lo);
         __syncwarp();
         if (lane == 0) mbar_arrive(bar(iAE + sa));          // smem tile fully consumed (see dnmf_tc.cu)
-#endif
-        if (!(dbg & 0x80)) tmem_st_wait();
+        tmem_st_wait();
         tc_fence_before();
         __syncwarp();
         if (lane == 0) mbar_arrive(bar(iTF + ts));
       }
-#if TC_STEP_GROUPS
       tile = tile0 + max(0, kt1 - kt0);
-#endif
       pair_base += (kt1 - kt0 + 1) >> 1;
     }
-    if (MODE == 2 || MODE == 3) {
+    if (MODE == 3) {
       // one (residual, norm) pair per splitter thread; summed in a fixed order by the caller
-      double* pairs = pairs_out + ((int64_t)blockIdx.x * KL_PAIRS + (group * 4 + q) * 32 + lane) * 2;
+      double* pairs = pairs_out + ((int64_t)blockIdx.x * Cfg::PAIRS + (group * 4 + q) * 32 + lane) * 2;
       pairs[0] = res_sum;
       pairs[1] = a_sum;
     }
-    if (prof && warp == first_split_warp && lane == 0) {
-      prof[blockIdx.x * 16 + 6] = t_afull; prof[blockIdx.x * 16 + 7] = t_load; prof[blockIdx.x * 16 + 8] = t_sfull;
-      prof[blockIdx.x * 16 + 9] = t_div; prof[blockIdx.x * 16 + 10] = t_tfree; prof[blockIdx.x * 16 + 11] = t_store;
-    }
   } else {
-#if KL_GROUPS == 3
-    asm volatile("setmaxnreg.dec.sync.aligned.u32 80;");
-#endif
-    // ===================== drain warps 4-7 =====================
+    if constexpr (WG_ALIGNED) asm volatile("setmaxnreg.dec.sync.aligned.u32 80;");
+    // ===================== drain warps =====================
     const int q = warp & 3;
     int buf = 0;
     uint32_t accphase = 0;
-    for (int unit = blockIdx.x; MODE != 2 && unit < num_units; unit += gridDim.x) {
+    for (int unit = blockIdx.x; unit < num_units; unit += gridDim.x) {
       const int xb = unit % x_blocks, sp = unit / x_blocks;
       const int kt0 = sp * kt_per_split, kt1 = min(kt_total, kt0 + kt_per_split);
-      const int nchunks = (kt1 - kt0 + KL_CHUNK - 1) / KL_CHUNK;
+      const int nchunks = (kt1 - kt0 + CHUNK - 1) / CHUNK;
       float acc[KK];
 #pragma unroll
       for (int j = 0; j < KK; ++j) acc[j] = 0.f;
       for (int c = 0; c < nchunks; ++c) {
-        mbar_wait(bar(iCF + buf), accphase);
+        mbar_wait_spin(bar(iCF + buf), accphase);
         tc_fence_after();
         const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(Cfg::ACC_COL0 + buf * N2);
         constexpr int DCH = (KK > 32) ? 16 : KK;      // columns folded per batch of loads (register budget at KK = 64)
@@ -717,7 +472,7 @@ __global__ void __launch_bounds__(256) kl_split_fr_kernel(const float* __restric
     const int r = idx / KK, j = idx % KK;
     if (r0 + r < r_pad) {
       const float w = j < k ? tile[r][j] : 0.f;
-      const float hi = tf32_hi(w, 1);
+      const float hi = tf32_rn(w);
       FrCat[(r0 + r) * KK + j] = hi;
       FrCat[(r_pad + r0 + r) * KK + j] = tf32_round_up(w - hi);
     }
@@ -825,9 +580,9 @@ int KL_FN(tc_kl_run)(int mode, const float* A, int64_t lda, const float* W, int6
       if (e != cudaSuccess) return cuda_fail(e, "tc_kl_kernel smem attribute");
       attr_set[mode] = true;
     }
-    kern<<<pl.grid, KL_THREADS, KlCfg::SMEM_BYTES, st>>>(tmA, tmB, tmF, Fx, ldfx, kp.r_pad, P, split_stride, x_len,
-                                                          pl.x_blocks, pl.kt_total, pl.kt_per_split, pl.num_units,
-                                                          k_real, eps, tc_dbg_flags(), nullptr, tc_prof_ptr());
+    kern<<<pl.grid, KlCfg::THREADS, KlCfg::SMEM_BYTES, st>>>(tmA, tmB, tmF, Fx, ldfx, kp.r_pad, P, split_stride, x_len,
+                                                              pl.x_blocks, pl.kt_total, pl.kt_per_split, pl.num_units,
+                                                              k_real, eps, nullptr);
     DNMF_LAUNCH_CHECK("tc_kl_kernel");
     return 0;
   };
@@ -852,7 +607,8 @@ int KL_FN(tc_kl_run)(int mode, const float* A, int64_t lda, const float* W, int6
 // ws = [Bcat | FrCat | partials | pairs (grid x 256 x 2 float64)]
 int64_t tc_ah_residual_workspace_bytes(int64_t m, int64_t n) {
   const KlPlan p = kl_plan(0, m, n);
-  return p.base.bcat_bytes + p.frcat_bytes + p.base.partial_bytes + round_up((int64_t)p.base.grid * KL_PAIRS * 2 * (int64_t)sizeof(double), 1024);
+  return p.base.bcat_bytes + p.frcat_bytes + p.base.partial_bytes +
+         round_up((int64_t)p.base.grid * KlCfg::PAIRS * 2 * (int64_t)sizeof(double), 1024);
 }
 
 int tc_ah_residual_run(const float* A, int64_t lda, const float* W, int64_t ldw, const float* H, int64_t ldh, float* V,
@@ -892,66 +648,13 @@ int tc_ah_residual_run(const float* A, int64_t lda, const float* W, int64_t ldw,
     attr_set = true;
   }
   const int64_t split_stride = m * KK;
-  kern<<<pl.grid, KL_THREADS, KlCfg::SMEM_BYTES, st>>>(tmA, tmB, tmF, W, ldw, kp.r_pad, P, split_stride, m, pl.x_blocks,
-                                                        pl.kt_total, pl.kt_per_split, pl.num_units, k, 0.f, tc_dbg_flags(),
-                                                        pairs, tc_prof_ptr());
+  kern<<<pl.grid, KlCfg::THREADS, KlCfg::SMEM_BYTES, st>>>(tmA, tmB, tmF, W, ldw, kp.r_pad, P, split_stride, m, pl.x_blocks,
+                                                            pl.kt_total, pl.kt_per_split, pl.num_units, k, 0.f, pairs);
   DNMF_LAUNCH_CHECK("tc_kl_kernel<3>");
   reduce_partials_kernel<float><<<(unsigned)ceil_div(m * k, 256), 256, 0, st>>>(P, split_stride, pl.splits, m, k, V, ldv, 1, KK);
   DNMF_LAUNCH_CHECK("reduce_partials_kernel");
   *out_pairs = pairs;
-  *n_pairs = (int64_t)pl.grid * KL_PAIRS;
-  return 0;
-}
-
-// ---- ||A - W H||^2 and ||A||^2 through the same pipeline (MODE 2) ---------------------------------------------------
-// Opt-in (DNMF_TC_RESIDUAL=1): written at the end of round 1 and NOT yet run on hardware; the default stays the
-// CUDA-core residual kernel.  ws = [FrCat | pairs (grid x 256 x 2 float64)]; out_pairs receives the per-thread pairs,
-// *n_pairs their count (the caller sums them in a fixed order).
-namespace { int g_tc_residual = -1; }
-bool tc_residual_enabled() {
-  if (g_tc_residual < 0) { const char* e = getenv("DNMF_TC_RESIDUAL"); g_tc_residual = (e && atoi(e) != 0) ? 1 : 0; }
-  return g_tc_residual == 1;
-}
-void tc_set_residual(int on) { g_tc_residual = on ? 1 : 0; }
-
-int64_t tc_residual_workspace_bytes(int64_t m, int64_t n) {
-  const KlPlan p = kl_plan(0, m, n);
-  return p.frcat_bytes + round_up((int64_t)p.base.grid * KL_PAIRS * 2 * (int64_t)sizeof(double), 1024);
-}
-
-int tc_residual_run(const float* A, int64_t lda, const float* W, int64_t ldw, const float* H, int64_t ldh, int64_t m,
-                    int64_t n, int k, void* ws, int64_t ws_bytes, double** out_pairs, int64_t* n_pairs, cudaStream_t st) {
-  if (k < 1 || k > KK) return fail(DNMF_E_UNSUPPORTED, "tcgen05 residual: k must be in [1, %d]", KK);
-  const KlPlan kp = kl_plan(0, m, n);
-  const TcPlan& pl = kp.base;
-  const int64_t need = tc_residual_workspace_bytes(m, n);
-  if (ws == nullptr || ws_bytes < need)
-    return fail(DNMF_E_WORKSPACE, "tcgen05 residual needs %lld workspace bytes, got %lld", (long long)need, (long long)ws_bytes);
-  if (((uintptr_t)ws % 256) != 0) return fail(DNMF_E_ARG, "workspace must be 256-byte aligned");
-  uint8_t* wsb = reinterpret_cast<uint8_t*>(ws);
-  float* FrCat = reinterpret_cast<float*>(wsb);
-  double* pairs = reinterpret_cast<double*>(wsb + kp.frcat_bytes);
-  kl_split_fr_kernel<true><<<(unsigned)ceil_div(kp.r_pad, 64), 256, 0, st>>>(H, ldh, FrCat, n, kp.r_pad, k);
-  DNMF_LAUNCH_CHECK("kl_split_fr_kernel<T>");
-  alignas(64) CUtensorMap tmA, tmF;
-  int rc = tc_make_map(&tmA, A, m, n, lda, TC_BK, TC_BM, CU_TENSOR_MAP_SWIZZLE_128B);
-  if (rc) return rc;
-  rc = tc_make_map(&tmF, FrCat, 2 * kp.r_pad, KK, KK, 32, KlCfg::F_ROWS, CU_TENSOR_MAP_SWIZZLE_128B);
-  if (rc) return rc;
-  auto kern = tc_kl_kernel<2>;
-  static bool attr_set = false;
-  if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, KlCfg::SMEM_BYTES);
-    if (e != cudaSuccess) return cuda_fail(e, "tc_kl_kernel<2> smem attribute");
-    attr_set = true;
-  }
-  // (the GEMM2 operand map is unused in this mode: tmF stands in for it)
-  kern<<<pl.grid, KL_THREADS, KlCfg::SMEM_BYTES, st>>>(tmA, tmF, tmF, W, ldw, kp.r_pad, nullptr, 0, m,
-                                                        pl.x_blocks, pl.kt_total, pl.kt_per_split, pl.num_units, k, 0.f,
-                                                        0, pairs, tc_prof_ptr());
-  DNMF_LAUNCH_CHECK("tc_kl_kernel<2>");
-  *out_pairs = pairs;
-  *n_pairs = (int64_t)pl.grid * KL_PAIRS;
+  *n_pairs = (int64_t)pl.grid * KlCfg::PAIRS;
   return 0;
 }
 

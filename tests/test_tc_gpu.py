@@ -180,23 +180,6 @@ def test_ah_residual_fused_pass(ops, m, n, k):
     assert abs(got[0] - sep[0]) <= 2e-6 * rr and abs(got[1] - sep[1]) <= 1e-6 * ar
 
 
-def test_residual_on_the_tensor_pipeline(ops):
-    """tc_kl_kernel<2> (dnmf_set_tc_residual(1)) against the CUDA-core residual kernel and float64 numpy."""
-    from pydnmfk_b200 import _lib as L
-    rs = np.random.RandomState(5)
-    m, n, k = 2048, 2048, 32
-    A, W, H = rs.rand(m, n).astype(np.float32), rs.rand(m, k).astype(np.float32), rs.rand(k, n).astype(np.float32)
-    ref = ops.residual_sqnorm(_dev(A), _dev(W), _dev(H)).cpu().numpy()
-    L.call('dnmf_set_tc_residual', 1)
-    try:
-        got = ops.residual_sqnorm(_dev(A), _dev(W), _dev(H)).cpu().numpy()
-    finally:
-        L.call('dnmf_set_tc_residual', 0)
-    f = np.float64
-    rr = np.linalg.norm(A.astype(f) - W.astype(f) @ H.astype(f)) ** 2
-    assert abs(got[0] - rr) <= 2e-6 * rr and abs(got[0] - ref[0]) <= 2e-6 * rr and abs(got[1] - ref[1]) <= 1e-6 * ref[1]
-
-
 @pytest.mark.parametrize('m,n,k', [(2048, 2048, 32), (1000, 1000, 32), (515, 2052, 20), (4100, 300, 64), (8192, 1024, 10),
                                    (1024, 8192, 32)])
 def test_fused_epilogue_is_bit_identical(ops, m, n, k):

@@ -2,8 +2,8 @@
 depths, wait flavour): run the four A-streaming contractions of both on a list of shapes (ragged edges, odd tile counts,
 one x-block with a deep split-K, k = 10 / 16 / 32 / 48 / 64) and compare the outputs bit for bit (one GPU, one process).
 
-    tools/build_variant.sh step "-DTC_STEP_GROUPS=1"
-    python tools/ab_bitexact.py step            # libdnmf.so against libdnmf_step.so
+    cp <other build>/libdnmf.so pydnmfk_b200/libdnmf_other.so
+    python tools/ab_bitexact.py other           # libdnmf.so against libdnmf_other.so
 
 Exit code 0 = identical everywhere and every call took the tcgen05 path in both libraries."""
 import ctypes as C

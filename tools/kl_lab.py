@@ -1,13 +1,12 @@
-"""A/B laboratory for the A-streaming tcgen05 kernels (one GPU, ONE process):
+"""A/B timing of the A-streaming tcgen05 kernels of two or more builds of the library (one GPU, ONE process):
 
-    python tools/kl_lab.py --variants default,late --dbg 0,1,65536 [--m 65536 --n 65536 --k 32] [--rounds 6]
+    python tools/kl_lab.py --variants default,parent [--m 65536 --n 65536 --k 32] [--rounds 6]
 
-Every library variant (pydnmfk_b200/libdnmf_<name>.so from tools/build_variant.sh; "default" = libdnmf.so) is loaded
-side by side with ctypes and the (variant, flag set, op) combinations are timed in a reshuffled order for `--rounds`
-rounds, each paired with a reference launch issued right before it (see below); the report is the median ratio to the
-reference plus the median and minimum time per combination.
-Flag sets are the timing-ablation bits of dnmf_set_tc_debug (non-zero values give wrong results; they only locate the
-bottleneck).  For flags 0 every variant is also checked against float64 numpy on a 2048 x 1536 shard."""
+Every variant is a library file loaded side by side with ctypes: "default" = pydnmfk_b200/libdnmf.so, any other name =
+pydnmfk_b200/libdnmf_<name>.so (for example the build of another commit, copied there).  The (variant, op) combinations
+are timed in a reshuffled order for `--rounds` rounds, each paired with a reference launch issued right before it (see
+below); the report is the median ratio to the reference plus the median and minimum time per combination.  Every
+variant is also checked against float64 numpy on a 2048 x 1536 shard."""
 import argparse
 import ctypes as C
 import json
@@ -22,7 +21,6 @@ sys.path.insert(0, ROOT)
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--variants', default='default')
-    ap.add_argument('--dbg', default='0')
     ap.add_argument('--ops', default='ah,wta,kl_uht,kl_wtu')
     ap.add_argument('--m', type=int, default=65536)
     ap.add_argument('--n', type=int, default=65536)
@@ -68,7 +66,7 @@ def main():
         nb = max(lib.dnmf_workspace_bytes(op, m, n, k, 0) for op in range(4))
         return torch.empty(nb, dtype=torch.uint8, device='cuda'), nb
 
-    # accuracy of every variant (flags 0) on a small shard
+    # accuracy of every variant on a small shard
     rs = np.random.RandomState(1)
     m0, n0 = 2048, 1536
     A0, W0, H0 = rs.rand(m0, n0).astype(np.float32), rs.rand(m0, k).astype(np.float32), rs.rand(k, n0).astype(np.float32)
@@ -80,8 +78,6 @@ def main():
     names = a.ops.split(',')
     for v, lib in libs.items():
         lib.dnmf_set_tc_min_elems(1)
-        if hasattr(lib, 'dnmf_set_tc_debug'):
-            lib.dnmf_set_tc_debug(0)
         o = outs(m0, n0)
         ws, wsb = workspace(lib, m0, n0)
         for nm in names:
@@ -96,10 +92,9 @@ def main():
     o = outs(a.m, a.n)
     gb = a.m * a.n * 4 / 1e9
     wss = {v: workspace(lib, a.m, a.n) for v, lib in libs.items()}
-    flags = [int(x, 0) for x in a.dbg.split(',')]
     first = a.variants.split(',')[0]
-    combos = [(v, fl, nm) for v in libs for fl in (flags if v == first else [0]) for nm in names]
-    # Every measurement is PAIRED with a reference launch (the first variant's FRO pass `ah`, flags 0) issued right
+    combos = [(v, nm) for v in libs for nm in names]
+    # Every measurement is PAIRED with a reference launch (the first variant's FRO pass `ah`) issued right
     # before it on the same stream with no host synchronisation in between: the whole round is one back-to-back queue
     # (sustained clocks, like the product's loop), the order of the combinations is reshuffled every round, and the
     # report is the median of the per-pair ratio t / t_ref next to the absolute times -- box drift cancels in the ratio.
@@ -112,21 +107,15 @@ def main():
         order = combos[:]
         rng.shuffle(order)
         evs = []
-        for (v, fl, nm) in order:
+        for (v, nm) in order:
             lib = libs[v]
             e0, e1, e2 = (torch.cuda.Event(enable_timing=True) for _ in range(3))
-            if hasattr(libs[first], 'dnmf_set_tc_debug'):
-                libs[first].dnmf_set_tc_debug(0)
             e0.record()
             run(libs[first], 'ah', A, W, H, o['ah'], *wss[first])
             e1.record()
-            if hasattr(lib, 'dnmf_set_tc_debug'):
-                lib.dnmf_set_tc_debug(fl)
             run(lib, nm, A, W, H, o[nm], *wss[v])
             e2.record()
-            if hasattr(lib, 'dnmf_set_tc_debug'):
-                lib.dnmf_set_tc_debug(0)
-            evs.append(((v, fl, nm), e0, e1, e2))
+            evs.append(((v, nm), e0, e1, e2))
         torch.cuda.synchronize()
         if rnd > 0:                          # round 0 = warm-up (attributes, calibration)
             for c, e0, e1, e2 in evs:
@@ -137,13 +126,12 @@ def main():
     print(json.dumps({'reference': first + ':ah', 'median_ms': statistics.median(ref_times), 'min_ms': min(ref_times),
                       'max_ms': max(ref_times)}), flush=True)
     for v in libs:
-        for fl in (flags if v == first else [0]):
-            rec = {'variant': v, 'dbg': fl}
-            for nm in names:
-                t = times[(v, fl, nm)]
-                rec[nm] = {'median_ms': statistics.median(t), 'min_ms': min(t), 'ratio_to_ref_median': statistics.median(ratios[(v, fl, nm)]),
-                           'GBps_median': gb / statistics.median(t) * 1e3}
-            print(json.dumps(rec), flush=True)
+        rec = {'variant': v}
+        for nm in names:
+            t = times[(v, nm)]
+            rec[nm] = {'median_ms': statistics.median(t), 'min_ms': min(t), 'ratio_to_ref_median': statistics.median(ratios[(v, nm)]),
+                       'GBps_median': gb / statistics.median(t) * 1e3}
+        print(json.dumps(rec), flush=True)
 
     if a.sustained:
         # Sustained blocks: `--sustained` back-to-back repetitions of the op list per variant with no host sync (what a

@@ -17,8 +17,6 @@ ap.add_argument('--n', type=int, default=32768)
 ap.add_argument('--k', type=int, default=32)
 ap.add_argument('--reps', type=int, default=3)
 ap.add_argument('--kl', action='store_true')
-ap.add_argument('--roles', action='store_true', help='print the per-warp-role cycle split of the tcgen05 kernel')
-ap.add_argument('--dbg', default='0', help='timing-ablation bits (dnmf_set_tc_debug) for the role timers')
 a = ap.parse_args()
 ops = D.default_ops()
 
@@ -51,39 +49,3 @@ for _ in range(a.reps):
     if a.kl:
         msg += '  kl_uht %.3f ms  kl_wtu %.3f ms' % (e[2].elapsed_time(e[3]), e[3].elapsed_time(e[4]))
     print(msg, flush=True)
-
-if a.roles:
-    from pydnmfk_b200 import _lib as L
-    names = ['A-prod wait a_free', 'A-prod issue', 'MMA wait acce', 'MMA wait t_full', 'MMA wait b_full', 'MMA issue', 'MMA commit',
-             'split wait a_full', 'split load+math', 'split wait t_free', 'split store', 'drain wait accf', 'drain work', '', '', 'total']
-    for nm, fn in (('ah', lambda: ops.ah(A, H)), ('wta', lambda: ops.wta(A, W))):
-        buf = torch.zeros(148 * 16, dtype=torch.int64, device='cuda')
-        L.call('dnmf_set_tc_profile', buf.data_ptr())
-        fn()
-        torch.cuda.synchronize()
-        L.call('dnmf_set_tc_profile', None)
-        v = buf.cpu().numpy().reshape(148, 16).astype(float)
-        tot = v[:, 15].mean()
-        print(nm, 'cycles per CTA %.0f' % tot)
-        for i, n in enumerate(names):
-            if n and i != 15:
-                print('   %-22s %5.1f%%' % (n, 100 * v[:, i].mean() / tot))
-
-if a.roles and a.kl:
-    from pydnmfk_b200 import _lib as L
-    L.call('dnmf_set_tc_debug', int(a.dbg, 0))
-    print('role timers with debug flags', a.dbg)
-    names = ['MMA gemm1 wait(Fr,S free)', 'MMA gemm1 issue', 'MMA wait acce', 'MMA wait t_full', 'MMA wait b_full', 'MMA gemm2 issue+loop',
-             'split wait a_full', 'split load A', 'split wait S', 'split ldtm+div+lo', 'split wait t_free', 'split store', '', '', '', 'total']
-    for nm, fn in (('kl_uht', lambda: ops.kl_uht(A, W, H, 1.2e-7)), ('kl_wtu', lambda: ops.kl_wtu(A, W, H, 1.2e-7))):
-        buf = torch.zeros(148 * 16, dtype=torch.int64, device='cuda')
-        L.call('dnmf_set_tc_profile', buf.data_ptr())
-        fn()
-        torch.cuda.synchronize()
-        L.call('dnmf_set_tc_profile', None)
-        v = buf.cpu().numpy().reshape(148, 16).astype(float)
-        tot = v[:, 15].mean()
-        print(nm, 'cycles per CTA %.0f' % tot)
-        for i, n in enumerate(names):
-            if n and i != 15:
-                print('   %-28s %5.1f%%' % (n, 100 * v[:, i].mean() / tot))
