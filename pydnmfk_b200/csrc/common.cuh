@@ -35,6 +35,19 @@ int cuda_fail(cudaError_t e, const char* where);
     if (_e != cudaSuccess) return ::dnmf::cuda_fail(_e, where);   \
   } while (0)
 
+// Raise kernel KERN's dynamic shared-memory limit to `bytes`, once per kernel: on its first launch, which is eager (never
+// during a stream capture).
+template <auto KERN>
+int smem_attr_once(int bytes, const char* where) {
+  static bool done = false;
+  if (!done) {
+    cudaError_t e = cudaFuncSetAttribute(KERN, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+    if (e != cudaSuccess) return cuda_fail(e, where);
+    done = true;
+  }
+  return 0;
+}
+
 int sm_count();
 
 inline int64_t ceil_div(int64_t a, int64_t b) { return (a + b - 1) / b; }

@@ -33,6 +33,47 @@ inline int check_a(int64_t m, int64_t n, int64_t k, int dtype) {
 // element size of the factors and outputs
 inline size_t esize(int dtype) { return dtype == DNMF_F64 ? 8 : 4; }
 
+// records which kernels serve an A-streaming pass (dnmf_last_path, dnmf_pass_count)
+void note_pass(bool tc) {
+  tls().last_path = tc ? 1 : 0;
+  (tc ? tls().tc_passes : tls().generic_passes)++;
+}
+
+// The A-streaming passes: AH (out = V = A H^T), WTA (out = Y = W^T A, or Y^T with transposed_out) and the KL forms
+// KL_UHT / KL_WTU (A / (W H + eps) in place of A); W (AH) and H (WTA) are not read.  view4 == nullptr: the plain entry
+// point, tcgen05 kernels when eligible, generic kernels otherwise.  view4 != nullptr: the _p form, which leaves the
+// split partials in the workspace and describes them in view4, and serves only calls the tcgen05 path takes.
+int run_pass(int op, const void* A, int64_t lda, const void* W, int64_t ldw, const void* H, int64_t ldh, void* out,
+             int64_t ldo, int64_t m, int64_t n, int64_t k, double eps, int transposed_out, int dtype, void* ws,
+             int64_t ws_bytes, int64_t* view4, cudaStream_t st) {
+  const bool kl = op == DNMF_OP_KL_UHT || op == DNMF_OP_KL_WTU;
+  const bool rows = op == DNMF_OP_AH || op == DNMF_OP_KL_UHT;    // one output row per row of A
+  const bool deferred = view4 != nullptr;
+  if (int rc = check_a(m, n, k, dtype)) return rc;
+  DNMF_CHECK_ARG(A && (op == DNMF_OP_AH || W) && (op == DNMF_OP_WTA || H) && (deferred || out), "null pointer");
+  DNMF_CHECK_ARG(lda >= n && (op == DNMF_OP_AH || ldw >= k) && (op == DNMF_OP_WTA || ldh >= n) &&
+                 (deferred || ldo >= (rows || transposed_out ? k : n)), "leading dimension too small");
+  if ((rows ? m : n) == 0 || k == 0) return deferred ? DNMF_E_UNSUPPORTED : 0;
+  const bool tc = tc_eligible(op, A, lda, m, n, k, dtype);
+  if (deferred && !tc) return DNMF_E_UNSUPPORTED;
+  note_pass(tc);
+  if (tc) {
+    TcPartials d;
+    if (int rc = tc_pass(op, dtype, A, lda, (const float*)W, ldw, (const float*)H, ldh, (float*)out, ldo, m, n, (int)k,
+                         (float)eps, transposed_out, ws, ws_bytes, st, deferred ? &d : nullptr))
+      return rc;
+    if (deferred) {
+      view4[0] = (int64_t)(uintptr_t)d.P; view4[1] = d.ldp; view4[2] = d.splits; view4[3] = d.split_stride;
+    }
+    return 0;
+  }
+  DISPATCH_A(dtype, {
+    if (rows) return row_pass_dispatch<T, TA>(kl, (const TA*)A, lda, (const T*)H, ldh, (const T*)W, ldw, (T*)out, ldo, m, n, (int)k, (T)eps, ws, ws_bytes, st);
+    return col_pass_dispatch<T, TA>(kl, (const TA*)A, lda, (const T*)W, ldw, (const T*)H, ldh, (T*)out, ldo, m, n, (int)k, (T)eps, transposed_out, ws, ws_bytes, st);
+  });
+  return 0;
+}
+
 }  // namespace
 
 extern "C" {
@@ -73,10 +114,6 @@ int64_t dnmf_workspace_bytes(int op, int64_t m, int64_t n, int64_t k, int dtype)
       const int64_t a = dnmf_workspace_bytes(DNMF_OP_AH, m, n, k, dtype);
       const int64_t r = dnmf_workspace_bytes(DNMF_OP_RESIDUAL, m, n, k, dtype);
       bytes = a > r ? a : r;
-      if (dtype == DNMF_F32 && k <= 32) {
-        const int64_t t = tc_ah_residual_workspace_bytes(m, n);
-        if (t > bytes) bytes = t;
-      }
       break;
     }
     case DNMF_OP_SUMS: {
@@ -104,79 +141,24 @@ int64_t dnmf_workspace_bytes(int op, int64_t m, int64_t n, int64_t k, int dtype)
 
 int dnmf_ah(const void* A, int64_t lda, const void* H, int64_t ldh, void* V, int64_t ldv, int64_t m, int64_t n,
             int64_t k, int dtype, int math_mode, void* ws, int64_t ws_bytes, void* stream) {
-  if (int rc = check_a(m, n, k, dtype)) return rc;
-  DNMF_CHECK_ARG(A && H && V, "null pointer");
-  DNMF_CHECK_ARG(lda >= n && ldh >= n && ldv >= k, "leading dimension too small");
-  if (m == 0 || k == 0) return 0;
-  cudaStream_t st = (cudaStream_t)stream;
-  if (tc_eligible(DNMF_OP_AH, A, lda, m, n, k, dtype)) {
-    tls().last_path = 1;
-    tls().tc_passes++;
-    if (is_a16(dtype)) return tc16_ah(A, lda, (const float*)H, ldh, (float*)V, ldv, m, n, (int)k, dtype, ws, ws_bytes, st);
-    return tc_ah((const float*)A, lda, (const float*)H, ldh, (float*)V, ldv, m, n, (int)k, math_mode, ws, ws_bytes, st);
-  }
-  tls().last_path = 0;
-  tls().generic_passes++;
-  DISPATCH_A(dtype, return row_pass_dispatch<T, TA>(false, (const TA*)A, lda, (const T*)H, ldh, (const T*)nullptr, 0, (T*)V, ldv, m, n, (int)k, T(0), ws, ws_bytes, st));
-  return 0;
+  return run_pass(DNMF_OP_AH, A, lda, nullptr, 0, H, ldh, V, ldv, m, n, k, 0.0, 0, dtype, ws, ws_bytes, nullptr, (cudaStream_t)stream);
 }
 
 int dnmf_wta(const void* A, int64_t lda, const void* W, int64_t ldw, void* Y, int64_t ldy, int64_t m, int64_t n,
              int64_t k, int transposed_out, int dtype, int math_mode, void* ws, int64_t ws_bytes, void* stream) {
-  if (int rc = check_a(m, n, k, dtype)) return rc;
-  DNMF_CHECK_ARG(A && W && Y, "null pointer");
-  DNMF_CHECK_ARG(lda >= n && ldw >= k && ldy >= (transposed_out ? k : n), "leading dimension too small");
-  if (n == 0 || k == 0) return 0;
-  cudaStream_t st = (cudaStream_t)stream;
-  if (tc_eligible(DNMF_OP_WTA, A, lda, m, n, k, dtype)) {
-    tls().last_path = 1;
-    tls().tc_passes++;
-    if (is_a16(dtype))
-      return tc16_wta(A, lda, (const float*)W, ldw, (float*)Y, ldy, m, n, (int)k, transposed_out, dtype, ws, ws_bytes, st);
-    return tc_wta((const float*)A, lda, (const float*)W, ldw, (float*)Y, ldy, m, n, (int)k, transposed_out, math_mode, ws, ws_bytes, st);
-  }
-  tls().last_path = 0;
-  tls().generic_passes++;
-  DISPATCH_A(dtype, return col_pass_dispatch<T, TA>(false, (const TA*)A, lda, (const T*)W, ldw, (const T*)nullptr, 0, (T*)Y, ldy, m, n, (int)k, T(0), transposed_out, ws, ws_bytes, st));
-  return 0;
+  return run_pass(DNMF_OP_WTA, A, lda, W, ldw, nullptr, 0, Y, ldy, m, n, k, 0.0, transposed_out, dtype, ws, ws_bytes, nullptr, (cudaStream_t)stream);
 }
 
 int dnmf_kl_uht(const void* A, int64_t lda, const void* W, int64_t ldw, const void* H, int64_t ldh, void* V,
                 int64_t ldv, int64_t m, int64_t n, int64_t k, double eps, int dtype, int math_mode, void* ws,
                 int64_t ws_bytes, void* stream) {
-  if (int rc = check_a(m, n, k, dtype)) return rc;
-  DNMF_CHECK_ARG(A && W && H && V, "null pointer");
-  DNMF_CHECK_ARG(lda >= n && ldh >= n && ldw >= k && ldv >= k, "leading dimension too small");
-  if (m == 0 || k == 0) return 0;
-  cudaStream_t st = (cudaStream_t)stream;
-  if (tc_eligible(DNMF_OP_KL_UHT, A, lda, m, n, k, dtype)) {
-    tls().last_path = 1;
-    tls().tc_passes++;
-    return tc_kl_uht((const float*)A, lda, (const float*)W, ldw, (const float*)H, ldh, (float*)V, ldv, m, n, (int)k, (float)eps, math_mode, ws, ws_bytes, st);
-  }
-  tls().last_path = 0;
-  tls().generic_passes++;
-  DISPATCH_A(dtype, return row_pass_dispatch<T, TA>(true, (const TA*)A, lda, (const T*)H, ldh, (const T*)W, ldw, (T*)V, ldv, m, n, (int)k, (T)eps, ws, ws_bytes, st));
-  return 0;
+  return run_pass(DNMF_OP_KL_UHT, A, lda, W, ldw, H, ldh, V, ldv, m, n, k, eps, 0, dtype, ws, ws_bytes, nullptr, (cudaStream_t)stream);
 }
 
 int dnmf_kl_wtu(const void* A, int64_t lda, const void* W, int64_t ldw, const void* H, int64_t ldh, void* Y,
                 int64_t ldy, int64_t m, int64_t n, int64_t k, double eps, int transposed_out, int dtype,
                 int math_mode, void* ws, int64_t ws_bytes, void* stream) {
-  if (int rc = check_a(m, n, k, dtype)) return rc;
-  DNMF_CHECK_ARG(A && W && H && Y, "null pointer");
-  DNMF_CHECK_ARG(lda >= n && ldh >= n && ldw >= k && ldy >= (transposed_out ? k : n), "leading dimension too small");
-  if (n == 0 || k == 0) return 0;
-  cudaStream_t st = (cudaStream_t)stream;
-  if (tc_eligible(DNMF_OP_KL_WTU, A, lda, m, n, k, dtype)) {
-    tls().last_path = 1;
-    tls().tc_passes++;
-    return tc_kl_wtu((const float*)A, lda, (const float*)W, ldw, (const float*)H, ldh, (float*)Y, ldy, m, n, (int)k, (float)eps, transposed_out, math_mode, ws, ws_bytes, st);
-  }
-  tls().last_path = 0;
-  tls().generic_passes++;
-  DISPATCH_A(dtype, return col_pass_dispatch<T, TA>(true, (const TA*)A, lda, (const T*)W, ldw, (const T*)H, ldh, (T*)Y, ldy, m, n, (int)k, (T)eps, transposed_out, ws, ws_bytes, st));
-  return 0;
+  return run_pass(DNMF_OP_KL_WTU, A, lda, W, ldw, H, ldh, Y, ldy, m, n, k, eps, transposed_out, dtype, ws, ws_bytes, nullptr, (cudaStream_t)stream);
 }
 
 int dnmf_gram(const void* X, int64_t ldx, int64_t rows, int64_t k, int trans, void* G, int dtype, void* ws,
@@ -280,67 +262,24 @@ int dnmf_kl_update_h(void* H, int64_t ldh, const void* Y, int64_t y_stride_k, in
 }
 
 // ---- deferred split reduction: pass -> partial view -> update that sums the splits itself -----------------------------
-namespace {
-int fill_view(const TcPartials& d, int64_t* view4) {
-  view4[0] = (int64_t)(uintptr_t)d.P; view4[1] = d.ldp; view4[2] = d.splits; view4[3] = d.split_stride;
-  return 0;
-}
-}  // namespace
-
 int dnmf_ah_p(const void* A, int64_t lda, const void* H, int64_t ldh, int64_t m, int64_t n, int64_t k, int dtype,
               int math_mode, void* ws, int64_t ws_bytes, int64_t* view4, void* stream) {
-  if (int rc = check_a(m, n, k, dtype)) return rc;
-  DNMF_CHECK_ARG(A && H && view4, "null pointer");
-  if (m == 0 || k == 0 || !tc_eligible(DNMF_OP_AH, A, lda, m, n, k, dtype)) return DNMF_E_UNSUPPORTED;
-  tls().last_path = 1;
-  tls().tc_passes++;
-  TcPartials d;
-  if (is_a16(dtype)) {
-    if (int rc = tc16_ah(A, lda, (const float*)H, ldh, nullptr, 0, m, n, (int)k, dtype, ws, ws_bytes, (cudaStream_t)stream, &d)) return rc;
-    return fill_view(d, view4);
-  }
-  if (int rc = tc_ah((const float*)A, lda, (const float*)H, ldh, nullptr, 0, m, n, (int)k, math_mode, ws, ws_bytes, (cudaStream_t)stream, &d)) return rc;
-  return fill_view(d, view4);
+  return run_pass(DNMF_OP_AH, A, lda, nullptr, 0, H, ldh, nullptr, 0, m, n, k, 0.0, 0, dtype, ws, ws_bytes, view4, (cudaStream_t)stream);
 }
 
 int dnmf_wta_p(const void* A, int64_t lda, const void* W, int64_t ldw, int64_t m, int64_t n, int64_t k, int dtype,
                int math_mode, void* ws, int64_t ws_bytes, int64_t* view4, void* stream) {
-  if (int rc = check_a(m, n, k, dtype)) return rc;
-  DNMF_CHECK_ARG(A && W && view4, "null pointer");
-  if (n == 0 || k == 0 || !tc_eligible(DNMF_OP_WTA, A, lda, m, n, k, dtype)) return DNMF_E_UNSUPPORTED;
-  tls().last_path = 1;
-  tls().tc_passes++;
-  TcPartials d;
-  if (is_a16(dtype)) {
-    if (int rc = tc16_wta(A, lda, (const float*)W, ldw, nullptr, 0, m, n, (int)k, 1, dtype, ws, ws_bytes, (cudaStream_t)stream, &d)) return rc;
-    return fill_view(d, view4);
-  }
-  if (int rc = tc_wta((const float*)A, lda, (const float*)W, ldw, nullptr, 0, m, n, (int)k, 1, math_mode, ws, ws_bytes, (cudaStream_t)stream, &d)) return rc;
-  return fill_view(d, view4);
+  return run_pass(DNMF_OP_WTA, A, lda, W, ldw, nullptr, 0, nullptr, 0, m, n, k, 0.0, 1, dtype, ws, ws_bytes, view4, (cudaStream_t)stream);
 }
 
 int dnmf_kl_uht_p(const void* A, int64_t lda, const void* W, int64_t ldw, const void* H, int64_t ldh, int64_t m, int64_t n,
                   int64_t k, double eps, int dtype, int math_mode, void* ws, int64_t ws_bytes, int64_t* view4, void* stream) {
-  if (int rc = check_a(m, n, k, dtype)) return rc;
-  DNMF_CHECK_ARG(A && W && H && view4, "null pointer");
-  if (m == 0 || k == 0 || !tc_eligible(DNMF_OP_KL_UHT, A, lda, m, n, k, dtype)) return DNMF_E_UNSUPPORTED;
-  tls().last_path = 1;
-  tls().tc_passes++;
-  TcPartials d;
-  if (int rc = tc_kl_uht((const float*)A, lda, (const float*)W, ldw, (const float*)H, ldh, nullptr, 0, m, n, (int)k, (float)eps, math_mode, ws, ws_bytes, (cudaStream_t)stream, &d)) return rc;
-  return fill_view(d, view4);
+  return run_pass(DNMF_OP_KL_UHT, A, lda, W, ldw, H, ldh, nullptr, 0, m, n, k, eps, 0, dtype, ws, ws_bytes, view4, (cudaStream_t)stream);
 }
 
 int dnmf_kl_wtu_p(const void* A, int64_t lda, const void* W, int64_t ldw, const void* H, int64_t ldh, int64_t m, int64_t n,
                   int64_t k, double eps, int dtype, int math_mode, void* ws, int64_t ws_bytes, int64_t* view4, void* stream) {
-  if (int rc = check_a(m, n, k, dtype)) return rc;
-  DNMF_CHECK_ARG(A && W && H && view4, "null pointer");
-  if (n == 0 || k == 0 || !tc_eligible(DNMF_OP_KL_WTU, A, lda, m, n, k, dtype)) return DNMF_E_UNSUPPORTED;
-  tls().last_path = 1;
-  tls().tc_passes++;
-  TcPartials d;
-  if (int rc = tc_kl_wtu((const float*)A, lda, (const float*)W, ldw, (const float*)H, ldh, nullptr, 0, m, n, (int)k, (float)eps, 1, math_mode, ws, ws_bytes, (cudaStream_t)stream, &d)) return rc;
-  return fill_view(d, view4);
+  return run_pass(DNMF_OP_KL_WTU, A, lda, W, ldw, H, ldh, nullptr, 0, m, n, k, eps, 1, dtype, ws, ws_bytes, view4, (cudaStream_t)stream);
 }
 
 #define DNMF_VIEW(view4)                                                                                         \
@@ -563,8 +502,7 @@ int dnmf_ah_residual(const void* A, int64_t lda, const void* W, int64_t ldw, con
   if (m > 0 && n > 0 && k >= 1 && k <= 32 && tc_eligible(DNMF_OP_KL_UHT, A, lda, m, n, k, dtype)) {
     double* pairs = nullptr;
     int64_t n_pairs = 0;
-    tls().last_path = 1;
-    tls().tc_passes++;
+    note_pass(true);
     if (int rc = tc_ah_residual_run((const float*)A, lda, (const float*)W, ldw, (const float*)H, ldh, (float*)V, ldv, m, n,
                                     (int)k, ws, ws_bytes, &pairs, &n_pairs, st))
       return rc;
@@ -572,7 +510,7 @@ int dnmf_ah_residual(const void* A, int64_t lda, const void* W, int64_t ldw, con
     DNMF_LAUNCH_CHECK("sum_pairs_kernel");
     return 0;
   }
-  if (int rc = dnmf_ah(A, lda, H, ldh, V, ldv, m, n, k, dtype, DNMF_MATH_ACCURATE, ws, ws_bytes, stream)) return rc;
+  if (int rc = run_pass(DNMF_OP_AH, A, lda, nullptr, 0, H, ldh, V, ldv, m, n, k, 0.0, 0, dtype, ws, ws_bytes, nullptr, st)) return rc;
   return dnmf_residual_sqnorm(A, lda, W, ldw, H, ldh, m, n, k, out, dtype, ws, ws_bytes, stream);
 }
 

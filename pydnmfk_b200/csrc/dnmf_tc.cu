@@ -358,23 +358,6 @@ EncodeTiledFn encode_fn() {
   return fn;
 }
 
-// 2-D fp32 row-major tensor [rows][cols] with leading dimension ld; box = {box_cols, box_rows}; 128B swizzle;
-// out-of-bounds elements read as zero (ragged edges need no special casing in the kernel)
-int make_map(CUtensorMap* map, const float* ptr, int64_t rows, int64_t cols, int64_t ld, int box_cols, int box_rows,
-             CUtensorMapSwizzle swz = CU_TENSOR_MAP_SWIZZLE_128B) {
-  EncodeTiledFn fn = encode_fn();
-  if (!fn) return fail(DNMF_E_UNSUPPORTED, "cuTensorMapEncodeTiled is not available from this driver");
-  cuuint64_t dims[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
-  cuuint64_t strides[1] = {(cuuint64_t)ld * sizeof(float)};
-  cuuint32_t box[2] = {(cuuint32_t)box_cols, (cuuint32_t)box_rows};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, (void*)ptr, dims, strides, box, estr,
-                  CU_TENSOR_MAP_INTERLEAVE_NONE, swz, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) return fail(DNMF_E_ARG, "cuTensorMapEncodeTiled failed with CUresult %d", (int)r);
-  return 0;
-}
-
 }  // namespace
 
 int tc_padded_k(int k) { return k <= 16 ? 16 : (k <= 32 ? 32 : 64); }
@@ -414,6 +397,48 @@ TcPlan tc_plan(int64_t x_len, int64_t r_len, int k, int bk) {
   return p;
 }
 
+int tc_begin(void* ws, int64_t ws_bytes, int64_t need, int64_t bcat_bytes, bool padded, cudaStream_t st) {
+  if (ws == nullptr || ws_bytes < need)
+    return fail(DNMF_E_WORKSPACE, "tcgen05 pass needs %lld workspace bytes, got %lld", (long long)need, (long long)ws_bytes);
+  if (((uintptr_t)ws % 256) != 0) return fail(DNMF_E_ARG, "workspace must be 256-byte aligned");
+  if (padded) {
+    cudaError_t e = cudaMemsetAsync(ws, 0, (size_t)bcat_bytes, st);
+    if (e != cudaSuccess) return cuda_fail(e, "Bcat memset");
+  }
+  return 0;
+}
+
+int tc_make_map(CUtensorMap* map, CUtensorMapDataType type, const void* ptr, int64_t rows, int64_t cols, int64_t ld,
+                int box_cols, int box_rows, CUtensorMapSwizzle swz) {
+  EncodeTiledFn fn = encode_fn();
+  if (!fn) return fail(DNMF_E_UNSUPPORTED, "cuTensorMapEncodeTiled is not available from this driver");
+  const int64_t esize = type == CU_TENSOR_MAP_DATA_TYPE_FLOAT32 ? 4 : 2;
+  cuuint64_t dims[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
+  cuuint64_t strides[1] = {(cuuint64_t)(ld * esize)};
+  cuuint32_t box[2] = {(cuuint32_t)box_cols, (cuuint32_t)box_rows};
+  cuuint32_t estr[2] = {1, 1};
+  CUresult r = fn(map, type, 2, const_cast<void*>(ptr), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, swz,
+                  CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  if (r != CUDA_SUCCESS) return fail(DNMF_E_ARG, "cuTensorMapEncodeTiled failed with CUresult %d", (int)r);
+  return 0;
+}
+
+int tc_map_a(CUtensorMap* map, const float* A, int64_t lda, int64_t m, int64_t n, int mode) {
+  if (mode == 1) return tc_make_map(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, A, m, n, lda, TC_BM, TC_BK, CU_TENSOR_MAP_SWIZZLE_NONE);
+  return tc_make_map(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, A, m, n, lda, TC_BK, TC_BM);
+}
+
+int tc_launch_split_h(const float* H, int64_t ldh, float* Bcat, int64_t ldb, int k, int kp, int64_t n, cudaStream_t st) {
+  tc_split_h_kernel<<<(unsigned)ceil_div((int64_t)k * n, 256), 256, 0, st>>>(H, ldh, Bcat, ldb, k, kp, n);
+  DNMF_LAUNCH_CHECK("tc_split_h_kernel");
+  return 0;
+}
+int tc_launch_split_wt(const float* W, int64_t ldw, float* Bcat, int64_t ldb, int k, int kp, int64_t m, cudaStream_t st) {
+  tc_split_wt_kernel<<<(unsigned)ceil_div(m, 64), 256, 0, st>>>(W, ldw, Bcat, ldb, k, kp, m);
+  DNMF_LAUNCH_CHECK("tc_split_wt_kernel");
+  return 0;
+}
+
 namespace {
 
 int g_tc_usable = -1;   // -1 not probed yet, 1 the tensor core truncates tf32 operands as the splitters assume, 0 it does not
@@ -422,15 +447,9 @@ int64_t g_min_elems = -1;
 template <int K, int MODE>
 int launch_pass(const CUtensorMap& tmA, const CUtensorMap& tmB, float* P, int64_t split_stride, int64_t x_len,
                 const TcPlan& pl, cudaStream_t st) {
-  auto kern = tc_pass_kernel<K, MODE>;
-  static bool attr_set = false;      // once per instantiation (and never during a stream capture)
-  if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, TcCfg<K>::SMEM_BYTES);
-    if (e != cudaSuccess) return cuda_fail(e, "tc_pass_kernel smem attribute");
-    attr_set = true;
-  }
-  kern<<<pl.grid, TcCfg<K>::THREADS, TcCfg<K>::SMEM_BYTES, st>>>(tmA, tmB, P, split_stride, x_len, pl.x_blocks, pl.kt_total,
-                                                            pl.kt_per_split, pl.num_units);
+  if (int rc = smem_attr_once<tc_pass_kernel<K, MODE>>(TcCfg<K>::SMEM_BYTES, "tc_pass_kernel smem attribute")) return rc;
+  tc_pass_kernel<K, MODE><<<pl.grid, TcCfg<K>::THREADS, TcCfg<K>::SMEM_BYTES, st>>>(
+      tmA, tmB, P, split_stride, x_len, pl.x_blocks, pl.kt_total, pl.kt_per_split, pl.num_units);
   DNMF_LAUNCH_CHECK("tc_pass_kernel");
   return 0;
 }
@@ -446,55 +465,43 @@ int launch_pass_k(int k, const CUtensorMap& tmA, const CUtensorMap& tmB, float* 
   return fail(DNMF_E_UNSUPPORTED, "tcgen05 path: k must be 16, 32 or 64");
 }
 
-// V (AH) or Y / Y^T (WTA) through the tensor path.  ws = [Bcat | partials]
+// ws = [Bcat | partials].  The kernels exist for 16 / 32 / 64 factor columns: smaller k ride along zero-padded.
+struct FroLayout {
+  TcPlan pl;
+  int kp;
+  int64_t total;
+};
+FroLayout fro_layout(int mode, int64_t m, int64_t n, int k) {
+  FroLayout L;
+  L.kp = tc_padded_k(k);
+  L.pl = mode == 0 ? tc_plan(m, n, L.kp) : tc_plan(n, m, L.kp);
+  L.total = L.pl.bcat_bytes + L.pl.partial_bytes;
+  return L;
+}
+
+// V (AH, mode 0) or Y / Y^T (WTA, mode 1) through the tensor path
 int tc_run(int mode, const float* A, int64_t lda, const float* B, int64_t ldbsrc, float* out, int64_t ldo,
            int64_t m, int64_t n, int k, int transposed_out, void* ws, int64_t ws_bytes, cudaStream_t st,
            TcPartials* defer) {
+  const FroLayout L = fro_layout(mode, m, n, k);
+  const TcPlan& pl = L.pl;
   const int64_t x_len = mode == 0 ? m : n;
   const int64_t r_len = mode == 0 ? n : m;
-  const int kp = tc_padded_k(k);      // the kernels exist for 16 / 32 / 64 factor columns: smaller k ride along zero-padded
-  const TcPlan pl = tc_plan(x_len, r_len, kp);
-  const int64_t need = pl.bcat_bytes + pl.partial_bytes;
-  if (ws == nullptr || ws_bytes < need)
-    return fail(DNMF_E_WORKSPACE, "tcgen05 pass needs %lld workspace bytes, got %lld", (long long)need, (long long)ws_bytes);
-  if (((uintptr_t)ws % 256) != 0) return fail(DNMF_E_ARG, "workspace must be 256-byte aligned");
+  if (int rc = tc_begin(ws, ws_bytes, L.total, pl.bcat_bytes, L.kp != k, st)) return rc;
   float* Bcat = reinterpret_cast<float*>(ws);
   float* P = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(ws) + pl.bcat_bytes);
-  if (kp != k) {
-    cudaError_t e = cudaMemsetAsync(Bcat, 0, (size_t)pl.bcat_bytes, st);
-    if (e != cudaSuccess) return cuda_fail(e, "Bcat memset");
-  }
-  if (mode == 0) {
-    tc_split_h_kernel<<<(unsigned)ceil_div((int64_t)k * n, 256), 256, 0, st>>>(B, ldbsrc, Bcat, pl.ldb, k, kp, n);
-    DNMF_LAUNCH_CHECK("tc_split_h_kernel");
-  } else {
-    tc_split_wt_kernel<<<(unsigned)ceil_div(m, 64), 256, 0, st>>>(B, ldbsrc, Bcat, pl.ldb, k, kp, m);
-    DNMF_LAUNCH_CHECK("tc_split_wt_kernel");
-  }
+  int rc = mode == 0 ? tc_launch_split_h(B, ldbsrc, Bcat, pl.ldb, k, L.kp, n, st)
+                     : tc_launch_split_wt(B, ldbsrc, Bcat, pl.ldb, k, L.kp, m, st);
+  if (rc) return rc;
   alignas(64) CUtensorMap tmA, tmB;
-  int rc;
-  if (mode == 0) rc = make_map(&tmA, A, m, n, lda, TC_BK, TC_BM);
-  else rc = make_map(&tmA, A, m, n, lda, TC_BM, TC_BK, CU_TENSOR_MAP_SWIZZLE_NONE);
+  if ((rc = tc_map_a(&tmA, A, lda, m, n, mode)) ||
+      (rc = tc_make_map(&tmB, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, Bcat, 2 * L.kp, r_len, pl.ldb, TC_BK, 2 * L.kp)))
+    return rc;
+  const int64_t split_stride = x_len * L.kp;
+  rc = mode == 0 ? launch_pass_k<0>(L.kp, tmA, tmB, P, split_stride, x_len, pl, st)
+                 : launch_pass_k<1>(L.kp, tmA, tmB, P, split_stride, x_len, pl, st);
   if (rc) return rc;
-  rc = make_map(&tmB, Bcat, 2 * kp, r_len, pl.ldb, TC_BK, 2 * kp);
-  if (rc) return rc;
-  const int64_t split_stride = x_len * kp;
-  rc = mode == 0 ? launch_pass_k<0>(kp, tmA, tmB, P, split_stride, x_len, pl, st)
-                 : launch_pass_k<1>(kp, tmA, tmB, P, split_stride, x_len, pl, st);
-  if (rc) return rc;
-  if (defer != nullptr) {      // the consumer (an update kernel) sums the splits itself, in the same order
-    defer->P = P; defer->ldp = kp; defer->split_stride = split_stride; defer->splits = pl.splits;
-    return 0;
-  }
-  // fixed-order sum of the split partials P[s][x][kk]  ->  out  (only the k real columns)
-  int64_t so_r, so_c;   // strides of (x, kk) in the output
-  if (mode == 0) { so_r = ldo; so_c = 1; }                        // V[x][kk]
-  else if (transposed_out) { so_r = ldo; so_c = 1; }              // Y^T[x][kk]
-  else { so_r = 1; so_c = ldo; }                                  // Y[kk][x]
-  reduce_partials_kernel<float><<<(unsigned)ceil_div(x_len * k, 256), 256, 0, st>>>(P, split_stride, pl.splits, x_len, k,
-                                                                                     out, so_r, so_c, kp);
-  DNMF_LAUNCH_CHECK("reduce_partials_kernel");
-  return 0;
+  return tc_finish(P, x_len, L.kp, pl.splits, mode, k, transposed_out, out, ldo, st, defer);
 }
 
 // One-time probe: does kind::tf32 truncate the fp32 bits it reads, as the splitters assume?  A = 1 + 1.5 * 2^-11
@@ -503,8 +510,7 @@ void calibrate() {
   if (g_tc_usable >= 0) return;
   g_tc_usable = 0;
   const int m = 128, n = 32, k = 16;
-  const TcPlan pl = tc_plan(m, n, k);
-  const int64_t wsb = pl.bcat_bytes + pl.partial_bytes;
+  const int64_t wsb = fro_layout(0, m, n, k).total;
   float *dA = nullptr, *dH = nullptr, *dV = nullptr;
   void* dws = nullptr;
   if (cudaMalloc(&dA, m * n * 4) != cudaSuccess || cudaMalloc(&dH, k * n * 4) != cudaSuccess ||
@@ -555,34 +561,6 @@ bool device_is_sm100() {
 
 }  // namespace
 
-int tc_make_map(CUtensorMap* map, const float* ptr, int64_t rows, int64_t cols, int64_t ld, int box_cols, int box_rows,
-                CUtensorMapSwizzle swz) {
-  return make_map(map, ptr, rows, cols, ld, box_cols, box_rows, swz);
-}
-// the same for a 16-bit (fp16 / bf16) row-major tensor, 128-byte swizzle (dnmf_tc16.cu)
-int tc_make_map_16(CUtensorMap* map, const void* ptr, int64_t rows, int64_t cols, int64_t ld, int box_cols, int box_rows,
-                   int bf16) {
-  EncodeTiledFn fn = encode_fn();
-  if (!fn) return fail(DNMF_E_UNSUPPORTED, "cuTensorMapEncodeTiled is not available from this driver");
-  cuuint64_t dims[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
-  cuuint64_t strides[1] = {(cuuint64_t)ld * 2};
-  cuuint32_t box[2] = {(cuuint32_t)box_cols, (cuuint32_t)box_rows};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = fn(map, bf16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, const_cast<void*>(ptr),
-                  dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
-                  CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) return fail(DNMF_E_ARG, "cuTensorMapEncodeTiled failed with CUresult %d", (int)r);
-  return 0;
-}
-void tc_launch_split_h(const float* H, int64_t ldh, float* Bcat, int64_t ldb, int k, int kp, int64_t n, cudaStream_t st) {
-  tc_split_h_kernel<<<(unsigned)ceil_div((int64_t)k * n, 256), 256, 0, st>>>(H, ldh, Bcat, ldb, k, kp, n);
-  tls().launches++;
-}
-void tc_launch_split_wt(const float* W, int64_t ldw, float* Bcat, int64_t ldb, int k, int kp, int64_t m, cudaStream_t st) {
-  tc_split_wt_kernel<<<(unsigned)ceil_div(m, 64), 256, 0, st>>>(W, ldw, Bcat, ldb, k, kp, m);
-  tls().launches++;
-}
-
 bool tc_eligible(int op, const void* A, int64_t lda, int64_t m, int64_t n, int64_t k, int dtype) {
   if (tls().force_generic) return false;
   const bool kl = (op == DNMF_OP_KL_UHT || op == DNMF_OP_KL_WTU);
@@ -597,7 +575,6 @@ bool tc_eligible(int op, const void* A, int64_t lda, int64_t m, int64_t n, int64
     if (((uintptr_t)A % 16) != 0 || (lda % 8) != 0) return false;
     return m * n >= g_min_elems && device_is_sm100();
   }
-  if (kl && !tc_kl_supported(k) && !tc_kl_supported_k64(k)) return false;
   if (dtype != DNMF_F32) return false;
   if (k < 1 || k > 64) return false;
   if (((uintptr_t)A % 16) != 0 || (lda % 4) != 0) return false;
@@ -610,36 +587,29 @@ bool tc_eligible(int op, const void* A, int64_t lda, int64_t m, int64_t n, int64
 void tc_set_min_elems(int64_t elems) { g_min_elems = elems < 0 ? 0 : elems; }
 
 int64_t tc_workspace_bytes(int op, int64_t m, int64_t n, int64_t k, int dtype) {
-  if ((dtype == DNMF_A_F16 || dtype == DNMF_A_BF16) && k >= 1 && k <= 64) return tc16_workspace_bytes(op, m, n, k, dtype);
-  if (dtype != DNMF_F32 || k < 1 || k > 64) return 0;
-  if (op == DNMF_OP_AH) { const TcPlan p = tc_plan(m, n, tc_padded_k((int)k)); return p.bcat_bytes + p.partial_bytes; }
-  if (op == DNMF_OP_WTA) { const TcPlan p = tc_plan(n, m, tc_padded_k((int)k)); return p.bcat_bytes + p.partial_bytes; }
-  if ((op == DNMF_OP_KL_UHT || op == DNMF_OP_KL_WTU) && tc_kl_supported(k)) return tc_kl_workspace_bytes(op, m, n, k);
-  if ((op == DNMF_OP_KL_UHT || op == DNMF_OP_KL_WTU) && tc_kl_supported_k64(k)) return tc_kl_workspace_bytes_k64(op, m, n, k);
+  if (op == DNMF_OP_AH_RESIDUAL) return dtype == DNMF_F32 && k <= 32 ? tc_kl_layout(3, m, n).total : 0;
+  const bool a16 = dtype == DNMF_A_F16 || dtype == DNMF_A_BF16;
+  if ((dtype != DNMF_F32 && !a16) || k < 1 || k > 64) return 0;
+  const int mode = (op == DNMF_OP_AH || op == DNMF_OP_KL_UHT) ? 0 : 1;
+  if (op == DNMF_OP_AH || op == DNMF_OP_WTA)
+    return a16 ? tc16_layout(mode, m, n, (int)k, dtype).total : fro_layout(mode, m, n, (int)k).total;
+  if ((op == DNMF_OP_KL_UHT || op == DNMF_OP_KL_WTU) && !a16)
+    return k > 32 ? tc_kl_layout_k64(mode, m, n).total : tc_kl_layout(mode, m, n).total;
   return 0;
 }
 
-int tc_ah(const float* A, int64_t lda, const float* H, int64_t ldh, float* V, int64_t ldv, int64_t m, int64_t n, int k,
-          int math_mode, void* ws, int64_t ws_bytes, cudaStream_t st, TcPartials* defer) {
-  return tc_run(0, A, lda, H, ldh, V, ldv, m, n, k, 0, ws, ws_bytes, st, defer);
-}
-
-int tc_wta(const float* A, int64_t lda, const float* W, int64_t ldw, float* Y, int64_t ldy, int64_t m, int64_t n, int k,
-           int transposed_out, int math_mode, void* ws, int64_t ws_bytes, cudaStream_t st, TcPartials* defer) {
-  return tc_run(1, A, lda, W, ldw, Y, ldy, m, n, k, transposed_out, ws, ws_bytes, st, defer);
-}
-
-int tc_kl_uht(const float* A, int64_t lda, const float* W, int64_t ldw, const float* H, int64_t ldh, float* V, int64_t ldv,
-              int64_t m, int64_t n, int k, float eps, int math_mode, void* ws, int64_t ws_bytes, cudaStream_t st,
-              TcPartials* defer) {
-  if (k > 32) return tc_kl_run_k64(0, A, lda, W, ldw, H, ldh, V, ldv, m, n, k, eps, 0, ws, ws_bytes, st, defer);
-  return tc_kl_run(0, A, lda, W, ldw, H, ldh, V, ldv, m, n, k, eps, 0, ws, ws_bytes, st, defer);
-}
-int tc_kl_wtu(const float* A, int64_t lda, const float* W, int64_t ldw, const float* H, int64_t ldh, float* Y, int64_t ldy,
-              int64_t m, int64_t n, int k, float eps, int transposed_out, int math_mode, void* ws, int64_t ws_bytes,
-              cudaStream_t st, TcPartials* defer) {
-  if (k > 32) return tc_kl_run_k64(1, A, lda, W, ldw, H, ldh, Y, ldy, m, n, k, eps, transposed_out, ws, ws_bytes, st, defer);
-  return tc_kl_run(1, A, lda, W, ldw, H, ldh, Y, ldy, m, n, k, eps, transposed_out, ws, ws_bytes, st, defer);
+int tc_pass(int op, int dtype, const void* A, int64_t lda, const float* W, int64_t ldw, const float* H, int64_t ldh,
+            float* out, int64_t ldo, int64_t m, int64_t n, int k, float eps, int transposed_out, void* ws,
+            int64_t ws_bytes, cudaStream_t st, TcPartials* defer) {
+  const int mode = (op == DNMF_OP_AH || op == DNMF_OP_KL_UHT) ? 0 : 1;
+  if (op == DNMF_OP_KL_UHT || op == DNMF_OP_KL_WTU)
+    return (k > 32 ? tc_kl_run_k64 : tc_kl_run)(mode, (const float*)A, lda, W, ldw, H, ldh, out, ldo, m, n, k, eps,
+                                                 transposed_out, ws, ws_bytes, st, defer);
+  const float* B = mode == 0 ? H : W;          // the small operand: H (AH) or W (WTA)
+  const int64_t ldbsrc = mode == 0 ? ldh : ldw;
+  if (dtype == DNMF_A_F16 || dtype == DNMF_A_BF16)
+    return tc16_run(mode, A, lda, B, ldbsrc, out, ldo, m, n, k, transposed_out, dtype, ws, ws_bytes, st, defer);
+  return tc_run(mode, (const float*)A, lda, B, ldbsrc, out, ldo, m, n, k, transposed_out, ws, ws_bytes, st, defer);
 }
 
 }  // namespace dnmf

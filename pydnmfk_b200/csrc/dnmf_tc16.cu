@@ -31,9 +31,6 @@
 
 namespace dnmf {
 
-int tc_make_map_16(CUtensorMap* map, const void* ptr, int64_t rows, int64_t cols, int64_t ld, int box_cols, int box_rows,
-                   int bf16);
-
 namespace {
 
 constexpr int TC16_BK = 64;       // reduced-dimension tile: 64 16-bit elements = one 128-byte swizzle row = 4 MMA K steps
@@ -315,15 +312,11 @@ __global__ void __launch_bounds__(256) tc16_split_kernel(const float* __restrict
   }
 }
 
-// ---------------------------------------------------------------------------------------------------------
-// host side.  Workspace = [Bcat | amax[64] + s[64] | partials]
-// ---------------------------------------------------------------------------------------------------------
-struct Tc16Layout {
-  TcPlan pl;
-  int kp, np;
-  int64_t ldb, bcat_bytes, aux_bytes, total;
-};
+}  // namespace
 
+// ---------------------------------------------------------------------------------------------------------
+// host side
+// ---------------------------------------------------------------------------------------------------------
 Tc16Layout tc16_layout(int mode, int64_t m, int64_t n, int k, int dtype) {
   Tc16Layout L;
   const int64_t x_len = mode == 0 ? m : n;
@@ -338,18 +331,15 @@ Tc16Layout tc16_layout(int mode, int64_t m, int64_t n, int k, int dtype) {
   return L;
 }
 
+namespace {
+
 template <int KP, int NP, int MODE>
 int launch16(const CUtensorMap& tmA, const CUtensorMap& tmB, const int* sexp, float* P, int64_t split_stride,
              int64_t x_len, const TcPlan& pl, cudaStream_t st) {
-  auto kern = tc16_pass_kernel<KP, NP, MODE>;
-  static bool attr_set = false;      // once per instantiation (and never during a stream capture)
-  if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Tc16Cfg<KP, NP>::SMEM_BYTES);
-    if (e != cudaSuccess) return cuda_fail(e, "tc16_pass_kernel smem attribute");
-    attr_set = true;
-  }
-  kern<<<pl.grid, TC16_THREADS, Tc16Cfg<KP, NP>::SMEM_BYTES, st>>>(tmA, tmB, sexp, P, split_stride, x_len, pl.x_blocks,
-                                                                   pl.kt_total, pl.kt_per_split, pl.num_units);
+  using Cfg = Tc16Cfg<KP, NP>;
+  if (int rc = smem_attr_once<tc16_pass_kernel<KP, NP, MODE>>(Cfg::SMEM_BYTES, "tc16_pass_kernel smem attribute")) return rc;
+  tc16_pass_kernel<KP, NP, MODE><<<pl.grid, TC16_THREADS, Cfg::SMEM_BYTES, st>>>(
+      tmA, tmB, sexp, P, split_stride, x_len, pl.x_blocks, pl.kt_total, pl.kt_per_split, pl.num_units);
   DNMF_LAUNCH_CHECK("tc16_pass_kernel");
   return 0;
 }
@@ -365,6 +355,8 @@ int launch16_k(int kp, const CUtensorMap& tmA, const CUtensorMap& tmB, const int
   return fail(DNMF_E_UNSUPPORTED, "tcgen05 kind::f16 path: k must be padded to 16, 32 or 64");
 }
 
+}  // namespace
+
 int tc16_run(int mode, const void* A, int64_t lda, const float* B, int64_t ldbsrc, float* out, int64_t ldo, int64_t m,
              int64_t n, int k, int transposed_out, int dtype, void* ws, int64_t ws_bytes, cudaStream_t st,
              TcPartials* defer) {
@@ -372,19 +364,12 @@ int tc16_run(int mode, const void* A, int64_t lda, const float* B, int64_t ldbsr
   const TcPlan& pl = L.pl;
   const int64_t x_len = mode == 0 ? m : n;
   const int64_t r_len = mode == 0 ? n : m;
-  if (ws == nullptr || ws_bytes < L.total)
-    return fail(DNMF_E_WORKSPACE, "tcgen05 kind::f16 pass needs %lld workspace bytes, got %lld", (long long)L.total,
-                (long long)ws_bytes);
-  if (((uintptr_t)ws % 256) != 0) return fail(DNMF_E_ARG, "workspace must be 256-byte aligned");
+  if (int rc = tc_begin(ws, ws_bytes, L.total, L.bcat_bytes, L.kp != k, st)) return rc;
   uint8_t* w8 = reinterpret_cast<uint8_t*>(ws);
   uint16_t* Bcat = reinterpret_cast<uint16_t*>(w8);
   unsigned* amax = reinterpret_cast<unsigned*>(w8 + L.bcat_bytes);
   int* sexp = reinterpret_cast<int*>(w8 + L.bcat_bytes + 256);
   float* P = reinterpret_cast<float*>(w8 + L.bcat_bytes + L.aux_bytes);
-  if (L.kp != k) {
-    cudaError_t e = cudaMemsetAsync(Bcat, 0, (size_t)L.bcat_bytes, st);
-    if (e != cudaSuccess) return cuda_fail(e, "Bcat memset");
-  }
   const int64_t sj = mode == 0 ? ldbsrc : 1, sc = mode == 0 ? 1 : ldbsrc;
   const int row_major = mode == 0 ? 1 : 0;
   const int64_t total = (int64_t)k * r_len;
@@ -403,47 +388,17 @@ int tc16_run(int mode, const void* A, int64_t lda, const float* B, int64_t ldbsr
   }
   DNMF_LAUNCH_CHECK("tc16_split_kernel");
   alignas(64) CUtensorMap tmA, tmB;
-  const int bf16 = dtype == DNMF_A_BF16 ? 1 : 0;
-  int rc = mode == 0 ? tc_make_map_16(&tmA, A, m, n, lda, TC16_BK, TC_BM, bf16)
-                     : tc_make_map_16(&tmA, A, m, n, lda, 64, TC16_BK, bf16);
-  if (rc) return rc;
-  rc = tc_make_map_16(&tmB, Bcat, (int64_t)L.np * L.kp, r_len, L.ldb, TC16_BK, L.np * L.kp, bf16);
-  if (rc) return rc;
+  const CUtensorMapDataType type = dtype == DNMF_A_BF16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16;
+  int rc = mode == 0 ? tc_make_map(&tmA, type, A, m, n, lda, TC16_BK, TC_BM)
+                     : tc_make_map(&tmA, type, A, m, n, lda, 64, TC16_BK);
+  if (rc || (rc = tc_make_map(&tmB, type, Bcat, (int64_t)L.np * L.kp, r_len, L.ldb, TC16_BK, L.np * L.kp))) return rc;
   const int64_t split_stride = x_len * L.kp;
   if (L.np == 2) rc = mode == 0 ? launch16_k<2, 0>(L.kp, tmA, tmB, sexp, P, split_stride, x_len, pl, st)
                                 : launch16_k<2, 1>(L.kp, tmA, tmB, sexp, P, split_stride, x_len, pl, st);
   else rc = mode == 0 ? launch16_k<3, 0>(L.kp, tmA, tmB, sexp, P, split_stride, x_len, pl, st)
                       : launch16_k<3, 1>(L.kp, tmA, tmB, sexp, P, split_stride, x_len, pl, st);
   if (rc) return rc;
-  if (defer != nullptr) {      // the consumer (an update kernel or the exchange) sums the splits itself, in the same order
-    defer->P = P; defer->ldp = L.kp; defer->split_stride = split_stride; defer->splits = pl.splits;
-    return 0;
-  }
-  int64_t so_r, so_c;   // strides of (x, kk) in the output
-  if (mode == 0 || transposed_out) { so_r = ldo; so_c = 1; }
-  else { so_r = 1; so_c = ldo; }
-  reduce_partials_kernel<float><<<(unsigned)ceil_div(x_len * k, 256), 256, 0, st>>>(P, split_stride, pl.splits, x_len, k,
-                                                                                     out, so_r, so_c, L.kp);
-  DNMF_LAUNCH_CHECK("reduce_partials_kernel");
-  return 0;
-}
-
-}  // namespace
-
-int64_t tc16_workspace_bytes(int op, int64_t m, int64_t n, int64_t k, int dtype) {
-  if (op == DNMF_OP_AH) return tc16_layout(0, m, n, (int)k, dtype).total;
-  if (op == DNMF_OP_WTA) return tc16_layout(1, m, n, (int)k, dtype).total;
-  return 0;
-}
-
-int tc16_ah(const void* A, int64_t lda, const float* H, int64_t ldh, float* V, int64_t ldv, int64_t m, int64_t n, int k,
-            int dtype, void* ws, int64_t ws_bytes, cudaStream_t st, TcPartials* defer) {
-  return tc16_run(0, A, lda, H, ldh, V, ldv, m, n, k, 0, dtype, ws, ws_bytes, st, defer);
-}
-
-int tc16_wta(const void* A, int64_t lda, const float* W, int64_t ldw, float* Y, int64_t ldy, int64_t m, int64_t n, int k,
-             int transposed_out, int dtype, void* ws, int64_t ws_bytes, cudaStream_t st, TcPartials* defer) {
-  return tc16_run(1, A, lda, W, ldw, Y, ldy, m, n, k, transposed_out, dtype, ws, ws_bytes, st, defer);
+  return tc_finish(P, x_len, L.kp, pl.splits, mode, k, transposed_out, out, ldo, st, defer);
 }
 
 }  // namespace dnmf

@@ -495,66 +495,63 @@ __global__ void __launch_bounds__(256) kl_transpose_kernel(const float* __restri
   }
 }
 
-struct KlPlan {
-  TcPlan base;
-  int64_t r_pad, frcat_bytes, ht_bytes;
-};
-
-KlPlan kl_plan(int mode, int64_t m, int64_t n) {       // every size is for the padded factor width KK
-  KlPlan p;
-  const int64_t x_len = mode == 0 ? m : n, r_len = mode == 0 ? n : m;
-  p.base = tc_plan(x_len, r_len, KK);
-  p.r_pad = round_up(r_len, 64);
-  p.frcat_bytes = round_up(2 * p.r_pad * KK * 4, 1024);
-  p.ht_bytes = round_up(n * (int64_t)KK * 4, 1024);      // plain H^T (Fx of WTU)
-  return p;
+template <int MODE>
+int kl_launch(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMap& tmF, const float* Fx, int64_t ldfx,
+              const KlLayout& L, float* P, int64_t x_len, int k_real, float eps, double* pairs, cudaStream_t st) {
+  if (int rc = smem_attr_once<tc_kl_kernel<MODE>>(KlCfg::SMEM_BYTES, "tc_kl_kernel smem attribute")) return rc;
+  tc_kl_kernel<MODE><<<L.pl.grid, KlCfg::THREADS, KlCfg::SMEM_BYTES, st>>>(
+      tmA, tmB, tmF, Fx, ldfx, L.r_pad, P, x_len * KK, x_len, L.pl.x_blocks, L.pl.kt_total, L.pl.kt_per_split,
+      L.pl.num_units, k_real, eps, pairs);
+  DNMF_LAUNCH_CHECK("tc_kl_kernel");
+  return 0;
 }
 
 }  // namespace
 
-bool KL_FN(tc_kl_supported)(int64_t k) { return k >= 1 && k <= KK; }
-
-int64_t KL_FN(tc_kl_workspace_bytes)(int op, int64_t m, int64_t n, int64_t k) {
-  const KlPlan p = kl_plan(op == DNMF_OP_KL_UHT ? 0 : 1, m, n);
-  return p.base.bcat_bytes + p.frcat_bytes + p.ht_bytes + p.base.partial_bytes;
+// every size is for the padded factor width KK
+KlLayout KL_FN(tc_kl_layout)(int mode, int64_t m, int64_t n) {
+  KlLayout L;
+  const int64_t x_len = mode == 1 ? n : m, r_len = mode == 1 ? m : n;
+  L.pl = tc_plan(x_len, r_len, KK);
+  L.r_pad = round_up(r_len, 64);
+  L.frcat_bytes = round_up(2 * L.r_pad * KK * 4, 1024);
+  L.ht_bytes = mode == 3 ? 0 : round_up(n * (int64_t)KK * 4, 1024);      // plain H^T (Fx of WTU)
+  L.pairs_bytes = mode == 3 ? round_up((int64_t)L.pl.grid * KlCfg::PAIRS * 2 * (int64_t)sizeof(double), 1024) : 0;
+  L.total = L.pl.bcat_bytes + L.frcat_bytes + L.ht_bytes + L.pl.partial_bytes + L.pairs_bytes;
+  return L;
 }
 
-// ws = [Bcat | FrCat | Ht | partials].  The kernel is written for KK = 32 factor columns; smaller k ride along zero-padded
-// (zero columns of W / rows of H add nothing to S = W H, and their output columns are dropped by the final reduction).
+// The kernel is written for KK factor columns; smaller k ride along zero-padded (zero columns of W / rows of H add nothing
+// to S = W H, and their output columns are dropped by the final reduction).
 int KL_FN(tc_kl_run)(int mode, const float* A, int64_t lda, const float* W, int64_t ldw, const float* H, int64_t ldh, float* out,
                      int64_t ldo, int64_t m, int64_t n, int k, float eps, int transposed_out, void* ws, int64_t ws_bytes,
                      cudaStream_t st, TcPartials* defer) {
   if (k < 1 || k > KK) return fail(DNMF_E_UNSUPPORTED, "tcgen05 KL path: k must be in [1, %d]", KK);
-  const KlPlan kp = kl_plan(mode, m, n);
-  const TcPlan& pl = kp.base;
-  const int64_t x_len = mode == 0 ? m : n, r_len = mode == 0 ? n : m;
-  const int64_t need = pl.bcat_bytes + kp.frcat_bytes + kp.ht_bytes + pl.partial_bytes;
-  if (ws == nullptr || ws_bytes < need)
-    return fail(DNMF_E_WORKSPACE, "tcgen05 KL pass needs %lld workspace bytes, got %lld", (long long)need, (long long)ws_bytes);
-  if (((uintptr_t)ws % 256) != 0) return fail(DNMF_E_ARG, "workspace must be 256-byte aligned");
+  const KlLayout L = KL_FN(tc_kl_layout)(mode, m, n);
+  const TcPlan& pl = L.pl;
+  const int64_t x_len = mode == 1 ? n : m, r_len = mode == 1 ? m : n;
+  if (int rc = tc_begin(ws, ws_bytes, L.total, pl.bcat_bytes, k != KK, st)) return rc;
   uint8_t* wsb = reinterpret_cast<uint8_t*>(ws);
   float* Bcat = reinterpret_cast<float*>(wsb);
   float* FrCat = reinterpret_cast<float*>(wsb + pl.bcat_bytes);
-  float* Ht = reinterpret_cast<float*>(wsb + pl.bcat_bytes + kp.frcat_bytes);
-  float* P = reinterpret_cast<float*>(wsb + pl.bcat_bytes + kp.frcat_bytes + kp.ht_bytes);
-  const unsigned fr_blocks = (unsigned)ceil_div(kp.r_pad, 64);
-  if (k != KK) {
-    cudaError_t e = cudaMemsetAsync(Bcat, 0, (size_t)pl.bcat_bytes, st);
-    if (e != cudaSuccess) return cuda_fail(e, "Bcat memset");
-  }
+  float* Ht = reinterpret_cast<float*>(wsb + pl.bcat_bytes + L.frcat_bytes);
+  float* P = reinterpret_cast<float*>(wsb + pl.bcat_bytes + L.frcat_bytes + L.ht_bytes);
+  double* pairs = mode == 3 ? reinterpret_cast<double*>(wsb + L.total - L.pairs_bytes) : nullptr;
+  const unsigned fr_blocks = (unsigned)ceil_div(L.r_pad, 64);
   const float* Fx;
   int64_t ldfx;
-  if (mode == 0) {
-    // UHT: GEMM2 B = split(H); GEMM1 r-side factor = H^T rows (columns of A); x-side factor = W rows
-    tc_launch_split_h(H, ldh, Bcat, pl.ldb, k, KK, n, st);
-    kl_split_fr_kernel<true><<<fr_blocks, 256, 0, st>>>(H, ldh, FrCat, r_len, kp.r_pad, k);
+  int rc;
+  if (mode != 1) {
+    // UHT (and mode 3): GEMM2 B = split(H); GEMM1 r-side factor = H^T rows (columns of A); x-side factor = W rows
+    if ((rc = tc_launch_split_h(H, ldh, Bcat, pl.ldb, k, KK, n, st))) return rc;
+    kl_split_fr_kernel<true><<<fr_blocks, 256, 0, st>>>(H, ldh, FrCat, r_len, L.r_pad, k);
     DNMF_LAUNCH_CHECK("kl_split_fr_kernel<T>");
     Fx = W;
     ldfx = ldw;
   } else {
     // WTU: GEMM2 B = split(W^T); GEMM1 r-side factor = W rows; x-side factor = H^T rows (columns of A)
-    tc_launch_split_wt(W, ldw, Bcat, pl.ldb, k, KK, m, st);
-    kl_split_fr_kernel<false><<<fr_blocks, 256, 0, st>>>(W, ldw, FrCat, r_len, kp.r_pad, k);
+    if ((rc = tc_launch_split_wt(W, ldw, Bcat, pl.ldb, k, KK, m, st))) return rc;
+    kl_split_fr_kernel<false><<<fr_blocks, 256, 0, st>>>(W, ldw, FrCat, r_len, L.r_pad, k);
     DNMF_LAUNCH_CHECK("kl_split_fr_kernel<N>");
     kl_transpose_kernel<<<(unsigned)ceil_div(n, 64), 256, 0, st>>>(H, ldh, Ht, n, k);    // H^T [n x KK], zero padded
     DNMF_LAUNCH_CHECK("kl_transpose_kernel");
@@ -562,102 +559,35 @@ int KL_FN(tc_kl_run)(int mode, const float* A, int64_t lda, const float* W, int6
     ldfx = KK;
   }
   alignas(64) CUtensorMap tmA, tmB, tmF;
-  int rc;
-  if (mode == 0) rc = tc_make_map(&tmA, A, m, n, lda, TC_BK, TC_BM, CU_TENSOR_MAP_SWIZZLE_128B);
-  else rc = tc_make_map(&tmA, A, m, n, lda, TC_BM, TC_BK, CU_TENSOR_MAP_SWIZZLE_NONE);
-  if (rc) return rc;
-  rc = tc_make_map(&tmB, Bcat, 2 * KK, r_len, pl.ldb, TC_BK, 2 * KK, CU_TENSOR_MAP_SWIZZLE_128B);
-  if (rc) return rc;
-  rc = tc_make_map(&tmF, FrCat, 2 * kp.r_pad, KK, KK, 32, KlCfg::F_ROWS, CU_TENSOR_MAP_SWIZZLE_128B);
-  if (rc) return rc;
-  const int64_t split_stride = x_len * KK;
+  if ((rc = tc_map_a(&tmA, A, lda, m, n, mode)) ||
+      (rc = tc_make_map(&tmB, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, Bcat, 2 * KK, r_len, pl.ldb, TC_BK, 2 * KK)) ||
+      (rc = tc_make_map(&tmF, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, FrCat, 2 * L.r_pad, KK, KK, 32, KlCfg::F_ROWS)))
+    return rc;
   // (for UHT the x-side factor rows are read straight from W with its own leading dimension: only k_real columns exist)
-  const int k_real = mode == 0 ? k : KK;
-  auto launch = [&](auto kern) -> int {
-    static bool attr_set[2] = {false, false};
-    if (!attr_set[mode]) {
-      cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, KlCfg::SMEM_BYTES);
-      if (e != cudaSuccess) return cuda_fail(e, "tc_kl_kernel smem attribute");
-      attr_set[mode] = true;
-    }
-    kern<<<pl.grid, KlCfg::THREADS, KlCfg::SMEM_BYTES, st>>>(tmA, tmB, tmF, Fx, ldfx, kp.r_pad, P, split_stride, x_len,
-                                                              pl.x_blocks, pl.kt_total, pl.kt_per_split, pl.num_units,
-                                                              k_real, eps, nullptr);
-    DNMF_LAUNCH_CHECK("tc_kl_kernel");
-    return 0;
-  };
-  rc = mode == 0 ? launch(tc_kl_kernel<0>) : launch(tc_kl_kernel<1>);
-  if (rc) return rc;
-  if (defer != nullptr) {      // the consumer sums the splits itself, in the same order
-    defer->P = P; defer->ldp = KK; defer->split_stride = split_stride; defer->splits = pl.splits;
-    return 0;
+  const int k_real = mode == 1 ? KK : k;
+  switch (mode) {
+    case 0: rc = kl_launch<0>(tmA, tmB, tmF, Fx, ldfx, L, P, x_len, k_real, eps, pairs, st); break;
+    case 1: rc = kl_launch<1>(tmA, tmB, tmF, Fx, ldfx, L, P, x_len, k_real, eps, pairs, st); break;
+#if KL_KK == 32      // the residual variant (BCD, k <= 32) exists in the 32-wide build only
+    case 3: rc = kl_launch<3>(tmA, tmB, tmF, Fx, ldfx, L, P, x_len, k_real, eps, pairs, st); break;
+#endif
+    default: return fail(DNMF_E_UNSUPPORTED, "tcgen05 KL path: no kernel for mode %d", mode);
   }
-  int64_t so_r, so_c;
-  if (mode == 0) { so_r = ldo; so_c = 1; }
-  else if (transposed_out) { so_r = ldo; so_c = 1; }
-  else { so_r = 1; so_c = ldo; }
-  reduce_partials_kernel<float><<<(unsigned)ceil_div(x_len * k, 256), 256, 0, st>>>(P, split_stride, pl.splits, x_len, k, out,
-                                                                                     so_r, so_c, KK);
-  DNMF_LAUNCH_CHECK("reduce_partials_kernel");
-  return 0;
+  if (rc) return rc;
+  return tc_finish(P, x_len, KK, pl.splits, mode == 1 ? 1 : 0, k, transposed_out, out, ldo, st, defer);
 }
 
-#if KL_KK == 32      // the residual variants (BCD, k <= 32) exist in the 32-wide build only
+#if KL_KK == 32
 // ---- V = A H^T together with ||A - W H||^2 and ||A||^2 in ONE pass over A (MODE 3) -------------------------------------
-// ws = [Bcat | FrCat | partials | pairs (grid x 256 x 2 float64)]
-int64_t tc_ah_residual_workspace_bytes(int64_t m, int64_t n) {
-  const KlPlan p = kl_plan(0, m, n);
-  return p.base.bcat_bytes + p.frcat_bytes + p.base.partial_bytes +
-         round_up((int64_t)p.base.grid * KlCfg::PAIRS * 2 * (int64_t)sizeof(double), 1024);
-}
-
 int tc_ah_residual_run(const float* A, int64_t lda, const float* W, int64_t ldw, const float* H, int64_t ldh, float* V,
                        int64_t ldv, int64_t m, int64_t n, int k, void* ws, int64_t ws_bytes, double** out_pairs,
                        int64_t* n_pairs, cudaStream_t st) {
-  if (k < 1 || k > KK) return fail(DNMF_E_UNSUPPORTED, "tcgen05 A H^T + residual: k must be in [1, %d]", KK);
-  const KlPlan kp = kl_plan(0, m, n);
-  const TcPlan& pl = kp.base;
-  const int64_t need = tc_ah_residual_workspace_bytes(m, n);
-  if (ws == nullptr || ws_bytes < need)
-    return fail(DNMF_E_WORKSPACE, "tcgen05 A H^T + residual needs %lld workspace bytes, got %lld", (long long)need, (long long)ws_bytes);
-  if (((uintptr_t)ws % 256) != 0) return fail(DNMF_E_ARG, "workspace must be 256-byte aligned");
-  uint8_t* wsb = reinterpret_cast<uint8_t*>(ws);
-  float* Bcat = reinterpret_cast<float*>(wsb);
-  float* FrCat = reinterpret_cast<float*>(wsb + pl.bcat_bytes);
-  float* P = reinterpret_cast<float*>(wsb + pl.bcat_bytes + kp.frcat_bytes);
-  double* pairs = reinterpret_cast<double*>(wsb + pl.bcat_bytes + kp.frcat_bytes + pl.partial_bytes);
-  if (k != KK) {
-    cudaError_t e = cudaMemsetAsync(Bcat, 0, (size_t)pl.bcat_bytes, st);
-    if (e != cudaSuccess) return cuda_fail(e, "Bcat memset");
-  }
-  tc_launch_split_h(H, ldh, Bcat, pl.ldb, k, KK, n, st);
-  kl_split_fr_kernel<true><<<(unsigned)ceil_div(kp.r_pad, 64), 256, 0, st>>>(H, ldh, FrCat, n, kp.r_pad, k);
-  DNMF_LAUNCH_CHECK("kl_split_fr_kernel<T>");
-  alignas(64) CUtensorMap tmA, tmB, tmF;
-  int rc = tc_make_map(&tmA, A, m, n, lda, TC_BK, TC_BM, CU_TENSOR_MAP_SWIZZLE_128B);
-  if (rc) return rc;
-  rc = tc_make_map(&tmB, Bcat, 2 * KK, n, pl.ldb, TC_BK, 2 * KK, CU_TENSOR_MAP_SWIZZLE_128B);
-  if (rc) return rc;
-  rc = tc_make_map(&tmF, FrCat, 2 * kp.r_pad, KK, KK, 32, KlCfg::F_ROWS, CU_TENSOR_MAP_SWIZZLE_128B);
-  if (rc) return rc;
-  auto kern = tc_kl_kernel<3>;
-  static bool attr_set = false;
-  if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, KlCfg::SMEM_BYTES);
-    if (e != cudaSuccess) return cuda_fail(e, "tc_kl_kernel<3> smem attribute");
-    attr_set = true;
-  }
-  const int64_t split_stride = m * KK;
-  kern<<<pl.grid, KlCfg::THREADS, KlCfg::SMEM_BYTES, st>>>(tmA, tmB, tmF, W, ldw, kp.r_pad, P, split_stride, m, pl.x_blocks,
-                                                            pl.kt_total, pl.kt_per_split, pl.num_units, k, 0.f, pairs);
-  DNMF_LAUNCH_CHECK("tc_kl_kernel<3>");
-  reduce_partials_kernel<float><<<(unsigned)ceil_div(m * k, 256), 256, 0, st>>>(P, split_stride, pl.splits, m, k, V, ldv, 1, KK);
-  DNMF_LAUNCH_CHECK("reduce_partials_kernel");
-  *out_pairs = pairs;
-  *n_pairs = (int64_t)pl.grid * KlCfg::PAIRS;
+  if (int rc = tc_kl_run(3, A, lda, W, ldw, H, ldh, V, ldv, m, n, k, 0.f, 0, ws, ws_bytes, st, nullptr)) return rc;
+  const KlLayout L = tc_kl_layout(3, m, n);
+  *out_pairs = reinterpret_cast<double*>(reinterpret_cast<uint8_t*>(ws) + L.total - L.pairs_bytes);
+  *n_pairs = (int64_t)L.pl.grid * KlCfg::PAIRS;
   return 0;
 }
-
 #endif  // KL_KK == 32
 
 }  // namespace dnmf

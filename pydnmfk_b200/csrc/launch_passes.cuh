@@ -29,12 +29,13 @@ Split col_pass_plan(int64_t m, int64_t n) {
   return plan_split(n, (int64_t)kColPassThreads * ColPassCfg<T, KP, KL>::CPT, m, kColPassBR, kColPassBR);
 }
 
+// fixed-order sum of split partials with rows ldp apart (see reduce_partials_kernel)
 template <typename T>
-inline int launch_reduce(const T* P, int64_t split_stride, int splits, int64_t R, int64_t C, T* out, int64_t so_r,
-                  int64_t so_c, cudaStream_t st) {
+inline int launch_reduce(const T* P, int64_t split_stride, int splits, int64_t R, int64_t C, int64_t ldp, T* out,
+                         int64_t so_r, int64_t so_c, cudaStream_t st) {
   const int64_t tot = R * C;
   if (tot == 0) return 0;
-  reduce_partials_kernel<T><<<(unsigned)ceil_div(tot, 256), 256, 0, st>>>(P, split_stride, splits, R, C, out, so_r, so_c, C);
+  reduce_partials_kernel<T><<<(unsigned)ceil_div(tot, 256), 256, 0, st>>>(P, split_stride, splits, R, C, out, so_r, so_c, ldp);
   DNMF_LAUNCH_CHECK("reduce_partials_kernel");
   return 0;
 }
@@ -47,12 +48,8 @@ int run_row_pass(const TA* A, int64_t lda, const T* H, int64_t ldh, const T* W, 
   const Split sp = row_pass_plan<T, KP, KL>(m, n);
   const int vec_ok = (((uintptr_t)A % (Cfg::VN * sizeof(TA))) == 0) && (lda % Cfg::VN == 0);
   auto kern = row_pass_kernel<T, KP, KL, TA>;
-  static bool attr_set = false;
-  if (Cfg::smem_bytes > 48 * 1024 && !attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::smem_bytes);
-    if (e != cudaSuccess) return cuda_fail(e, "row_pass smem attribute");
-    attr_set = true;
-  }
+  if (Cfg::smem_bytes > 48 * 1024)
+    if (int rc = smem_attr_once<row_pass_kernel<T, KP, KL, TA>>((int)Cfg::smem_bytes, "row_pass smem attribute")) return rc;
   dim3 grid((unsigned)sp.blocks, (unsigned)sp.splits);
   if (sp.splits == 1) {
     kern<<<grid, kRowPassThreads, Cfg::smem_bytes, st>>>(A, lda, H, ldh, W, ldw, V, ldv, 0, m, n, k, sp.chunk, eps, vec_ok);
@@ -64,7 +61,7 @@ int run_row_pass(const TA* A, int64_t lda, const T* H, int64_t ldh, const T* W, 
   T* P = reinterpret_cast<T*>(ws);
   kern<<<grid, kRowPassThreads, Cfg::smem_bytes, st>>>(A, lda, H, ldh, W, ldw, P, k, m * k, m, n, k, sp.chunk, eps, vec_ok);
   DNMF_LAUNCH_CHECK("row_pass_kernel");
-  return launch_reduce<T>(P, m * k, (int)sp.splits, m, k, V, ldv, 1, st);
+  return launch_reduce<T>(P, m * k, (int)sp.splits, m, k, k, V, ldv, 1, st);
 }
 
 // Y[k x n] = W^T A  or  W^T (A/(WH+eps));  transposed_out: Y^T [n x k]
@@ -86,8 +83,8 @@ int run_col_pass(const TA* A, int64_t lda, const T* W, int64_t ldw, const T* H, 
   T* P = reinterpret_cast<T*>(ws);
   col_pass_kernel<T, KP, KL, TA><<<grid, kColPassThreads, 0, st>>>(A, lda, W, ldw, H, ldh, P, n, (int64_t)k * n, m, n, k, sp.chunk, eps, vec_ok);
   DNMF_LAUNCH_CHECK("col_pass_kernel");
-  if (transposed_out) return launch_reduce<T>(P, (int64_t)k * n, (int)sp.splits, k, n, Y, 1, ldy, st);
-  return launch_reduce<T>(P, (int64_t)k * n, (int)sp.splits, k, n, Y, ldy, 1, st);
+  if (transposed_out) return launch_reduce<T>(P, (int64_t)k * n, (int)sp.splits, k, n, n, Y, 1, ldy, st);
+  return launch_reduce<T>(P, (int64_t)k * n, (int)sp.splits, k, n, n, Y, ldy, 1, st);
 }
 
 

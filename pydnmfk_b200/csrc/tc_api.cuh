@@ -9,6 +9,8 @@ namespace dnmf {
 // AH / WTA only, lda % 8 == 0 (the kind::f16 kernels of dnmf_tc16.cu).
 bool tc_eligible(int op, const void* A, int64_t lda, int64_t m, int64_t n, int64_t k, int dtype);
 void tc_set_min_elems(int64_t elems);
+// workspace bytes of the tcgen05 pass for (op, dtype), 0 when there is none; DNMF_OP_AH_RESIDUAL: the fused pass of
+// tc_ah_residual_run
 int64_t tc_workspace_bytes(int op, int64_t m, int64_t n, int64_t k, int dtype);
 
 // Split-K partials an A-streaming pass leaves in its workspace when the final reduction is deferred to the consumer:
@@ -19,28 +21,16 @@ struct TcPartials {
   int splits = 0;
 };
 
-// (`defer` != nullptr: skip the final reduce_partials launch and describe the partials instead; `out` is then unused)
-int tc_ah(const float* A, int64_t lda, const float* H, int64_t ldh, float* V, int64_t ldv, int64_t m, int64_t n,
-          int k, int math_mode, void* ws, int64_t ws_bytes, cudaStream_t st, TcPartials* defer = nullptr);
-int tc_wta(const float* A, int64_t lda, const float* W, int64_t ldw, float* Y, int64_t ldy, int64_t m, int64_t n,
-           int k, int transposed_out, int math_mode, void* ws, int64_t ws_bytes, cudaStream_t st, TcPartials* defer = nullptr);
-int tc_kl_uht(const float* A, int64_t lda, const float* W, int64_t ldw, const float* H, int64_t ldh, float* V,
-              int64_t ldv, int64_t m, int64_t n, int k, float eps, int math_mode, void* ws, int64_t ws_bytes,
-              cudaStream_t st, TcPartials* defer = nullptr);
-int tc_kl_wtu(const float* A, int64_t lda, const float* W, int64_t ldw, const float* H, int64_t ldh, float* Y,
-              int64_t ldy, int64_t m, int64_t n, int k, float eps, int transposed_out, int math_mode, void* ws,
-              int64_t ws_bytes, cudaStream_t st, TcPartials* defer = nullptr);
-
-// 16-bit A (dtype DNMF_A_F16 / DNMF_A_BF16), fp32 factors and outputs: the tcgen05 kind::f16 kernels of dnmf_tc16.cu
-int64_t tc16_workspace_bytes(int op, int64_t m, int64_t n, int64_t k, int dtype);
-int tc16_ah(const void* A, int64_t lda, const float* H, int64_t ldh, float* V, int64_t ldv, int64_t m, int64_t n, int k,
-            int dtype, void* ws, int64_t ws_bytes, cudaStream_t st, TcPartials* defer = nullptr);
-int tc16_wta(const void* A, int64_t lda, const float* W, int64_t ldw, float* Y, int64_t ldy, int64_t m, int64_t n, int k,
-             int transposed_out, int dtype, void* ws, int64_t ws_bytes, cudaStream_t st, TcPartials* defer = nullptr);
+// One A-streaming pass on the tcgen05 kernels, for a call tc_eligible accepted: op DNMF_OP_AH (out = V = A H^T),
+// DNMF_OP_WTA (out = Y = W^T A, or Y^T with transposed_out), DNMF_OP_KL_UHT / DNMF_OP_KL_WTU (the same with A / (W H + eps)
+// in place of A).  A is fp32 or, for AH / WTA, 16-bit (dtype).  `defer` != nullptr: skip the final reduction and
+// describe the partials instead; `out` is then unused.
+int tc_pass(int op, int dtype, const void* A, int64_t lda, const float* W, int64_t ldw, const float* H, int64_t ldh,
+            float* out, int64_t ldo, int64_t m, int64_t n, int k, float eps, int transposed_out, void* ws,
+            int64_t ws_bytes, cudaStream_t st, TcPartials* defer);
 
 // V = A H^T plus ||A - W H||^2, ||A||^2 in one pass (fp32, k <= 32): per-thread float64 pairs in the workspace, to be
 // summed by the caller in a fixed order
-int64_t tc_ah_residual_workspace_bytes(int64_t m, int64_t n);
 int tc_ah_residual_run(const float* A, int64_t lda, const float* W, int64_t ldw, const float* H, int64_t ldh, float* V,
                        int64_t ldv, int64_t m, int64_t n, int k, void* ws, int64_t ws_bytes, double** out_pairs,
                        int64_t* n_pairs, cudaStream_t st);

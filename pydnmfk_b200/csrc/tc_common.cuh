@@ -4,6 +4,8 @@
 #include <cuda.h>
 
 #include "common.cuh"
+#include "launch_passes.cuh"
+#include "tc_api.cuh"
 
 namespace dnmf {
 
@@ -352,10 +354,10 @@ __device__ __forceinline__ void tf32_lo_bits2(uint32_t raw0, uint32_t raw1, uint
 
 }  // namespace
 
-// ---- host helpers defined in dnmf_tc.cu ------------------------------------------------------------------
-// 2-D fp32 row-major tensor map [rows][cols] with leading dimension ld, box {box_cols, box_rows}; OOB reads are zero
-int tc_make_map(CUtensorMap* map, const float* ptr, int64_t rows, int64_t cols, int64_t ld, int box_cols, int box_rows,
-                CUtensorMapSwizzle swz);
+// ---------------------------------------------------------------------------------------------------------
+// host side: planning and the launch skeleton shared by the drivers tc_run (dnmf_tc.cu), tc16_run (dnmf_tc16.cu),
+// tc_kl_run (dnmf_tc_kl.cu; also the A H^T + residual pass) -- defined in dnmf_tc.cu unless inline
+// ---------------------------------------------------------------------------------------------------------
 struct TcPlan {
   int x_blocks, kt_total, kt_per_split, splits, num_units, grid;
   int64_t ldb;            // leading dimension of Bcat (reduced length rounded up to 4)
@@ -365,22 +367,58 @@ int tc_padded_k(int k);
 // bk: reduced-dimension elements per tile (TC_BK fp32, TC16_BK for a 16-bit A)
 TcPlan tc_plan(int64_t x_len, int64_t r_len, int k, int bk = TC_BK);
 
-// small-operand split kernels (dnmf_tc.cu)
-void tc_launch_split_h(const float* H, int64_t ldh, float* Bcat, int64_t ldb, int k, int kp, int64_t n, cudaStream_t st);
-void tc_launch_split_wt(const float* W, int64_t ldw, float* Bcat, int64_t ldb, int k, int kp, int64_t m, cudaStream_t st);
+// Start of a pass: the workspace must hold `need` bytes at 256-byte alignment; its first `bcat_bytes` (the split factor
+// Bcat) are zeroed when the kernel runs on zero-padded factor rows.
+int tc_begin(void* ws, int64_t ws_bytes, int64_t need, int64_t bcat_bytes, bool padded, cudaStream_t st);
+// 2-D row-major tensor map [rows][cols] of `type` (fp32, fp16 or bf16) elements with leading dimension ld, box
+// {box_cols, box_rows}; out-of-bounds elements read as zero (ragged edges need no special casing in the kernels)
+int tc_make_map(CUtensorMap* map, CUtensorMapDataType type, const void* ptr, int64_t rows, int64_t cols, int64_t ld,
+                int box_cols, int box_rows, CUtensorMapSwizzle swz = CU_TENSOR_MAP_SWIZZLE_128B);
+// the map of an fp32 A: mode 1 (WTA / WTU, x = columns of A) MN-major tiles, box {TC_BM, TC_BK}, no swizzle; any other
+// mode (x = rows of A) K-major tiles, box {TC_BK, TC_BM}, 128-byte swizzle
+int tc_map_a(CUtensorMap* map, const float* A, int64_t lda, int64_t m, int64_t n, int mode);
+// End of a pass: the split partials P[split][x][kp] are described in *defer, or summed in a fixed order into the k real
+// columns of out: V[x][kk] (mode 0), Y[kk][x] (mode 1) or Y^T[x][kk] (mode 1, transposed_out).  Inline, so that every
+// driver's translation unit keeps its own reduce_partials_kernel.
+inline int tc_finish(float* P, int64_t x_len, int kp, int splits, int mode, int k, int transposed_out, float* out,
+                     int64_t ldo, cudaStream_t st, TcPartials* defer) {
+  const int64_t split_stride = x_len * kp;
+  if (defer != nullptr) {
+    defer->P = P; defer->ldp = kp; defer->split_stride = split_stride; defer->splits = splits;
+    return 0;
+  }
+  const bool x_rows = mode == 0 || transposed_out;   // x indexes the rows of out
+  return launch_reduce<float>(P, split_stride, splits, x_len, k, kp, out, x_rows ? ldo : 1, x_rows ? 1 : ldo, st);
+}
 
-// fused KL contractions (dnmf_tc_kl.cu)
-int64_t tc_kl_workspace_bytes(int op, int64_t m, int64_t n, int64_t k);
-bool tc_kl_supported(int64_t k);
-// the 64-wide build (dnmf_tc_kl64.cu): 32 < k <= 64
-int64_t tc_kl_workspace_bytes_k64(int op, int64_t m, int64_t n, int64_t k);
-bool tc_kl_supported_k64(int64_t k);
-struct TcPartials;
+// small-operand split kernels (dnmf_tc.cu)
+int tc_launch_split_h(const float* H, int64_t ldh, float* Bcat, int64_t ldb, int k, int kp, int64_t n, cudaStream_t st);
+int tc_launch_split_wt(const float* W, int64_t ldw, float* Bcat, int64_t ldb, int k, int kp, int64_t m, cudaStream_t st);
+
+// 16-bit A (dtype DNMF_A_F16 / DNMF_A_BF16), fp32 factors and outputs (dnmf_tc16.cu).  ws = [Bcat | amax + s | partials]
+struct Tc16Layout {
+  TcPlan pl;
+  int kp, np;
+  int64_t ldb, bcat_bytes, aux_bytes, total;
+};
+Tc16Layout tc16_layout(int mode, int64_t m, int64_t n, int k, int dtype);
+int tc16_run(int mode, const void* A, int64_t lda, const float* B, int64_t ldbsrc, float* out, int64_t ldo, int64_t m,
+             int64_t n, int k, int transposed_out, int dtype, void* ws, int64_t ws_bytes, cudaStream_t st,
+             TcPartials* defer);
+
+// fused KL contractions (dnmf_tc_kl.cu: k <= 32; the _k64 build, dnmf_tc_kl64.cu: 32 < k <= 64).  mode 0 UHT, 1 WTU,
+// 3 A H^T + residual (32-wide build only).  ws = [Bcat | FrCat | Ht (modes 0, 1) | partials | residual pairs (mode 3)]
+struct KlLayout {
+  TcPlan pl;
+  int64_t r_pad, frcat_bytes, ht_bytes, pairs_bytes, total;
+};
+KlLayout tc_kl_layout(int mode, int64_t m, int64_t n);
+KlLayout tc_kl_layout_k64(int mode, int64_t m, int64_t n);
 int tc_kl_run(int mode, const float* A, int64_t lda, const float* W, int64_t ldw, const float* H, int64_t ldh, float* out,
               int64_t ldo, int64_t m, int64_t n, int k, float eps, int transposed_out, void* ws, int64_t ws_bytes,
-              cudaStream_t st, TcPartials* defer = nullptr);
+              cudaStream_t st, TcPartials* defer);
 int tc_kl_run_k64(int mode, const float* A, int64_t lda, const float* W, int64_t ldw, const float* H, int64_t ldh, float* out,
                   int64_t ldo, int64_t m, int64_t n, int k, float eps, int transposed_out, void* ws, int64_t ws_bytes,
-                  cudaStream_t st, TcPartials* defer = nullptr);
+                  cudaStream_t st, TcPartials* defer);
 
 }  // namespace dnmf
