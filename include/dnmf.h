@@ -40,9 +40,11 @@ extern "C" {
  * is fp32 (dnmf_compact: 16-bit in, 16-bit out).  Only the entry points that read A accept these codes:
  *   dnmf_workspace_bytes, dnmf_ah[_p], dnmf_wta[_p], dnmf_kl_uht[_p], dnmf_kl_wtu[_p], dnmf_residual_sqnorm,
  *   dnmf_ah_residual, dnmf_column_err, dnmf_sqnorm (for ||A||^2), dnmf_nnz_counts, dnmf_compact.
- * Every other entry point rejects them with DNMF_E_ARG.  dnmf_ah / dnmf_wta (and their _p forms) run on the tcgen05
- * kind::f16 kernel (dnmf_tc16.cu) for 16-byte aligned shards with lda % 8 == 0, >= 2^20 elements and k <= 64; the
- * KL contractions and everything else stream the 16-bit shard through the generic CUDA-core kernels.
+ * Every other entry point rejects them with DNMF_E_ARG.  For 16-byte aligned shards with lda % 8 == 0, >= 2^20 elements
+ * and k <= 64 the passes run on tcgen05 kernels: dnmf_ah / dnmf_wta (and their _p forms) on the kind::f16 kernel
+ * (dnmf_tc16.cu); dnmf_kl_uht / dnmf_kl_wtu (and their _p forms) and, for k <= 32, dnmf_ah_residual on the 16-bit build
+ * of the fused KL kernel (dnmf_tc_kl.cu), bit-identical to the same call on the fp32 copy of A.  Other shards, and
+ * everything else, stream the 16-bit shard through the generic CUDA-core kernels.
  * (2 is DNMF_I64, which the collectives accept, so the 16-bit codes start at 3.) */
 #define DNMF_A_F16 3
 #define DNMF_A_BF16 4
@@ -298,8 +300,8 @@ int dnmf_mu_fit_resident(const void* const* A_ptrs, int64_t lda, void* const* W_
                          int64_t m, int64_t n, int64_t k, int kl, int w_update, int64_t it_begin, int64_t it_end,
                          double eps, int dtype, void* stream);
 
-/* V = A H^T and out[0] = ||A - W H||_F^2, out[1] = ||A||_F^2 in ONE pass over A (fp32, k <= 32: tcgen05 kernel that
- * recomputes each W H tile on the tensor cores like the KL path; otherwise the two separate passes): the BCD iteration's
+/* V = A H^T and out[0] = ||A - W H||_F^2, out[1] = ||A||_F^2 in ONE pass over A (fp32 or 16-bit A, k <= 32: tcgen05 kernel
+ * that recomputes each W H tile on the tensor cores like the KL path; otherwise the two separate passes): the BCD iteration's
  * dist_nmf.py:1023 (A H^T) and :1024 (objective), which the reference runs as two passes plus an m x n temporary. */
 int dnmf_ah_residual(const void* A, int64_t lda, const void* W, int64_t ldw, const void* H, int64_t ldh, void* V,
                      int64_t ldv, int64_t m, int64_t n, int64_t k, double* out, int dtype, void* ws, int64_t ws_bytes,

@@ -503,7 +503,7 @@ int dnmf_ah_residual(const void* A, int64_t lda, const void* W, int64_t ldw, con
     double* pairs = nullptr;
     int64_t n_pairs = 0;
     note_pass(true);
-    if (int rc = tc_ah_residual_run((const float*)A, lda, (const float*)W, ldw, (const float*)H, ldh, (float*)V, ldv, m, n,
+    if (int rc = tc_ah_residual_run(A, dtype, lda, (const float*)W, ldw, (const float*)H, ldh, (float*)V, ldv, m, n,
                                     (int)k, ws, ws_bytes, &pairs, &n_pairs, st))
       return rc;
     sum_pairs_kernel<<<1, 256, 0, st>>>(pairs, n_pairs, out);

@@ -423,9 +423,13 @@ int tc_make_map(CUtensorMap* map, CUtensorMapDataType type, const void* ptr, int
   return 0;
 }
 
-int tc_map_a(CUtensorMap* map, const float* A, int64_t lda, int64_t m, int64_t n, int mode) {
-  if (mode == 1) return tc_make_map(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, A, m, n, lda, TC_BM, TC_BK, CU_TENSOR_MAP_SWIZZLE_NONE);
-  return tc_make_map(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, A, m, n, lda, TC_BK, TC_BM);
+int tc_map_a(CUtensorMap* map, const void* A, int dtype, int64_t lda, int64_t m, int64_t n, int mode) {
+  const CUtensorMapDataType type = dtype == DNMF_A_F16    ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16
+                                   : dtype == DNMF_A_BF16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16
+                                                          : CU_TENSOR_MAP_DATA_TYPE_FLOAT32;
+  if (mode == 1) return tc_make_map(map, type, A, m, n, lda, TC_BM, TC_BK, CU_TENSOR_MAP_SWIZZLE_NONE);
+  return tc_make_map(map, type, A, m, n, lda, TC_BK, TC_BM,
+                     dtype == DNMF_F32 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B);
 }
 
 int tc_launch_split_h(const float* H, int64_t ldh, float* Bcat, int64_t ldb, int k, int kp, int64_t n, cudaStream_t st) {
@@ -494,7 +498,7 @@ int tc_run(int mode, const float* A, int64_t lda, const float* B, int64_t ldbsrc
                      : tc_launch_split_wt(B, ldbsrc, Bcat, pl.ldb, k, L.kp, m, st);
   if (rc) return rc;
   alignas(64) CUtensorMap tmA, tmB;
-  if ((rc = tc_map_a(&tmA, A, lda, m, n, mode)) ||
+  if ((rc = tc_map_a(&tmA, A, DNMF_F32, lda, m, n, mode)) ||
       (rc = tc_make_map(&tmB, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, Bcat, 2 * L.kp, r_len, pl.ldb, TC_BK, 2 * L.kp)))
     return rc;
   const int64_t split_stride = x_len * L.kp;
@@ -570,10 +574,14 @@ bool tc_eligible(int op, const void* A, int64_t lda, int64_t m, int64_t n, int64
     g_min_elems = env ? atoll(env) : (int64_t)1 << 20;
   }
   if (dtype == DNMF_A_F16 || dtype == DNMF_A_BF16) {
-    // 16-bit A: the kind::f16 kernel of dnmf_tc16.cu (AH / WTA only; an exact operand, no tf32 calibration involved)
-    if (kl || k < 1 || k > 64) return false;
+    if (k < 1 || k > 64) return false;
     if (((uintptr_t)A % 16) != 0 || (lda % 8) != 0) return false;
-    return m * n >= g_min_elems && device_is_sm100();
+    if (m * n < g_min_elems || !device_is_sm100()) return false;
+    // AH / WTA: the kind::f16 kernel of dnmf_tc16.cu (an exact operand, no tf32 calibration involved)
+    if (!kl) return true;
+    // KL: the 16-bit build of the fused KL kernel, whose two GEMMs are kind::tf32 like the fp32 path's
+    calibrate();
+    return g_tc_usable == 1;
   }
   if (dtype != DNMF_F32) return false;
   if (k < 1 || k > 64) return false;
@@ -587,13 +595,13 @@ bool tc_eligible(int op, const void* A, int64_t lda, int64_t m, int64_t n, int64
 void tc_set_min_elems(int64_t elems) { g_min_elems = elems < 0 ? 0 : elems; }
 
 int64_t tc_workspace_bytes(int op, int64_t m, int64_t n, int64_t k, int dtype) {
-  if (op == DNMF_OP_AH_RESIDUAL) return dtype == DNMF_F32 && k <= 32 ? tc_kl_layout(3, m, n).total : 0;
   const bool a16 = dtype == DNMF_A_F16 || dtype == DNMF_A_BF16;
+  if (op == DNMF_OP_AH_RESIDUAL) return (dtype == DNMF_F32 || a16) && k <= 32 ? tc_kl_layout(3, m, n).total : 0;
   if ((dtype != DNMF_F32 && !a16) || k < 1 || k > 64) return 0;
   const int mode = (op == DNMF_OP_AH || op == DNMF_OP_KL_UHT) ? 0 : 1;
   if (op == DNMF_OP_AH || op == DNMF_OP_WTA)
     return a16 ? tc16_layout(mode, m, n, (int)k, dtype).total : fro_layout(mode, m, n, (int)k).total;
-  if ((op == DNMF_OP_KL_UHT || op == DNMF_OP_KL_WTU) && !a16)
+  if (op == DNMF_OP_KL_UHT || op == DNMF_OP_KL_WTU)
     return k > 32 ? tc_kl_layout_k64(mode, m, n).total : tc_kl_layout(mode, m, n).total;
   return 0;
 }
@@ -603,7 +611,7 @@ int tc_pass(int op, int dtype, const void* A, int64_t lda, const float* W, int64
             int64_t ws_bytes, cudaStream_t st, TcPartials* defer) {
   const int mode = (op == DNMF_OP_AH || op == DNMF_OP_KL_UHT) ? 0 : 1;
   if (op == DNMF_OP_KL_UHT || op == DNMF_OP_KL_WTU)
-    return (k > 32 ? tc_kl_run_k64 : tc_kl_run)(mode, (const float*)A, lda, W, ldw, H, ldh, out, ldo, m, n, k, eps,
+    return (k > 32 ? tc_kl_run_k64 : tc_kl_run)(mode, A, dtype, lda, W, ldw, H, ldh, out, ldo, m, n, k, eps,
                                                  transposed_out, ws, ws_bytes, st, defer);
   const float* B = mode == 0 ? H : W;          // the small operand: H (AH) or W (WTA)
   const int64_t ldbsrc = mode == 0 ? ldh : ldw;

@@ -1,4 +1,4 @@
-// Fused KL contractions on the tcgen05 path (fp32 data, k = 32):
+// Fused KL contractions on the tcgen05 path (fp32 or 16-bit data, k <= 64):
 //
 //   UHT : V[m x k]   = (A / (W H + eps)) * H^T          (dist_nmf.py:338-339, :806,:810)
 //   WTU : Y^T[n x k] = (W^T * (A / (W H + eps)))^T      (dist_nmf.py:312-313, :806,:808)
@@ -27,6 +27,11 @@
 //   KK = 64: w0 A-TMA | w1 GEMM2 issuer | w2-5, w11-14 two splitter groups | w6-9 drain | w10 Bcat-TMA + Fr-TMA |
 //            w15 GEMM1 issuer
 // Barrier waits spin on try_wait without the suspend-time hint (mbar_wait_spin, see tc_common.cuh).
+//
+// A 16-bit A (fp16 / bf16, DNMF_A_F16 / DNMF_A_BF16) is read in one place only: the splitters widen their row (column) of
+// the smem tile to fp32 exactly, and everything after that -- U, the tf32 split, both GEMMs, the summation order -- is
+// the fp32 kernel's.  A 16-bit pass is therefore bit-identical to the fp32 pass on the widened matrix; only the tile
+// bytes (8 KB instead of 16 KB) and the swizzle of the MODE 0 / 3 tile (64-byte rows) differ.
 #include "generic_passes.cuh"
 #include "tc_common.cuh"
 #include "tc_api.cuh"
@@ -48,6 +53,7 @@ static_assert(KK == 32 || KK == 64, "KL_KK must be 32 or 64");
 #define KL_FN(name) name
 #endif
 
+template <typename TA>
 struct KlCfg {
   // GROUPS splitter groups of 4 warps work on tiles round-robin; the per-tile chain (A tile -> S load -> divide -> split ->
   // tensor-memory store -> GEMM2 -> slot free) is latency-bound, so the number of tiles in flight sets the pass time.
@@ -58,12 +64,13 @@ struct KlCfg {
   static constexpr int PAIRS = GROUPS * 128;         // residual pairs per CTA (one per splitter thread)
   static constexpr int CHUNK = 4;                    // K-tiles accumulated in TMEM before the drain warps fold them
   static constexpr int N2 = 2 * KK;                    // 64
-  static constexpr int A_BYTES = TC_BM * TC_BK * 4;    // 16 KB
+  static constexpr int A_BYTES = TC_BM * TC_BK * (int)sizeof(TA);   // 16 KB fp32, 8 KB 16-bit
   static constexpr int B_BYTES = N2 * TC_BK * 4;       // 8 KB  Bcat tile  [2k][32 r]
   static constexpr int F_ROWS = 2 * TC_BK;             // reduced indices per factor tile: a pair of tiles
   static constexpr int F_ATOM_BYTES = F_ROWS * 128;    // F_ROWS rows of one 128-byte swizzle atom (32 factor columns)
   static constexpr int F_BYTES = 2 * KATOMS * F_ATOM_BYTES;   // FrCat tile [hi: KATOMS atoms | lo: KATOMS atoms]: 16 / 32 KB
-  // ring depths; KK = 64: 80 KB A ring + 3 x 16 KB Bcat + 2 x 32 KB FrCat pairs = 192 KB
+  // ring depths, in tiles for every element type of A; KK = 64, fp32: 80 KB A ring + 3 x 16 KB Bcat + 2 x 32 KB FrCat
+  // pairs = 192 KB
   static constexpr int SA = (KK == 32) ? 8 : 5, SB = (KK == 32) ? 4 : 3, SF = 2;
   static constexpr int NBUF = (KK == 32) ? 2 : 1, NT = (KK == 32) ? 3 : 2;
   static constexpr int NS = 2, S_COLS = 64;            // one S slot = the S tiles of a pair
@@ -85,15 +92,23 @@ struct KlCfg {
   static_assert(SMEM_BYTES <= 232448, "exceeds the 227 KB opt-in shared memory limit");
 };
 
-// MODE 0 (UHT): x = rows of A, A tile = TMA box {32 cols, 128 rows} with 128B swizzle, Fx = W rows
-// MODE 1 (WTU): x = columns of A, A tile = TMA box {128 cols, 32 rows} unswizzled,   Fx = H^T rows
-template <int MODE>
-__global__ void __launch_bounds__(KlCfg::THREADS, 1)
+// fp32 bits of a 16-bit element of A (fp16 or bf16; both widen exactly)
+template <typename TA>
+__device__ __forceinline__ uint32_t widen_bits(uint32_t b) {
+  if constexpr (std::is_same<TA, __half>::value) return __float_as_uint(__half2float(__ushort_as_half((unsigned short)b)));
+  else return b << 16;
+}
+
+// MODE 0 (UHT): x = rows of A, A tile = TMA box {32 cols, 128 rows} with 128B swizzle (64B for a 16-bit A), Fx = W rows
+// MODE 1 (WTU): x = columns of A, A tile = TMA box {128 cols, 32 rows} unswizzled,                      Fx = H^T rows
+// TA: element type of A (float, __half, __nv_bfloat16)
+template <int MODE, typename TA>
+__global__ void __launch_bounds__(KlCfg<TA>::THREADS, 1)
 tc_kl_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
              const __grid_constant__ CUtensorMap tmF, const float* __restrict__ Fx, int64_t ldfx, int64_t fr_rows_pad,
              float* __restrict__ P, int64_t split_stride, int64_t x_len, int x_blocks, int kt_total, int kt_per_split,
              int num_units, int k_real, float eps, double* __restrict__ pairs_out) {
-  using Cfg = KlCfg;
+  using Cfg = KlCfg<TA>;
   constexpr int SA = Cfg::SA, SB = Cfg::SB, SF = Cfg::SF, NT = Cfg::NT, NS = Cfg::NS, NBUF = Cfg::NBUF, N2 = Cfg::N2;
   constexpr int GROUPS = Cfg::GROUPS, CHUNK = Cfg::CHUNK;
   extern __shared__ uint8_t smem_raw[];
@@ -319,17 +334,40 @@ tc_kl_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
         mbar_wait_spin(bar(iAF + sa), pa);
         const uint8_t* tl = base_ptr + sa * Cfg::A_BYTES;
         uint32_t u[32], lo[32];
-        if (MODE != 1) {
-          const uint8_t* row = tl + r * 128;
+        if constexpr (sizeof(TA) == 4) {
+          if (MODE != 1) {
+            const uint8_t* row = tl + r * 128;
 #pragma unroll
-          for (int c = 0; c < 8; ++c) {
-            const uint4 v = *reinterpret_cast<const uint4*>(row + ((c ^ (r & 7)) << 4));
-            u[4 * c + 0] = v.x; u[4 * c + 1] = v.y; u[4 * c + 2] = v.z; u[4 * c + 3] = v.w;
+            for (int c = 0; c < 8; ++c) {
+              const uint4 v = *reinterpret_cast<const uint4*>(row + ((c ^ (r & 7)) << 4));
+              u[4 * c + 0] = v.x; u[4 * c + 1] = v.y; u[4 * c + 2] = v.z; u[4 * c + 3] = v.w;
+            }
+          } else {
+            const uint8_t* col = tl + r * 4;
+#pragma unroll
+            for (int j = 0; j < 32; ++j) u[j] = *reinterpret_cast<const uint32_t*>(col + j * 512);
           }
         } else {
-          const uint8_t* col = tl + r * 4;
+          // 16-bit A, widened to fp32 exactly (u then holds the bits of A16.float())
+          if (MODE != 1) {
+            // row r = 64 contiguous bytes, 16-byte chunk c stored at position c ^ ((r >> 1) & 3)  (SWIZZLE_64B): the
+            // eight threads of a quarter warp cover all 32 banks, as the fp32 read does
+            const uint8_t* row = tl + r * 64;
 #pragma unroll
-          for (int j = 0; j < 32; ++j) u[j] = *reinterpret_cast<const uint32_t*>(col + j * 512);
+            for (int c = 0; c < 4; ++c) {
+              const uint4 v = *reinterpret_cast<const uint4*>(row + ((c ^ ((r >> 1) & 3)) << 4));
+              const uint32_t w[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+              for (int e = 0; e < 4; ++e) {
+                u[8 * c + 2 * e] = widen_bits<TA>(w[e] & 0xFFFFu);
+                u[8 * c + 2 * e + 1] = widen_bits<TA>(w[e] >> 16);
+              }
+            }
+          } else {
+            const uint8_t* col = tl + r * 2;
+#pragma unroll
+            for (int j = 0; j < 32; ++j) u[j] = widen_bits<TA>(*reinterpret_cast<const uint16_t*>(col + j * 256));
+          }
         }
         // S tile of this accumulator row
         mbar_wait_spin(bar(iSF + ss), ps);
@@ -495,15 +533,29 @@ __global__ void __launch_bounds__(256) kl_transpose_kernel(const float* __restri
   }
 }
 
-template <int MODE>
+template <int MODE, typename TA>
 int kl_launch(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMap& tmF, const float* Fx, int64_t ldfx,
               const KlLayout& L, float* P, int64_t x_len, int k_real, float eps, double* pairs, cudaStream_t st) {
-  if (int rc = smem_attr_once<tc_kl_kernel<MODE>>(KlCfg::SMEM_BYTES, "tc_kl_kernel smem attribute")) return rc;
-  tc_kl_kernel<MODE><<<L.pl.grid, KlCfg::THREADS, KlCfg::SMEM_BYTES, st>>>(
+  using Cfg = KlCfg<TA>;
+  if (int rc = smem_attr_once<tc_kl_kernel<MODE, TA>>(Cfg::SMEM_BYTES, "tc_kl_kernel smem attribute")) return rc;
+  tc_kl_kernel<MODE, TA><<<L.pl.grid, Cfg::THREADS, Cfg::SMEM_BYTES, st>>>(
       tmA, tmB, tmF, Fx, ldfx, L.r_pad, P, x_len * KK, x_len, L.pl.x_blocks, L.pl.kt_total, L.pl.kt_per_split,
       L.pl.num_units, k_real, eps, pairs);
   DNMF_LAUNCH_CHECK("tc_kl_kernel");
   return 0;
+}
+
+// the instantiation for A's storage type (dtype: DNMF_F32, DNMF_A_F16 or DNMF_A_BF16)
+template <int MODE>
+int kl_launch_a(int dtype, const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMap& tmF, const float* Fx,
+                int64_t ldfx, const KlLayout& L, float* P, int64_t x_len, int k_real, float eps, double* pairs,
+                cudaStream_t st) {
+  switch (dtype) {
+    case DNMF_F32: return kl_launch<MODE, float>(tmA, tmB, tmF, Fx, ldfx, L, P, x_len, k_real, eps, pairs, st);
+    case DNMF_A_F16: return kl_launch<MODE, __half>(tmA, tmB, tmF, Fx, ldfx, L, P, x_len, k_real, eps, pairs, st);
+    case DNMF_A_BF16: return kl_launch<MODE, __nv_bfloat16>(tmA, tmB, tmF, Fx, ldfx, L, P, x_len, k_real, eps, pairs, st);
+  }
+  return fail(DNMF_E_UNSUPPORTED, "tcgen05 KL path: no kernel for dtype %d", dtype);
 }
 
 }  // namespace
@@ -516,16 +568,16 @@ KlLayout KL_FN(tc_kl_layout)(int mode, int64_t m, int64_t n) {
   L.r_pad = round_up(r_len, 64);
   L.frcat_bytes = round_up(2 * L.r_pad * KK * 4, 1024);
   L.ht_bytes = mode == 3 ? 0 : round_up(n * (int64_t)KK * 4, 1024);      // plain H^T (Fx of WTU)
-  L.pairs_bytes = mode == 3 ? round_up((int64_t)L.pl.grid * KlCfg::PAIRS * 2 * (int64_t)sizeof(double), 1024) : 0;
+  L.pairs_bytes = mode == 3 ? round_up((int64_t)L.pl.grid * KlCfg<float>::PAIRS * 2 * (int64_t)sizeof(double), 1024) : 0;
   L.total = L.pl.bcat_bytes + L.frcat_bytes + L.ht_bytes + L.pl.partial_bytes + L.pairs_bytes;
   return L;
 }
 
 // The kernel is written for KK factor columns; smaller k ride along zero-padded (zero columns of W / rows of H add nothing
 // to S = W H, and their output columns are dropped by the final reduction).
-int KL_FN(tc_kl_run)(int mode, const float* A, int64_t lda, const float* W, int64_t ldw, const float* H, int64_t ldh, float* out,
-                     int64_t ldo, int64_t m, int64_t n, int k, float eps, int transposed_out, void* ws, int64_t ws_bytes,
-                     cudaStream_t st, TcPartials* defer) {
+int KL_FN(tc_kl_run)(int mode, const void* A, int dtype, int64_t lda, const float* W, int64_t ldw, const float* H,
+                     int64_t ldh, float* out, int64_t ldo, int64_t m, int64_t n, int k, float eps, int transposed_out,
+                     void* ws, int64_t ws_bytes, cudaStream_t st, TcPartials* defer) {
   if (k < 1 || k > KK) return fail(DNMF_E_UNSUPPORTED, "tcgen05 KL path: k must be in [1, %d]", KK);
   const KlLayout L = KL_FN(tc_kl_layout)(mode, m, n);
   const TcPlan& pl = L.pl;
@@ -559,17 +611,17 @@ int KL_FN(tc_kl_run)(int mode, const float* A, int64_t lda, const float* W, int6
     ldfx = KK;
   }
   alignas(64) CUtensorMap tmA, tmB, tmF;
-  if ((rc = tc_map_a(&tmA, A, lda, m, n, mode)) ||
+  if ((rc = tc_map_a(&tmA, A, dtype, lda, m, n, mode)) ||
       (rc = tc_make_map(&tmB, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, Bcat, 2 * KK, r_len, pl.ldb, TC_BK, 2 * KK)) ||
-      (rc = tc_make_map(&tmF, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, FrCat, 2 * L.r_pad, KK, KK, 32, KlCfg::F_ROWS)))
+      (rc = tc_make_map(&tmF, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, FrCat, 2 * L.r_pad, KK, KK, 32, KlCfg<float>::F_ROWS)))
     return rc;
   // (for UHT the x-side factor rows are read straight from W with its own leading dimension: only k_real columns exist)
   const int k_real = mode == 1 ? KK : k;
   switch (mode) {
-    case 0: rc = kl_launch<0>(tmA, tmB, tmF, Fx, ldfx, L, P, x_len, k_real, eps, pairs, st); break;
-    case 1: rc = kl_launch<1>(tmA, tmB, tmF, Fx, ldfx, L, P, x_len, k_real, eps, pairs, st); break;
+    case 0: rc = kl_launch_a<0>(dtype, tmA, tmB, tmF, Fx, ldfx, L, P, x_len, k_real, eps, pairs, st); break;
+    case 1: rc = kl_launch_a<1>(dtype, tmA, tmB, tmF, Fx, ldfx, L, P, x_len, k_real, eps, pairs, st); break;
 #if KL_KK == 32      // the residual variant (BCD, k <= 32) exists in the 32-wide build only
-    case 3: rc = kl_launch<3>(tmA, tmB, tmF, Fx, ldfx, L, P, x_len, k_real, eps, pairs, st); break;
+    case 3: rc = kl_launch_a<3>(dtype, tmA, tmB, tmF, Fx, ldfx, L, P, x_len, k_real, eps, pairs, st); break;
 #endif
     default: return fail(DNMF_E_UNSUPPORTED, "tcgen05 KL path: no kernel for mode %d", mode);
   }
@@ -579,13 +631,13 @@ int KL_FN(tc_kl_run)(int mode, const float* A, int64_t lda, const float* W, int6
 
 #if KL_KK == 32
 // ---- V = A H^T together with ||A - W H||^2 and ||A||^2 in ONE pass over A (MODE 3) -------------------------------------
-int tc_ah_residual_run(const float* A, int64_t lda, const float* W, int64_t ldw, const float* H, int64_t ldh, float* V,
-                       int64_t ldv, int64_t m, int64_t n, int k, void* ws, int64_t ws_bytes, double** out_pairs,
+int tc_ah_residual_run(const void* A, int dtype, int64_t lda, const float* W, int64_t ldw, const float* H, int64_t ldh,
+                       float* V, int64_t ldv, int64_t m, int64_t n, int k, void* ws, int64_t ws_bytes, double** out_pairs,
                        int64_t* n_pairs, cudaStream_t st) {
-  if (int rc = tc_kl_run(3, A, lda, W, ldw, H, ldh, V, ldv, m, n, k, 0.f, 0, ws, ws_bytes, st, nullptr)) return rc;
+  if (int rc = tc_kl_run(3, A, dtype, lda, W, ldw, H, ldh, V, ldv, m, n, k, 0.f, 0, ws, ws_bytes, st, nullptr)) return rc;
   const KlLayout L = tc_kl_layout(3, m, n);
   *out_pairs = reinterpret_cast<double*>(reinterpret_cast<uint8_t*>(ws) + L.total - L.pairs_bytes);
-  *n_pairs = (int64_t)L.pl.grid * KlCfg::PAIRS;
+  *n_pairs = (int64_t)L.pl.grid * KlCfg<float>::PAIRS;
   return 0;
 }
 #endif  // KL_KK == 32

@@ -374,9 +374,10 @@ int tc_begin(void* ws, int64_t ws_bytes, int64_t need, int64_t bcat_bytes, bool 
 // {box_cols, box_rows}; out-of-bounds elements read as zero (ragged edges need no special casing in the kernels)
 int tc_make_map(CUtensorMap* map, CUtensorMapDataType type, const void* ptr, int64_t rows, int64_t cols, int64_t ld,
                 int box_cols, int box_rows, CUtensorMapSwizzle swz = CU_TENSOR_MAP_SWIZZLE_128B);
-// the map of an fp32 A: mode 1 (WTA / WTU, x = columns of A) MN-major tiles, box {TC_BM, TC_BK}, no swizzle; any other
-// mode (x = rows of A) K-major tiles, box {TC_BK, TC_BM}, 128-byte swizzle
-int tc_map_a(CUtensorMap* map, const float* A, int64_t lda, int64_t m, int64_t n, int mode);
+// the map of A (dtype DNMF_F32, or DNMF_A_F16 / DNMF_A_BF16 for the KL kernels) in TC_BK-element tiles: mode 1 (WTA /
+// WTU, x = columns of A) MN-major tiles, box {TC_BM, TC_BK}, no swizzle; any other mode (x = rows of A) K-major tiles,
+// box {TC_BK, TC_BM}, one swizzle row per tile row (128-byte swizzle for fp32, 64-byte for 16-bit elements)
+int tc_map_a(CUtensorMap* map, const void* A, int dtype, int64_t lda, int64_t m, int64_t n, int mode);
 // End of a pass: the split partials P[split][x][kp] are described in *defer, or summed in a fixed order into the k real
 // columns of out: V[x][kk] (mode 0), Y[kk][x] (mode 1) or Y^T[x][kk] (mode 1, transposed_out).  Inline, so that every
 // driver's translation unit keeps its own reduce_partials_kernel.
@@ -407,18 +408,19 @@ int tc16_run(int mode, const void* A, int64_t lda, const float* B, int64_t ldbsr
              TcPartials* defer);
 
 // fused KL contractions (dnmf_tc_kl.cu: k <= 32; the _k64 build, dnmf_tc_kl64.cu: 32 < k <= 64).  mode 0 UHT, 1 WTU,
-// 3 A H^T + residual (32-wide build only).  ws = [Bcat | FrCat | Ht (modes 0, 1) | partials | residual pairs (mode 3)]
+// 3 A H^T + residual (32-wide build only).  A is fp32 or 16-bit (dtype); the layout does not depend on it.
+// ws = [Bcat | FrCat | Ht (modes 0, 1) | partials | residual pairs (mode 3)]
 struct KlLayout {
   TcPlan pl;
   int64_t r_pad, frcat_bytes, ht_bytes, pairs_bytes, total;
 };
 KlLayout tc_kl_layout(int mode, int64_t m, int64_t n);
 KlLayout tc_kl_layout_k64(int mode, int64_t m, int64_t n);
-int tc_kl_run(int mode, const float* A, int64_t lda, const float* W, int64_t ldw, const float* H, int64_t ldh, float* out,
-              int64_t ldo, int64_t m, int64_t n, int k, float eps, int transposed_out, void* ws, int64_t ws_bytes,
-              cudaStream_t st, TcPartials* defer);
-int tc_kl_run_k64(int mode, const float* A, int64_t lda, const float* W, int64_t ldw, const float* H, int64_t ldh, float* out,
-                  int64_t ldo, int64_t m, int64_t n, int k, float eps, int transposed_out, void* ws, int64_t ws_bytes,
-                  cudaStream_t st, TcPartials* defer);
+int tc_kl_run(int mode, const void* A, int dtype, int64_t lda, const float* W, int64_t ldw, const float* H, int64_t ldh,
+              float* out, int64_t ldo, int64_t m, int64_t n, int k, float eps, int transposed_out, void* ws,
+              int64_t ws_bytes, cudaStream_t st, TcPartials* defer);
+int tc_kl_run_k64(int mode, const void* A, int dtype, int64_t lda, const float* W, int64_t ldw, const float* H,
+                  int64_t ldh, float* out, int64_t ldo, int64_t m, int64_t n, int k, float eps, int transposed_out,
+                  void* ws, int64_t ws_bytes, cudaStream_t st, TcPartials* defer);
 
 }  // namespace dnmf
