@@ -74,18 +74,22 @@ struct KlCfg {
   static constexpr int SA = (KK == 32) ? 8 : 5, SB = (KK == 32) ? 4 : 3, SF = 2;
   static constexpr int NBUF = (KK == 32) ? 2 : 1, NT = (KK == 32) ? 3 : 2;
   static constexpr int NS = 2, S_COLS = 64;            // one S slot = the S tiles of a pair
+  static constexpr int NSF = 2 * NS;                   // S-full barriers: pair p fills slot p % NS, signals p % NSF
   static constexpr int ACC_COL0 = 0;
   static constexpr int OP_COL0 = NBUF * N2;            // 128
   static constexpr int S_COL0 = OP_COL0 + NT * 64;
   static constexpr int FX_COL0 = S_COL0 + NS * S_COLS; // 448 (384 for KK = 64)
   static_assert(FX_COL0 + 2 * KK <= 512, "TMEM has 512 columns");
-  // A splitter group waits on a ring slot by phase PARITY, which is only unambiguous while the slot's previous use has
-  // completed.  The group knows that for every tile up to its own previous one (tile - GROUPS; GEMM1 and GEMM2 complete
-  // in tile order), and the slot's previous use is tile - NT (resp. pair p - NS, where the group knows every pair up to
-  // p - ceil(GROUPS / 2) complete): both rings need enough slots, otherwise a group that runs ahead passes the wait one
-  // phase early (observed as a hang with one S slot per tile, NS = 2 and 3 groups).
-  static_assert(2 * NS >= GROUPS + 1 && NT >= GROUPS, "S and operand rings too shallow for the splitter groups");
-  static constexpr int NBARS = 2 * SA + 2 * SB + 2 * SF + 2 * NT + 2 * NS + 2 * NBUF + 2;
+  // A splitter group waits on a full barrier by phase PARITY, which is only unambiguous while the barrier's previous
+  // phase has completed.  The group knows that for every tile up to its own previous one (tile - GROUPS; GEMM1 and GEMM2
+  // complete in tile order).  Operand ring: the barrier's previous use is tile - NT.  S ring: pair p's barrier was last
+  // used by pair p - NSF, and the group only knows pair(tile - GROUPS) >= p - GROUPS complete: a unit of odd tile count
+  // ends in a lone-tile pair, so with one-tile units every pair holds one tile.  With one full barrier per S slot
+  // (NSF = NS = 2, 3 groups) such units let a group pass the wait for pair p while pair p - 2 was still outstanding and
+  // read the S tile of pair p - 4 (tall UHT / residual passes with n <= 32, WTU with m <= 32).  Too shallow a ring also
+  // hangs (observed with one S slot per tile, NS = 2 and 3 groups).
+  static_assert(NSF >= GROUPS && NT >= GROUPS, "S barriers and operand ring too shallow for the splitter groups");
+  static constexpr int NBARS = 2 * SA + 2 * SB + 2 * SF + 2 * NT + NSF + NS + 2 * NBUF + 2;
   static constexpr int BAR_BYTES = 1024;
   static_assert((NBARS + 1) * 8 <= BAR_BYTES, "barrier area too small");
   static constexpr int SMEM_BYTES = SA * A_BYTES + SB * B_BYTES + SF * F_BYTES + 1024 + BAR_BYTES;
@@ -109,7 +113,8 @@ tc_kl_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
              float* __restrict__ P, int64_t split_stride, int64_t x_len, int x_blocks, int kt_total, int kt_per_split,
              int num_units, int k_real, float eps, double* __restrict__ pairs_out) {
   using Cfg = KlCfg<TA>;
-  constexpr int SA = Cfg::SA, SB = Cfg::SB, SF = Cfg::SF, NT = Cfg::NT, NS = Cfg::NS, NBUF = Cfg::NBUF, N2 = Cfg::N2;
+  constexpr int SA = Cfg::SA, SB = Cfg::SB, SF = Cfg::SF, NT = Cfg::NT, NS = Cfg::NS, NSF = Cfg::NSF, NBUF = Cfg::NBUF;
+  constexpr int N2 = Cfg::N2;
   constexpr int GROUPS = Cfg::GROUPS, CHUNK = Cfg::CHUNK;
   extern __shared__ uint8_t smem_raw[];
   const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
@@ -121,7 +126,7 @@ tc_kl_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
   const int iBF = bi; bi += SB;  const int iBE = bi; bi += SB;
   const int iFF = bi; bi += SF;  const int iFE = bi; bi += SF;
   const int iTF = bi; bi += NT;  const int iTE = bi; bi += NT;
-  const int iSF = bi; bi += NS;  const int iSE = bi; bi += NS;
+  const int iSF = bi; bi += NSF; const int iSE = bi; bi += NS;
   const int iCF = bi; bi += NBUF; const int iCE = bi; bi += NBUF;
   const int iXF = bi; bi += 1;   const int iXE = bi; bi += 1;
   const int iSLOT = bi;
@@ -140,7 +145,8 @@ tc_kl_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
     for (int s = 0; s < SB; ++s) { mbar_init(bar(iBF + s), 1); mbar_init(bar(iBE + s), 1); }
     for (int s = 0; s < SF; ++s) { mbar_init(bar(iFF + s), 1); mbar_init(bar(iFE + s), 1); }
     for (int s = 0; s < NT; ++s) { mbar_init(bar(iTF + s), 4); mbar_init(bar(iTE + s), 1); }
-    for (int s = 0; s < NS; ++s) { mbar_init(bar(iSF + s), 1); mbar_init(bar(iSE + s), 8); }
+    for (int s = 0; s < NSF; ++s) mbar_init(bar(iSF + s), 1);
+    for (int s = 0; s < NS; ++s) mbar_init(bar(iSE + s), 8);
     for (int b = 0; b < NBUF; ++b) { mbar_init(bar(iCF + b), 1); mbar_init(bar(iCE + b), 4); }
     mbar_init(bar(iXF), 4);
     mbar_init(bar(iXE), 1);
@@ -223,7 +229,7 @@ tc_kl_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
     // ===================== GEMM1 issuer: S = Fx . Fr^T on tile pairs, runs ahead of GEMM2 by up to NS pairs ==========
     //   cols [0,64) = Fx_hi*Fr_hi + Fx_hi*Fr_lo + Fx_lo*Fr_hi
     constexpr uint32_t idesc_pair = make_idesc(64, 0);      // N = 64 reduced indices
-    int sf = 0, ss = 0;
+    int sf = 0, ss = 0, sfull = 0;
     uint32_t pf = 0, ps = 0, pxu = 0;
     const uint32_t fx_tmem = tmem_base + (uint32_t)Cfg::FX_COL0;
     for (int unit = blockIdx.x; unit < num_units; unit += gridDim.x) {
@@ -238,13 +244,14 @@ tc_kl_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
         if constexpr (KK == 64)
           umma_tile_cat64(tmem_base + (uint32_t)(Cfg::S_COL0 + ss * Cfg::S_COLS), fx_tmem,
                           make_smem_desc(sF0 + sf * Cfg::F_BYTES, 16, 1024), idesc_pair,
-                          bar(iSF + ss), bar(iFE + sf), bar(iXE), (j + 2 >= ntiles) ? 1u : 0u);
+                          bar(iSF + sfull), bar(iFE + sf), bar(iXE), (j + 2 >= ntiles) ? 1u : 0u);
         else
           umma_tile_cat<64>(tmem_base + (uint32_t)(Cfg::S_COL0 + ss * Cfg::S_COLS), fx_tmem,
                             make_smem_desc(sF0 + sf * Cfg::F_BYTES, 16, 1024), idesc_pair,
-                            bar(iSF + ss), bar(iFE + sf), bar(iXE), (j + 2 >= ntiles) ? 1u : 0u);
+                            bar(iSF + sfull), bar(iFE + sf), bar(iXE), (j + 2 >= ntiles) ? 1u : 0u);
         if (++sf == SF) { sf = 0; pf ^= 1u; }
         if (++ss == NS) { ss = 0; ps ^= 1u; }
+        if (++sfull == NSF) sfull = 0;
         __syncwarp();
       }
       pxu ^= 1u;
@@ -327,9 +334,10 @@ tc_kl_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
         // S slots hold PAIRS of tiles: pair index inside this CTA's sequence, which half of the slot is this tile's, and
         // whether the tile has no partner (odd tile count of the unit: it then releases the slot for both)
         const int jt = kt - kt0;
-        const int pairid = pair_base + (jt >> 1);
-        const int ss = pairid % NS, s_half = jt & 1;
-        const uint32_t ps = (uint32_t)(pairid / NS) & 1u;
+        const uint32_t pairid = (uint32_t)(pair_base + (jt >> 1));
+        const int ss = (int)(pairid % NS), s_half = jt & 1;
+        const int sfull = (int)(pairid % NSF);
+        const uint32_t psf = (pairid / NSF) & 1u;
         const bool s_lone = (s_half == 0) && (kt == kt1 - 1);
         mbar_wait_spin(bar(iAF + sa), pa);
         const uint8_t* tl = base_ptr + sa * Cfg::A_BYTES;
@@ -370,7 +378,7 @@ tc_kl_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
           }
         }
         // S tile of this accumulator row
-        mbar_wait_spin(bar(iSF + ss), ps);
+        mbar_wait_spin(bar(iSF + sfull), psf);
         tc_fence_after();
         const uint32_t saddr = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(Cfg::S_COL0 + ss * Cfg::S_COLS + s_half * 32);
         {
