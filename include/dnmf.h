@@ -414,6 +414,44 @@ int dnmf_hals_w_sweep(void* W, int64_t ldw, const void* V, int64_t ldv, const vo
                       void* const* bases, int nranks, int me, int64_t xchg_n, void* scratch, int64_t scratch_bytes, int dtype,
                       void* stream);
 
+/* ---- sparse shards (csrc/dnmf_sparse.cu) ------------------------------------------------------------------------------
+ * The data shard A (m x n) held as compressed rows AND compressed columns, both canonical (indices sorted within each
+ * row / column, no duplicates, no stored zeros):
+ *   CSR: row_ptr int64[m+1], col_idx int32[nnz], val[nnz];   CSC: col_ptr int64[n+1], row_idx int32[nnz], val_t[nnz].
+ * val / val_t and the factors are DNMF_F32 or DNMF_F64; m, n < 2^31; nnz is int64.  The CSC serves W^T A without float
+ * atomics; memory 2 nnz (sizeof(val) + 4) + 8 (m + n + 2) bytes.  Each pass walks fixed chunks of non-zeros (one warp per
+ * chunk), so a heavy row or column does not serialise it; rows that span chunks add their partials in chunk order:
+ * deterministic, repeated calls are bit-identical.  W, H and the outputs are row-major dense, as for the dense entry
+ * points.  Workspace: dnmf_sp_workspace_bytes(m, n, nnz, k, dtype) bytes, for every entry point below.
+ *   dnmf_sp_ah:      V = A H^T over the CSR                                 dist_nmf.py:198, :730
+ *   dnmf_sp_wta:     Y = W^T A (k x n), or Y^T (n x k) with transposed_out, over the CSC   dist_nmf.py:166, :749
+ *   dnmf_sp_kl_uht:  V = (A / (W H + eps)) H^T, W H sampled at the non-zeros only   dist_nmf.py:338-339, :806,:810
+ *   dnmf_sp_kl_wtu:  Y = W^T (A / (W H + eps)), over the CSC                       dist_nmf.py:312-313, :806,:808
+ *   dnmf_sp_residual_sqnorm: out = [||A - W H||_F^2, ||A||_F^2] (float64 [2])     pyDNMF.py:205-210
+ *       = [sum_nz (a - s)^2 + (<W^T W, H H^T> - sum_nz s^2), sum_nz a^2], s = (W H)_ij formed in float64, float64 Grams;
+ *       the bracket (the zeros' share) has an absolute error of ~1e-16 ||W H||^2 and is 0 for a shard without zeros
+ *   dnmf_sp_ah_residual: V = A H^T and the same pair in one walk of the CSR     dist_nmf.py:1023-1024
+ * A zero entry of A contributes nothing to A H^T, W^T A or A / (W H + eps), so these equal the dense expressions. */
+int64_t dnmf_sp_workspace_bytes(int64_t m, int64_t n, int64_t nnz, int64_t k, int dtype);
+int dnmf_sp_ah(const int64_t* row_ptr, const int* col_idx, const void* val, const void* H, int64_t ldh, void* V,
+               int64_t ldv, int64_t m, int64_t n, int64_t nnz, int64_t k, int dtype, void* ws, int64_t ws_bytes,
+               void* stream);
+int dnmf_sp_wta(const int64_t* col_ptr, const int* row_idx, const void* val_t, const void* W, int64_t ldw, void* Y,
+                int64_t ldy, int64_t m, int64_t n, int64_t nnz, int64_t k, int transposed_out, int dtype, void* ws,
+                int64_t ws_bytes, void* stream);
+int dnmf_sp_kl_uht(const int64_t* row_ptr, const int* col_idx, const void* val, const void* W, int64_t ldw,
+                   const void* H, int64_t ldh, void* V, int64_t ldv, int64_t m, int64_t n, int64_t nnz, int64_t k,
+                   double eps, int dtype, void* ws, int64_t ws_bytes, void* stream);
+int dnmf_sp_kl_wtu(const int64_t* col_ptr, const int* row_idx, const void* val_t, const void* W, int64_t ldw,
+                   const void* H, int64_t ldh, void* Y, int64_t ldy, int64_t m, int64_t n, int64_t nnz, int64_t k,
+                   double eps, int transposed_out, int dtype, void* ws, int64_t ws_bytes, void* stream);
+int dnmf_sp_residual_sqnorm(const int64_t* row_ptr, const int* col_idx, const void* val, const void* W, int64_t ldw,
+                            const void* H, int64_t ldh, int64_t m, int64_t n, int64_t nnz, int64_t k, double* out,
+                            int dtype, void* ws, int64_t ws_bytes, void* stream);
+int dnmf_sp_ah_residual(const int64_t* row_ptr, const int* col_idx, const void* val, const void* W, int64_t ldw,
+                        const void* H, int64_t ldh, void* V, int64_t ldv, int64_t m, int64_t n, int64_t nnz, int64_t k,
+                        double* out, int dtype, void* ws, int64_t ws_bytes, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -116,11 +116,20 @@ SIGNATURES = {
     'dnmf_mu_fit_resident_smem_bytes': (i64, [i64, i64, i64, i32, i32]),
     'dnmf_mu_fit_resident_cluster_size': (i32, [i64, i64, i64, i32, i32]),
     'dnmf_mu_fit_resident': (i32, [vp, i64, vp, vp, i64, i64, i64, i64, i32, i32, i64, i64, dbl, i32, vp]),
+    # sparse shards (CSR + CSC)
+    'dnmf_sp_workspace_bytes': (i64, [i64, i64, i64, i64, i32]),
+    'dnmf_sp_ah': (i32, [vp, vp, vp, vp, i64, vp, i64, i64, i64, i64, i64, i32, vp, i64, vp]),
+    'dnmf_sp_wta': (i32, [vp, vp, vp, vp, i64, vp, i64, i64, i64, i64, i64, i32, i32, vp, i64, vp]),
+    'dnmf_sp_kl_uht': (i32, [vp, vp, vp, vp, i64, vp, i64, vp, i64, i64, i64, i64, i64, dbl, i32, vp, i64, vp]),
+    'dnmf_sp_kl_wtu': (i32, [vp, vp, vp, vp, i64, vp, i64, vp, i64, i64, i64, i64, i64, dbl, i32, i32, vp, i64, vp]),
+    'dnmf_sp_residual_sqnorm': (i32, [vp, vp, vp, vp, i64, vp, i64, i64, i64, i64, i64, vp, i32, vp, i64, vp]),
+    'dnmf_sp_ah_residual': (i32, [vp, vp, vp, vp, i64, vp, i64, vp, i64, i64, i64, i64, i64, vp, i32, vp, i64, vp]),
 }
 
 _NO_STATUS = {'dnmf_trace_terms_workspace_bytes', 'dnmf_xchg_bytes', 'dnmf_pass_count', 'dnmf_version', 'dnmf_last_error', 'dnmf_last_path', 'dnmf_launch_count', 'dnmf_workspace_bytes',
               'dnmf_set_force_generic', 'dnmf_set_tc_min_elems', 'dnmf_colsum_workspace_bytes',
-              'dnmf_matvec_workspace_bytes', 'dnmf_mu_fit_resident_smem_bytes', 'dnmf_mu_fit_resident_cluster_size'}
+              'dnmf_matvec_workspace_bytes', 'dnmf_mu_fit_resident_smem_bytes', 'dnmf_mu_fit_resident_cluster_size',
+              'dnmf_sp_workspace_bytes'}
 
 
 class DnmfError(RuntimeError):
@@ -165,6 +174,13 @@ def workspace_bytes(op, m, n, k, dtype):
     b = _lib.dnmf_workspace_bytes(op, m, n, k, dtype)
     if b < 0:
         raise DnmfError('dnmf_workspace_bytes', -1, _lib.dnmf_last_error().decode())
+    return b
+
+
+def sp_workspace_bytes(m, n, nnz, k, dtype):
+    b = _lib.dnmf_sp_workspace_bytes(m, n, nnz, k, dtype)
+    if b < 0:
+        raise DnmfError('dnmf_sp_workspace_bytes', -1, _lib.dnmf_last_error().decode())
     return b
 
 

@@ -12,6 +12,7 @@ import numpy as np
 import torch
 
 from . import _lib as L
+from .sparse import SparseShard
 
 _DT = {torch.float32: L.F32, torch.float64: L.F64}
 # dtype codes of the entry points that read the data shard A, which may also be stored in 16 bits
@@ -154,6 +155,8 @@ class DeviceOps:
     # ---- A-streaming contractions -----------------------------------------------------------
     def ah(self, A, H, out=None):
         """V = A @ H.T   (dist_nmf.py:198, :730)"""
+        if isinstance(A, SparseShard):
+            return self._sp_rows('dnmf_sp_ah', 'ah', A, None, H, out)
         m, n = A.shape
         k = H.shape[0]
         dt = _DT_A[A.dtype]
@@ -167,6 +170,8 @@ class DeviceOps:
 
     def wta(self, A, W, transposed_out=False, out=None):
         """Y = W.T @ A (k x n), or Y.T (n x k) when transposed_out   (dist_nmf.py:166, :749)"""
+        if isinstance(A, SparseShard):
+            return self._sp_cols('dnmf_sp_wta', 'wta', A, W, None, transposed_out, out)
         m, n = A.shape
         k = W.shape[1]
         dt = _DT_A[A.dtype]
@@ -180,6 +185,8 @@ class DeviceOps:
 
     def kl_uht(self, A, W, H, eps, out=None):
         """V = (A / (W @ H + eps)) @ H.T without materialising W @ H   (dist_nmf.py:338-339, :806,:810)"""
+        if isinstance(A, SparseShard):
+            return self._sp_rows('dnmf_sp_kl_uht', 'kl_uht', A, W, H, out, eps)
         m, n = A.shape
         k = H.shape[0]
         dt = _DT_A[A.dtype]
@@ -193,6 +200,8 @@ class DeviceOps:
 
     def kl_wtu(self, A, W, H, eps, transposed_out=False, out=None):
         """Y = W.T @ (A / (W @ H + eps))   (dist_nmf.py:312-313, :806,:808)"""
+        if isinstance(A, SparseShard):
+            return self._sp_cols('dnmf_sp_kl_wtu', 'kl_wtu', A, W, H, transposed_out, out, eps)
         m, n = A.shape
         k = H.shape[0]
         dt = _DT_A[A.dtype]
@@ -204,6 +213,52 @@ class DeviceOps:
                self._stream())
         self._t1(ev)
         return Y
+
+    # ---- sparse shards (csrc/dnmf_sparse.cu): the CSR serves A H^T and the residual, the CSC W^T A ------------------
+    def _sp_ws(self, A, k):
+        nb = L.sp_workspace_bytes(A.shape[0], A.shape[1], A.nnz, k, _DT[A.dtype])
+        return self.workspace(nb), max(nb, self._ws_bytes)
+
+    def _sp_rows(self, name, timer, A, W, H, out, eps=None):
+        m, n = A.shape
+        k = H.shape[0]
+        V = out if out is not None else self.empty((m, k), A.dtype)
+        ws, wsb = self._sp_ws(A, k)
+        w = (W.data_ptr(), _ld(W)) if W is not None else ()
+        e = (float(eps),) if eps is not None else ()
+        ev = self._t0(timer)
+        L.call(name, A.row_ptr.data_ptr(), A.col_idx.data_ptr(), A.val.data_ptr(), *w, H.data_ptr(), _ld(H), V.data_ptr(),
+               _ld(V), m, n, A.nnz, k, *e, _DT[A.dtype], ws, wsb, self._stream())
+        self._t1(ev)
+        return V
+
+    def _sp_cols(self, name, timer, A, W, H, transposed_out, out, eps=None):
+        m, n = A.shape
+        k = W.shape[1]
+        Y = out if out is not None else self.empty((n, k) if transposed_out else (k, n), A.dtype)
+        ws, wsb = self._sp_ws(A, k)
+        h = (H.data_ptr(), _ld(H)) if H is not None else ()
+        e = (float(eps),) if eps is not None else ()
+        ev = self._t0(timer)
+        L.call(name, A.col_ptr.data_ptr(), A.row_idx.data_ptr(), A.val_t.data_ptr(), W.data_ptr(), _ld(W), *h,
+               Y.data_ptr(), _ld(Y), m, n, A.nnz, k, *e, 1 if transposed_out else 0, _DT[A.dtype], ws, wsb, self._stream())
+        self._t1(ev)
+        return Y
+
+    def _sp_residual(self, A, W, H, V=None):
+        m, n = A.shape
+        k = W.shape[1]
+        out = self.empty((2,), torch.float64)
+        ws, wsb = self._sp_ws(A, k)
+        a = (A.row_ptr.data_ptr(), A.col_idx.data_ptr(), A.val.data_ptr(), W.data_ptr(), _ld(W), H.data_ptr(), _ld(H))
+        if V is None:
+            L.call('dnmf_sp_residual_sqnorm', *a, m, n, A.nnz, k, out.data_ptr(), _DT[A.dtype], ws, wsb, self._stream())
+        else:
+            ev = self._t0('ah_res')
+            L.call('dnmf_sp_ah_residual', *a, V.data_ptr(), _ld(V), m, n, A.nnz, k, out.data_ptr(), _DT[A.dtype], ws, wsb,
+                   self._stream())
+            self._t1(ev)
+        return out
 
     # ---- pass with the split reduction deferred to the consumer (include/dnmf.h: dnmf_*_p) ---------------------------
     def _pass_partials(self, name, timer, op, A, k, *args):
@@ -227,22 +282,30 @@ class DeviceOps:
         return view
 
     def ah_p(self, A, H):
+        if isinstance(A, SparseShard):
+            return None       # sparse passes have no deferred form: the caller takes the plain op
         m, n = A.shape
         k = H.shape[0]
         return self._pass_partials('dnmf_ah_p', 'ah', L.OP_AH, A, k, A.data_ptr(), _ld(A), H.data_ptr(), _ld(H), m, n, k)
 
     def wta_p(self, A, W):
+        if isinstance(A, SparseShard):
+            return None       # sparse passes have no deferred form: the caller takes the plain op
         m, n = A.shape
         k = W.shape[1]
         return self._pass_partials('dnmf_wta_p', 'wta', L.OP_WTA, A, k, A.data_ptr(), _ld(A), W.data_ptr(), _ld(W), m, n, k)
 
     def kl_uht_p(self, A, W, H, eps):
+        if isinstance(A, SparseShard):
+            return None       # sparse passes have no deferred form: the caller takes the plain op
         m, n = A.shape
         k = W.shape[1]
         return self._pass_partials('dnmf_kl_uht_p', 'kl_uht', L.OP_KL_UHT, A, k, A.data_ptr(), _ld(A), W.data_ptr(), _ld(W),
                                    H.data_ptr(), _ld(H), m, n, k, float(eps))
 
     def kl_wtu_p(self, A, W, H, eps):
+        if isinstance(A, SparseShard):
+            return None       # sparse passes have no deferred form: the caller takes the plain op
         m, n = A.shape
         k = W.shape[1]
         return self._pass_partials('dnmf_kl_wtu_p', 'kl_wtu', L.OP_KL_WTU, A, k, A.data_ptr(), _ld(A), W.data_ptr(), _ld(W),
@@ -327,7 +390,9 @@ class DeviceOps:
         return out
 
     def sqnorm(self, X):
-        """sum(X**2) as a float64 device scalar (shape [1])."""
+        """sum(X**2) as a float64 device scalar (shape [1]); for a sparse shard, of its non-zeros."""
+        if isinstance(X, SparseShard):
+            X = X.val.view(1, -1)
         r, c = X.shape
         out = self.empty((1,), torch.float64)
         ws, wsb = self._ws_for(L.OP_SUMS, r, c, min(c, L.MAX_K), _DT[out_dtype(X.dtype)])
@@ -356,6 +421,8 @@ class DeviceOps:
 
     def residual_sqnorm(self, A, W, H):
         """[||A - W H||_F^2, ||A||_F^2] as a float64 device tensor of shape [2]."""
+        if isinstance(A, SparseShard):
+            return self._sp_residual(A, W, H)
         m, n = A.shape
         k = W.shape[1]
         dt = _DT_A[A.dtype]
@@ -367,6 +434,9 @@ class DeviceOps:
 
     def ah_residual(self, A, W, H):
         """(A @ H.T, [||A - W H||_F^2, ||A||_F^2]) in one pass over A (dist_nmf.py:1023-1024)."""
+        if isinstance(A, SparseShard):
+            V = self.empty((A.shape[0], W.shape[1]), A.dtype)
+            return V, self._sp_residual(A, W, H, V)
         m, n = A.shape
         k = W.shape[1]
         dt = _DT_A[A.dtype]
@@ -469,6 +539,8 @@ class DeviceOps:
 
     # ---- shard ops ------------------------------------------------------------------------------
     def nnz_counts(self, A):
+        if isinstance(A, SparseShard):
+            return A.nnz_counts()
         m, n = A.shape
         rows = self.empty((m,), torch.int64)
         cols = self.empty((n,), torch.int64)

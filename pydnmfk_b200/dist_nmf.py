@@ -25,6 +25,7 @@ import torch
 
 from . import device as D
 from . import peer
+from .sparse import SparseShard, is_sparse_input
 from .utils import norm, comm_timing, parse, var_init  # noqa: F401  (re-exported like the reference)
 from .dist_comm import MPI  # noqa: F401
 
@@ -49,9 +50,9 @@ class _AlgBase:
         self.rank = self.comm1.rank
         self.ops = D.default_ops()
         self._A_orig = A_ij
-        self._numpy_io = not isinstance(A_ij, torch.Tensor)
+        self._numpy_io = not isinstance(A_ij, (torch.Tensor, SparseShard))
         self._np_dtype = A_ij.dtype if self._numpy_io else None
-        A = D.to_device(A_ij)
+        A = SparseShard.from_any(A_ij) if is_sparse_input(A_ij) else D.to_device(A_ij)
         # factor dtype: the data dtype, or float32 when the shard is stored in 16 bits (PyNMF's params.a_storage)
         self.fdtype = D.out_dtype(A.dtype)
         return A, D.to_device(W, self.fdtype), D.to_device(H, self.fdtype)
@@ -446,14 +447,22 @@ class nmf_algorithms_1D(_AlgBase):
         elif (B is self.A_ij or B is self._A_orig) and D.to_device_view(A, dt).shape[0] <= D.L.MAX_K:
             out = self.ops.wta(self.A_ij, D.to_device_view(A, dt).t().contiguous())
         else:
-            out = self._mm_chunked(D.to_device_view(A, dt).contiguous(), D.to_device_view(B, dt))
+            sparse_b = isinstance(self.A_ij, SparseShard) and (B is self.A_ij or B is self._A_orig)
+            out = self._mm_chunked(D.to_device_view(A, dt).contiguous(), self.A_ij if sparse_b else D.to_device_view(B, dt))
         return self.comm1.allreduce_(out) if p != 1 else out
 
     def _mm_chunked(self, A, B):
-        """A [r x c] @ B [c x s] for any s: out[:, j0:j1] = A (B[:, j0:j1]^T)^T in chunks of <= MAX_K columns."""
+        """A [r x c] @ B [c x s] for any s: out[:, j0:j1] = A (B[:, j0:j1]^T)^T in chunks of <= MAX_K columns.  A sparse
+        shard B is the right operand of W^T A instead: out[j0:j1] = (A[j0:j1]^T)^T B in chunks of <= MAX_K rows."""
         r, s_cols = A.shape[0], B.shape[1]
-        out = self.ops.empty((r, s_cols), D.out_dtype(A.dtype))
         step = D.L.MAX_K
+        if isinstance(B, SparseShard):
+            out = self.ops.empty((r, s_cols), B.dtype)
+            for j0 in range(0, r, step):
+                j1 = min(r, j0 + step)
+                self.ops.wta(B, A[j0:j1].t().contiguous(), out=out[j0:j1])
+            return out
+        out = self.ops.empty((r, s_cols), D.out_dtype(A.dtype))
         for j0 in range(0, s_cols, step):
             j1 = min(s_cols, j0 + step)
             out[:, j0:j1] = self.ops.ah(A, B[:, j0:j1].t().contiguous())

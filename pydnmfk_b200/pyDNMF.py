@@ -20,6 +20,7 @@ from .dist_nmf import nmf_algorithms_1D, nmf_algorithms_2D
 from .utils import data_operations, determine_block_params, var_init, comm_timing
 from .dist_comm import MPI
 from .graphs import StepGraphs, graphs_enabled
+from .sparse import SparseShard, is_sparse_input
 
 
 _A_STORAGE = {'float16': torch.float16, 'bfloat16': torch.bfloat16}
@@ -64,6 +65,15 @@ def draw_rand_factors(topo, p_c, rank, a_shape, factor_shape, k, dt):
     return W, H
 
 
+def _check_sparse_params(params):
+    """What a sparse A_ij does not support; raised before anything reaches the device."""
+    if getattr(params, 'a_storage', None) is not None:
+        raise ValueError('params.a_storage does not apply to a sparse A_ij (its values are stored as float32 / float64)')
+    if getattr(params, 'init', None) == 'nnsvd':
+        raise ValueError("init='nnsvd' is not supported for a sparse A_ij (DistSVD deflates a dense copy of A); use "
+                         "init='rand' or given factors")
+
+
 class PyNMF():
     r"""Distributed NMF decomposition of the matrix whose local shard is ``A_ij``.
 
@@ -71,6 +81,12 @@ class PyNMF():
     CUDA tensor), ``factors`` optional ``[W, H]`` shards, ``params`` attribute bag with ``init,
     comm1, comm, k, p_r, p_c (or grid), row_comm, col_comm, verbose`` and optional ``itr, norm,
     method, prune, W_update``, ``a_storage``.
+
+    ``A_ij`` may also be sparse: a ``scipy.sparse`` matrix / array (results come back as numpy arrays) or a ``torch``
+    sparse CSR tensor (results come back as tensors).  The shard is then held on the device as CSR + CSC
+    (``sparse.SparseShard``) and every pass reads only its non-zeros; FRO-MU, KL-MU, HALS and BCD, pruning, given
+    factors, ``err_monitor`` and CUDA-graph replay work as for dense data.  ``init='nnsvd'``, ``a_storage`` and
+    ``column_err`` raise ValueError for sparse data.
 
     ``params.a_storage`` = 'float16' / 'bfloat16' holds only the data shard in 16 bits on the device (half the memory and
     half the bytes each pass streams); W, H, every update and every reduction stay float32.  The fit is then the float32
@@ -82,7 +98,10 @@ class PyNMF():
     @comm_timing()
     def __init__(self, A_ij, factors=None, save_factors=False, params=None):
         self.params = params
-        self._numpy_in = not isinstance(A_ij, torch.Tensor)
+        self._sparse = is_sparse_input(A_ij)
+        if self._sparse:
+            _check_sparse_params(params)
+        self._numpy_in = not isinstance(A_ij, (torch.Tensor, SparseShard))
         self._a_dtype = a_storage_dtype(getattr(params, 'a_storage', None), A_ij)
         if self._a_dtype is not None:
             self._np_dtype = np.dtype(np.float32)                   # factors, eps and recon_err stay float32
@@ -123,7 +142,9 @@ class PyNMF():
         # the shard goes to HBM once and stays there.  From page-locked host memory the copy runs asynchronously while
         # the host draws the initial factors (the RNG replay below is ~0.1 s at 65536 x 32); the constructor waits for it
         # before returning, so the caller's buffer is never read after this call
-        if self._a_dtype is not None:
+        if self._sparse:
+            self.A_ij = SparseShard.from_any(A_ij)
+        elif self._a_dtype is not None:
             self.A_ij = D.to_device_a16(A_ij, self._a_dtype)
         else:
             self.A_ij = D.to_device(A_ij, self._tdtype, non_blocking=True)
@@ -189,7 +210,7 @@ class PyNMF():
         """Whole-fit on-chip path (dnmf_mu_fit_resident): single-process grid, MU, shard + factors fit in one SM."""
         W, H = self._get_factors()
         # (the on-chip kernel reads A in the factor dtype: a 16-bit shard takes the per-kernel path)
-        return (self._a_dtype is None and self.comm1.size == 1 and self.method.lower() == 'mu'
+        return (self._a_dtype is None and not self._sparse and self.comm1.size == 1 and self.method.lower() == 'mu'
                 and self.norm.lower() in ('fro', 'kl')
                 and var_init(self.params, 'resident_fit', True) and self.itr >= 1 and W.shape[0] > 0 and H.shape[1] > 0
                 and self.ops.resident_fit_fits(W.shape[0], H.shape[1], self.k, self.norm, self._tdtype))
@@ -302,6 +323,8 @@ class PyNMF():
     @comm_timing()
     def column_err(self):
         """Per-column relative L2 error over the global column range (pyDNMF.py:221-239)."""
+        if self._sparse:
+            raise ValueError('column_err is not available for a sparse A_ij')
         dtr_blk = determine_block_params(self.comm1, (self.p_r, self.p_c), (self.params.m, self.params.n))
         dtr_blk_idx = dtr_blk.determine_block_index_range_asymm()
         num, den = self.ops.column_err(self.A_ij, self.W_i, self.H_j)

@@ -14,6 +14,7 @@ from . import config   # noqa: F401
 from . import device as D
 from .pyDNMF import *  # noqa: F401,F403
 from .pyDNMF import PyNMF
+from .sparse import is_sparse_input
 from .utils import comm_timing, var_init, Checkpoint
 
 
@@ -84,6 +85,9 @@ class PyNMFk():
         if getattr(params, 'a_storage', None) is not None:
             raise ValueError('params.a_storage is not supported by PyNMFk: the perturbed ensemble would need its own '
                              'rounding rule; fit the rounded matrix in float32 instead')
+        if is_sparse_input(A_ij):
+            raise ValueError('PyNMFk does not take a sparse A_ij: its perturbations change every entry of the matrix, '
+                             'zeros included, and their random stream is part of the reference parity; densify the shard')
         self.A_ij = A_ij
         self.local_m, self.local_n = self.A_ij.shape
         self.params = params

@@ -17,6 +17,7 @@ import torch
 from . import config
 from .dist_comm import MPI
 from . import device as D
+from .sparse import SparseShard, is_sparse_input
 
 config.init(0)
 
@@ -111,7 +112,9 @@ class data_operations():
 
     # -- pruning -------------------------------------------------------------------------------
     def _device_data(self):
-        if not (isinstance(self.ten, torch.Tensor) and self.ten.is_cuda):
+        if is_sparse_input(self.ten):
+            self.ten = SparseShard.from_any(self.ten)
+        elif not (isinstance(self.ten, torch.Tensor) and self.ten.is_cuda):
             self.ten = D.to_device(self.ten)
         return self.ten
 
@@ -148,8 +151,13 @@ class data_operations():
         return torch.from_numpy(np.flatnonzero(mask).astype(np.int64))
 
     def prune(self, data, row_zero_idx, col_zero_idx):
-        """data[np.ix_(rows, cols)] as a device gather (utils.py:137-156)."""
+        """data[np.ix_(rows, cols)] as a device gather (utils.py:137-156).  A sparse shard is compacted instead: kept rows
+        and columns are renumbered, values and their order stay (the dropped rows and columns are empty)."""
         ops = D.default_ops()
+        if is_sparse_input(data):
+            X = SparseShard.from_any(data)
+            return X.compact(self._idx(row_zero_idx, X.shape[0]).to(X.device),
+                             self._idx(col_zero_idx, X.shape[1]).to(X.device))
         X = D.to_device(data)
         ri = self._idx(row_zero_idx, X.shape[0]).to(X.device)
         ci = self._idx(col_zero_idx, X.shape[1]).to(X.device)
